@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Gbases/s of the k-mer matrix build (k=31) on N B200s, with roofline, CPU baseline and parity check.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config auto|c1|c2|c3|c3w|c4|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config auto|c1|c2|c3|c3w|c4|c5] [--dump-outputs DIR]
     python bench.py --impl reference [...]        CPU arm: the oracle port on the host cores (rank 0 only)
     (N > 1: launched by torch.distributed.run, one rank per GPU)
 
@@ -20,6 +20,10 @@ Configs (BASELINE.json): c1 = 20 genomes, from-contigs (singletons dropped); c2 
 (singletons kept) -- the N = 1 default; c3 = 1,000 genomes over N GPUs (strong scaling); c3w = 125 genomes per GPU
 (weak scaling: the N > 1 default, 1,000 genomes at N = 8); c4 = 200 read sets of 30x 150 bp reads, min abundance 2;
 c5 = 500 genomes, k in {15, 21, 31} x singletons kept / dropped (one line with a sweep list).
+
+--dump-outputs DIR: after the timed steps, a fixed, seeded sample of the columns of the last timed build goes to DIR as
+.npy files (see dump_outputs), so that two builds of the project can be compared output for output: the inputs are the
+same bytes on every run with the same arguments.
 """
 from __future__ import annotations
 
@@ -41,6 +45,8 @@ UNIT = "Gbases/s"
 K = 31
 READS_PER_GENOME = 1_000_000      # 30x of a 5 Mbp genome at 150 bp
 CPU_SAMPLE_BASES = 5.0e8          # bounded sample of the CPU arms: about 6 s on 16 cores
+DUMP_BYTES = 48 << 20             # --dump-outputs: bytes of .npy data in all (the c5 sweep shares it among its builds)
+DUMP_SEED = 1
 
 CONFIGS = {
     "c1": dict(genomes=20, per_gpu=False, reads=False, min_ab=1, keep=False,
@@ -342,6 +348,40 @@ def e2e_files(texts, names, conf, k):
         shutil.rmtree(d, ignore_errors=True)
 
 
+def dump_outputs(db, out_dir, prefix, n_genomes, budget, rank, world, dist):
+    """Write a seeded sample of the columns of db's last build to out_dir/<prefix><name>.npy (rank 0; collective at N > 1):
+      kmers   float32 [n][k]  bases of each sampled k-mer, first base first, in the 2-bit code of the packed k-mers
+                              (A 0, C 1, T 2, G 3)
+      matrix  float32 [G][n]  1 where genome g holds the k-mer, else 0
+      columns float64 [n]     indices of the sampled columns in the result's column order (ascending)
+      n_kmers float64 [1]     number of columns of the result
+    Every value is a small integer, so a changed k-mer or presence bit differs by at least 1.  n is as many columns as
+    `budget` bytes hold; the sample is drawn with DUMP_SEED from the column count alone."""
+    import numpy as np
+    counts = db.slice_counts()                   # the global column order is the ranks' slices in rank order
+    U, off = sum(counts), sum(counts[:rank])
+    n = min(U, budget // (4 * (db.k + n_genomes) + 8))
+    cols = np.sort(np.random.default_rng(DUMP_SEED).choice(U, n, replace=False)) if n < U else np.arange(U)
+    mine = cols[(cols >= off) & (cols < off + counts[rank])] - off
+    km, mat = db.builder.kmers()[mine], db.builder.matrix()[:, mine]
+    if world > 1:
+        parts = [None] * world if rank == 0 else None
+        dist.gather_object((km, mat), parts, dst=0)
+        if rank != 0:
+            return
+        km, mat = np.concatenate([p[0] for p in parts]), np.concatenate([p[1] for p in parts], axis=1)
+    shifts = np.uint64(2) * np.arange(db.k - 1, -1, -1, dtype=np.uint64)
+    bases = (km[:, None] >> shifts) & np.uint64(3)
+    # genome g is bit 63 - g % 64 of word row g // 64: the bits of the big-endian bytes, most significant first
+    W = mat.shape[0]
+    bits = np.unpackbits(np.ascontiguousarray(mat, dtype=">u8").view(np.uint8).reshape(W, n, 8), axis=2)
+    presence = bits.transpose(0, 2, 1).reshape(W * 64, n)[:n_genomes]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("kmers", bases.astype(np.float32)), ("matrix", presence.astype(np.float32)),
+                    ("columns", cols.astype(np.float64)), ("n_kmers", np.array([U], dtype=np.float64))):
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -354,8 +394,14 @@ def main():
     ap.add_argument("--no-parity-check", action="store_true")
     ap.add_argument("--no-e2e-files", action="store_true")
     ap.add_argument("--no-e2e-pipeline", action="store_true", help="e2e with one context only (no builds in flight side by side)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a seeded sample of what the last timed build computed to DIR/*.npy (at most 48 MiB)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 0)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's result; the reference arm has none")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -433,6 +479,9 @@ def main():
             stats.update({k2: v for k2, v in db.local_stats.items() if k2 in (
                 "n_windows", "n_input_bytes", "n_bases", "n_records", "n_buckets", "n_units", "n_unit_entries", "n_wide",
                 "n_unit_buckets", "n_rounds", "n_solid_records")})
+            if args.dump_outputs:
+                dump_outputs(db, args.dump_outputs, "" if si == 0 else f"k{k}_{'kept' if keep else 'dropped'}_", G_total,
+                             DUMP_BYTES // len(sweep), rank, world, dist)
             res = {"k": k, "keep": keep, "ms": ms, "stage_acc": stage_acc, "launches": launches, "stats": stats,
                    "U_local": db.n_kmers, "clocks": clocks, "ms_e2e": 0.0, "e2e_steps": 0, "h2d": 0, "d2h": 0, "parity": None}
             if si == 0:

@@ -104,19 +104,41 @@ def test_surveyor_tsv_written_by_two_ranks(gpu, tmp_path):
 
 
 def test_bench_parity_check_under_torchrun(gpu, tmp_path):
-    """bench.py at N = 2 through the launcher the driver uses: the line must carry parity_check.ok (GPU checksum of the
-    ranks' slices, summed, against the oracle's matrix of the same genomes).  Needs two GPUs (NCCL refuses two ranks on
-    one device); on a one-GPU box the N = 1 line is checked instead."""
+    """bench.py at N = 2 under torch.distributed.run: the line must carry parity_check.ok (GPU checksum of the ranks'
+    slices, summed, against the oracle's matrix of the same genomes), and --dump-outputs must hold the oracle's k-mers
+    and presence bits at the sampled columns.  Needs two GPUs (NCCL refuses two ranks on one device); on a one-GPU box
+    the N = 1 line is checked instead."""
     import torch
+    from grm_b200 import synth
     n = 2 if torch.cuda.device_count() >= 2 else 1
     cmd = [sys.executable]
     if n > 1:
         cmd += ["-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(n), "--master-addr", "127.0.0.1",
                 "--master-port", "29533"]
+    out = tmp_path / "outputs"
     cmd += [os.path.join(ROOT, "bench.py"), "--gpus", str(n), "--steps", "2", "--warmup", "1", "--genomes", "6",
-            "--no-cpu-baseline"]
+            "--no-cpu-baseline", "--dump-outputs", str(out)]
     p = subprocess.run(cmd, cwd=ROOT, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=900)
     assert p.returncode == 0, p.stderr[-3000:]
     line = json.loads([ln for ln in p.stdout.splitlines() if ln.startswith("{")][-1])
     assert line["n_gpus"] == n and line["parity_check"]["ok"] is True, line.get("parity_check")
     assert line["parity_check"]["against"].startswith("oracle")
+
+    c = line["config"]
+    G, k = c["genomes"], c["k"]
+    cfg = synth.SynthConfig(seed=synth.MASTER_SEED + 1)           # bench.py's inputs, made on the host
+    ref = oracle.build([[(synth.genome_fasta(cfg, g), 0)] for g in range(G)], k, c["min_abundance"], c["keep_singletons"])
+    d = {name: np.load(out / f"{name}.npy") for name in ("kmers", "matrix", "columns", "n_kmers")}
+    assert sum(a.nbytes for a in d.values()) <= 64 << 20
+    assert d["kmers"].dtype == d["matrix"].dtype == np.float32 and d["columns"].dtype == np.float64
+    assert d["n_kmers"].tolist() == [ref.n_kmers]
+    cols = d["columns"].astype(np.int64)
+    assert 0 < len(cols) and np.all(np.diff(cols) > 0) and cols[-1] < ref.n_kmers
+    assert d["kmers"].shape == (len(cols), k) and d["matrix"].shape == (G, len(cols))
+    packed = np.zeros(len(cols), dtype=np.uint64)
+    for i in range(k):
+        packed = (packed << np.uint64(2)) | d["kmers"][:, i].astype(np.uint64)
+    assert np.array_equal(packed, ref.kmers[cols])
+    g = np.arange(G)
+    bits = (ref.matrix[g // 64][:, cols] >> (np.uint64(63) - (g % 64).astype(np.uint64))[:, None]) & np.uint64(1)
+    assert np.array_equal(d["matrix"], bits.astype(np.float32))
