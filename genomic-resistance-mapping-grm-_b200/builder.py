@@ -206,6 +206,49 @@ class KmerMatrixBuilder:
                                              C.c_void_p(out.ctypes.data), out.size))
         return out
 
+    def load_result(self, kmers, matrix, n_genomes: int) -> "KmerMatrixBuilder":
+        """An existing matrix (e.g. a .kover file's kmer_matrix, row-major ceil(G/64) x U words, and its packed k-mers)
+        as this context's result, as if it had been built: every result-side call then works on it."""
+        kmers = np.ascontiguousarray(kmers, dtype=np.uint64).reshape(-1)
+        matrix = np.ascontiguousarray(matrix, dtype=np.uint64)
+        W = (int(n_genomes) + 63) // 64
+        if matrix.shape != (W, kmers.size):
+            raise ValueError(f"matrix of shape {matrix.shape} for {kmers.size} k-mers and {n_genomes} genomes")
+        self._check(self._lib.grmkm_load_result(self._ctx, C.c_void_p(kmers.ctypes.data), C.c_void_p(matrix.ctypes.data),
+                                                kmers.size, int(n_genomes)))
+        return self
+
+    def scm_run(self, jobs, blacklist=()) -> list[tuple[np.ndarray, np.ndarray]]:
+        """Set Covering Machine fits on the resident matrix, all in one grmkm_scm_run.  jobs: (model_type, p, max_rules,
+        tiebreak, pos_mask, neg_mask) with masks of ceil(G/64) uint64 words.  -> per fit (steps, equivalent rules):
+        steps is a structured array with the fields of grmkm_scm_step."""
+        _, W, _ = self.dims
+        masks, arr = [], (native.ScmJob * max(1, len(jobs)))()
+        for i, (model_type, p, max_rules, tiebreak, pos, neg) in enumerate(jobs):
+            pos = np.ascontiguousarray(pos, dtype=np.uint64)
+            neg = np.ascontiguousarray(neg, dtype=np.uint64)
+            if pos.shape != (W,) or neg.shape != (W,):
+                raise ValueError(f"example masks of {pos.shape} / {neg.shape} words for {W} matrix word rows")
+            masks += [pos, neg]
+            arr[i] = native.ScmJob(C.sizeof(native.ScmJob), int(model_type), int(max_rules), int(bool(tiebreak)), float(p),
+                                   pos.ctypes.data, neg.ctypes.data)
+        bl = np.ascontiguousarray(blacklist if blacklist is not None else (), dtype=np.uint64).reshape(-1)
+        self._check(self._lib.grmkm_scm_run(self._ctx, len(jobs), arr, C.c_void_p(bl.ctypes.data), bl.size))
+        out = []
+        step_dtype = np.dtype([("rule", np.uint64), ("utility", np.float64), ("positive_errors", np.uint32),
+                               ("negative_covers", np.uint32), ("equiv_offset", np.uint64), ("equiv_count", np.uint64)])
+        for f in range(len(jobs)):
+            ns, ne = C.c_uint64(), C.c_uint64()
+            rc = self._lib.grmkm_scm_result(self._ctx, f, None, 0, C.byref(ns), None, 0, C.byref(ne))
+            if rc not in (native.OK, native.E_CAPACITY):
+                self._check(rc)
+            steps = np.zeros(ns.value, dtype=step_dtype)
+            eq = np.zeros(ne.value, dtype=np.uint64)
+            self._check(self._lib.grmkm_scm_result(self._ctx, f, C.c_void_p(steps.ctypes.data), steps.size, C.byref(ns),
+                                                   C.c_void_p(eq.ctypes.data), eq.size, C.byref(ne)))
+            out.append((steps, eq))
+        return out
+
     def device_result(self) -> tuple[int, int, int]:
         """(device pointer of kmers[U], device pointer of the matrix, row pitch in words): word row w of the matrix
         starts at pointer + 8 * w * pitch."""

@@ -5,6 +5,7 @@
 #include "grmkm_units.cuh"
 #include "grmkm_result.cuh"
 #include "grmkm_synth.cuh"
+#include "grmkm_scm.cuh"
 
 #include <nvtx3/nvToolsExt.h>      // header-only; the ranges cost nothing until a tool (nsys, ncu --nvtx) attaches
 #include <zlib.h>
@@ -95,7 +96,9 @@ struct grmkm_ctx {
         offsets, offsets2, bcounts, ukeys, uwords, kmers, matrix,
         scalars, fmt, synth, refs, stile_file, bbase, apub, masks, units, ucur, ubeg, wu, wide,
         racc,            // abundance builds: the solid presence records of the rounds done so far
-        aux;             // result-side kernels: row mask / per-column sums / checksum / bit rows / Gram matrix
+        aux,             // result-side kernels: row mask / per-column sums / checksum / bit rows / Gram matrix
+        scm,             // grmkm_scm_run: masks, bests, blacklist bits, per-CTA bests, selections
+        scm_list;        // grmkm_scm_run: the tie list and the statistics of its rules
     uint64_t racc_hint = 0;        // records of the previous abundance build + headroom
     uint32_t pack_ctas[2] = {0, 0};      // resident CTAs of the persistent k_pack (FASTA / FASTQ)
     std::vector<uint64_t> merge_h_off;   // row-block merge of a partial build: chunk offsets of the merge buckets
@@ -121,6 +124,7 @@ struct grmkm_ctx {
     uint64_t pitch = 0;            // u64 words between two word rows of `matrix` (>= U: the ordered emission writes every row at
                                    // the stride of its capacity guess, because U is only known when the last bucket is done)
     uint32_t W = 0, G = 0;
+    bool slice = false;            // the result is one owner's slice of a multi-GPU merge (grmkm_merge_partials, n_ranks > 1)
     grmkm_stats stats{};
     grmkm_times times{};
 
@@ -132,6 +136,10 @@ struct grmkm_ctx {
     uint32_t part_words = 0;
     uint32_t cur_bucket_bits = 0;
     int32_t xrank = -1;                  // this context's rank in the exchange (grmkm_set_exchange_rank); -1: the device index
+
+    // grmkm_scm_run results: per fit, its steps and their equivalent rules
+    std::vector<std::vector<grmkm_scm_step>> scm_steps;
+    std::vector<std::vector<uint64_t>> scm_equiv;
 };
 
 namespace {
@@ -1281,6 +1289,8 @@ static int build_impl(grmkm_ctx* c, uint32_t mode /*0 final, 1 partial*/, uint32
 // side-stream clear is counted on
 static int build_guarded(grmkm_ctx* c, uint32_t mode, uint32_t n_ranges) {
     NvtxRange nv(mode == 0 ? "grmkm_build" : "grmkm_build_partial");
+    c->slice = false;
+    c->scm_steps.clear(); c->scm_equiv.clear();
     const int r = build_impl(c, mode, n_ranges);
     if (r != GRMKM_OK) {
         const std::string msg = c->err;
@@ -1371,7 +1381,7 @@ void grmkm_destroy(grmkm_ctx* c) {
                      &c->fss, &c->codes, &c->valid, &c->hist, &c->offsets, &c->offsets2,
                      &c->bcounts, &c->ukeys, &c->uwords, &c->kmers, &c->matrix, &c->scalars, &c->fmt, &c->synth, &c->refs,
                      &c->stile_file, &c->bbase, &c->apub, &c->masks, &c->units, &c->ucur, &c->ubeg, &c->wu, &c->wide,
-                     &c->racc, &c->aux};
+                     &c->racc, &c->aux, &c->scm, &c->scm_list};
     for (DevBuf* b : all) release(c, *b);
     if (c->ev_ok) for (int i = 0; i < T_N; ++i) cudaEventDestroy(c->ev[i]);
     if (c->host_res) cudaFreeHost(c->host_res);
@@ -1397,6 +1407,8 @@ int grmkm_reset(grmkm_ctx* c) {
     c->built = false;
     c->U = 0; c->W = 0; c->G = 0;
     c->part_ranks = 0;
+    c->slice = false;
+    c->scm_steps.clear(); c->scm_equiv.clear();
     return GRMKM_OK;
 }
 
@@ -1864,7 +1876,10 @@ int grmkm_merge_partials(grmkm_ctx* c, const void* dev_parts, uint32_t n_ranks, 
         return fail(c, GRMKM_E_INVALID, "grmkm_merge_partials needs the bucket count the partial builds agreed on (grmkm_set_bucket_bits)");
     const uint32_t ob = n_ranks > 1 ? std::min(kUnitMaxBucketBits, c->cfg.bucket_bits) : 0u;
     const uint64_t own_lo = ((1ULL << ob) * rank) / n_ranks, own_hi = ((1ULL << ob) * (rank + 1)) / n_ranks;
-    return merge_sources(c, dev_parts, n_ranks, src_counts, src_words, total_genomes, ob, own_lo, own_hi, n_ranks, false, false);
+    c->scm_steps.clear(); c->scm_equiv.clear();
+    const int r = merge_sources(c, dev_parts, n_ranks, src_counts, src_words, total_genomes, ob, own_lo, own_hi, n_ranks, false, false);
+    c->slice = r == GRMKM_OK && n_ranks > 1;
+    return r;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1969,6 +1984,264 @@ int grmkm_tsv_pack(grmkm_ctx* c, const uint8_t* body, uint64_t n_rows, uint32_t 
     CU_TRY(c, cudaMemcpyAsync(&bad, d_bad, 4, cudaMemcpyDeviceToHost, st));
     CU_TRY(c, cudaStreamSynchronize(st));
     if (bad) return fail(c, GRMKM_E_INVALID, "the k-mer matrix is not binary (cells must be 0 or 1)");
+    return GRMKM_OK;
+}
+
+int grmkm_load_result(grmkm_ctx* c, const uint64_t* kmers, const uint64_t* matrix, uint64_t n_kmers, uint32_t n_genomes) {
+    if (check_ctx(c)) return GRMKM_E_INVALID;
+    if (n_genomes > kMaxGenomes) return fail(c, GRMKM_E_UNSUPPORTED, "at most 32768 genomes in one context");
+    const uint32_t W = (n_genomes + 63) / 64;
+    if (n_kmers && (!kmers || (W && !matrix))) return fail(c, GRMKM_E_INVALID, "null kmers or matrix");
+    if (n_genomes % 64 && n_kmers) {
+        const uint64_t beyond = ~0ULL >> (n_genomes % 64);     // bits of rows n_genomes .. 64 W - 1 in the last word row
+        const uint64_t* last = matrix + (uint64_t)(W - 1) * n_kmers;
+        for (uint64_t j = 0; j < n_kmers; ++j)
+            if (last[j] & beyond) return fail(c, GRMKM_E_INVALID, "the matrix has set bits at rows >= n_genomes");
+    }
+    CU_TRY(c, cudaSetDevice(c->device));
+    if (c->aux_stream) CU_TRY(c, cudaStreamSynchronize(c->aux_stream));
+    c->built = false;
+    ENSURE(c, c->kmers, n_kmers * 8);
+    ENSURE(c, c->matrix, n_kmers * W * 8);
+    if (n_kmers) {
+        CU_TRY(c, cudaMemcpyAsync(c->kmers.p, kmers, n_kmers * 8, cudaMemcpyHostToDevice, c->stream));
+        if (W) CU_TRY(c, cudaMemcpyAsync(c->matrix.p, matrix, n_kmers * W * 8, cudaMemcpyHostToDevice, c->stream));
+        CU_TRY(c, cudaStreamSynchronize(c->stream));
+    }
+    c->U = n_kmers; c->W = W; c->G = n_genomes; c->pitch = n_kmers;
+    c->built = true; c->slice = false; c->part_ranks = 0;
+    c->scm_steps.clear(); c->scm_equiv.clear();
+    c->stats = grmkm_stats{};
+    c->stats.n_kmers = c->stats.n_distinct = n_kmers;
+    c->stats.n_words = W; c->stats.n_genomes = n_genomes;
+    c->stats.h2d_bytes = n_kmers * (W + 1) * 8;
+    c->times = grmkm_times{};
+    return GRMKM_OK;
+}
+
+}  // extern "C"
+
+namespace {
+
+double scm_unkey(uint64_t k) {
+    const uint64_t b = (k >> 63) ? (k & ~(1ULL << 63)) : ~k;
+    double u;
+    memcpy(&u, &b, 8);
+    return u;
+}
+
+template <bool CACHED>
+int scm_launch_chunk(grmkm_ctx* c, const ScmFitArg* d_args, uint32_t n, const uint32_t* d_bl, const unsigned long long* d_masks,
+                     unsigned long long* d_best, unsigned long long* d_tile, unsigned long long* d_list,
+                     unsigned long long* d_count, uint64_t cap) {
+    const size_t smem = scm_smem_bytes(n, c->W);
+    CU_TRY(c, cudaFuncSetAttribute(k_scm_scan<CACHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CU_TRY(c, cudaFuncSetAttribute(k_scm_ties<CACHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int occ = 0;
+    CU_TRY(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_scm_scan<CACHED>, kScmThreads, smem));
+    const uint64_t n_tiles = (c->U + kScmThreads - 1) / kScmThreads;
+    const uint32_t grid = (uint32_t)std::min<uint64_t>(n_tiles, (uint64_t)c->sm_count * std::max(1, occ));
+    const unsigned long long* m = (const unsigned long long*)c->matrix.p;
+    k_scm_scan<CACHED><<<grid, kScmThreads, smem, c->stream>>>(m, c->U, c->pitch, c->W, d_bl, d_args, n, d_masks, d_best, d_tile);
+    k_scm_ties<CACHED><<<grid, kScmThreads, smem, c->stream>>>(m, c->U, c->pitch, c->W, d_bl, d_args, n, d_masks, d_best, d_tile,
+                                                               d_list, d_count, cap);
+    CU_TRY(c, cudaGetLastError());
+    c->stats.n_launches += 2;
+    return GRMKM_OK;
+}
+
+int scm_check_mask(grmkm_ctx* c, const uint64_t* m, const char* what) {
+    if (!m) return fail(c, GRMKM_E_INVALID, std::string("null ") + what + " mask");
+    if (c->G % 64 && (m[c->W - 1] & (~0ULL >> (c->G % 64))))
+        return fail(c, GRMKM_E_INVALID, std::string("the ") + what + " mask has bits at rows >= n_genomes");
+    return GRMKM_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int grmkm_scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, const uint64_t* blacklist, uint64_t n_blacklist) {
+    if (check_ctx(c)) return GRMKM_E_INVALID;
+    if (!c->built) return fail(c, GRMKM_E_INVALID, "no result: call grmkm_build or grmkm_load_result first");
+    if (c->slice)
+        return fail(c, GRMKM_E_UNSUPPORTED, "the result is one owner's slice of a multi-GPU build: its best rule is not the answer");
+    const uint64_t U = c->U;
+    const uint32_t W = c->W;
+    if (U >= (1ULL << 31)) return fail(c, GRMKM_E_UNSUPPORTED, "the SCM indexes rules with 32 bits: at most 2^31 - 1 k-mers");
+    if (n_fits && !jobs) return fail(c, GRMKM_E_INVALID, "null jobs");
+    if (n_blacklist && !blacklist) return fail(c, GRMKM_E_INVALID, "null blacklist");
+    for (uint32_t f = 0; f < n_fits; ++f) {
+        const grmkm_scm_job& j = jobs[f];
+        const std::string at = " (fit " + std::to_string(f) + ")";
+        if (j.struct_size != sizeof(grmkm_scm_job)) return fail(c, GRMKM_E_INVALID, "job struct_size is not sizeof(grmkm_scm_job)" + at);
+        if (j.model_type > GRMKM_SCM_DISJUNCTION) return fail(c, GRMKM_E_INVALID, "unknown model type" + at);
+        if (j.max_rules == 0) return fail(c, GRMKM_E_INVALID, "max_rules must be at least 1" + at);
+        if (j.tiebreak > 1) return fail(c, GRMKM_E_INVALID, "tiebreak must be 0 or 1" + at);
+        if (!(j.p >= 0.0) || j.p > 1.7976931348623157e308) return fail(c, GRMKM_E_INVALID, "p must be finite and >= 0" + at);
+        if (W) {
+            int r = scm_check_mask(c, j.pos, "positive");
+            if (!r) r = scm_check_mask(c, j.neg, "negative");
+            if (r) return r;
+            for (uint32_t w = 0; w < W; ++w)
+                if (j.pos[w] & j.neg[w]) return fail(c, GRMKM_E_INVALID, "positive and negative examples overlap" + at);
+        }
+    }
+    for (uint64_t i = 0; i < n_blacklist; ++i)
+        if (blacklist[i] >= 2 * U) return fail(c, GRMKM_E_INVALID, "blacklisted rule index >= 2 x n_kmers");
+
+    NvtxRange nv("grmkm_scm_run");
+    c->scm_steps.assign(n_fits, {});
+    c->scm_equiv.assign(n_fits, {});
+    std::vector<uint32_t> n_pos(n_fits), n_neg(n_fits), n_rules(n_fits, 0);
+    std::vector<char> done(n_fits, 0);
+    std::vector<uint64_t> h_masks((size_t)n_fits * 4 * W);
+    for (uint32_t f = 0; f < n_fits; ++f) {
+        const bool swap = jobs[f].model_type == GRMKM_SCM_DISJUNCTION;
+        const uint64_t* P0 = swap ? jobs[f].neg : jobs[f].pos;
+        const uint64_t* N0 = swap ? jobs[f].pos : jobs[f].neg;
+        uint32_t np = 0, nn = 0;
+        for (uint32_t w = 0; w < W; ++w) {
+            uint64_t* m = h_masks.data() + (size_t)f * 4 * W;
+            m[w] = m[2 * W + w] = P0[w];
+            m[W + w] = m[3 * W + w] = N0[w];
+            np += (uint32_t)__builtin_popcountll(P0[w]);
+            nn += (uint32_t)__builtin_popcountll(N0[w]);
+        }
+        n_pos[f] = np; n_neg[f] = nn;
+        done[f] = nn == 0 || U == 0;          // nothing to cover, or no rule at all
+    }
+    if (std::find(done.begin(), done.end(), 0) == done.end()) return GRMKM_OK;
+
+    CU_TRY(c, cudaSetDevice(c->device));
+    // chunk = fits whose masks share one CTA's shared memory; small enough for two CTAs per SM
+    const size_t smem_cap = (c->smem_optin ? c->smem_optin : 227 * 1024) - 1024;
+    const size_t per_fit = scm_smem_bytes(1, W);
+    const uint32_t chunk = (uint32_t)std::max<size_t>(1, std::min<size_t>(smem_cap / 2, 64 * 1024) / per_fit);
+    const uint64_t bl_words = (2 * U + 31) / 32;
+    const uint64_t max_grid = (uint64_t)c->sm_count * 8;
+    auto al = [](size_t b) { return (b + 255) & ~size_t(255); };
+    const size_t o_masks = 0, o_best = o_masks + al(h_masks.size() * 8), o_args = o_best + al((size_t)n_fits * 8),
+                 o_bl = o_args + al((size_t)n_fits * sizeof(ScmFitArg)), o_tile = o_bl + al(bl_words * 4),
+                 o_sel = o_tile + al((size_t)chunk * max_grid * 8), o_count = o_sel + al((size_t)n_fits * 8),
+                 total = o_count + 256;
+    ENSURE(c, c->scm, total);
+    uint8_t* base = (uint8_t*)c->scm.p;
+    unsigned long long* d_masks = (unsigned long long*)(base + o_masks);
+    unsigned long long* d_best = (unsigned long long*)(base + o_best);
+    ScmFitArg* d_args = (ScmFitArg*)(base + o_args);
+    uint32_t* d_bl = (uint32_t*)(base + o_bl);
+    unsigned long long* d_tile = (unsigned long long*)(base + o_tile);
+    unsigned long long* d_sel = (unsigned long long*)(base + o_sel);
+    unsigned long long* d_count = (unsigned long long*)(base + o_count);
+    std::vector<uint32_t> h_bl(bl_words, 0);
+    for (uint64_t i = 0; i < n_blacklist; ++i) h_bl[blacklist[i] >> 5] |= 1u << (blacklist[i] & 31);
+    CU_TRY(c, cudaMemcpyAsync(d_masks, h_masks.data(), h_masks.size() * 8, cudaMemcpyHostToDevice, c->stream));
+    CU_TRY(c, cudaMemcpyAsync(d_bl, h_bl.data(), bl_words * 4, cudaMemcpyHostToDevice, c->stream));
+
+    uint64_t cap = std::max<uint64_t>(1024, c->scm_list.cap / 20);      // tie list entries (8 bytes + 3 x 4 bytes of statistics)
+    std::vector<ScmFitArg> args;
+    std::vector<uint64_t> h_list, h_best(n_fits), sel;
+    std::vector<uint32_t> h_stats;
+    std::vector<size_t> order;
+    for (;;) {
+        args.clear();
+        for (uint32_t f = 0; f < n_fits; ++f)
+            if (!done[f]) args.push_back(ScmFitArg{jobs[f].p, f, n_pos[f], n_neg[f], 0});
+        if (args.empty()) break;
+        ENSURE(c, c->scm_list, cap * 20);
+        unsigned long long* d_list = (unsigned long long*)c->scm_list.p;
+        uint32_t* d_stats = (uint32_t*)(d_list + cap);
+        CU_TRY(c, cudaMemcpyAsync(d_args, args.data(), args.size() * sizeof(ScmFitArg), cudaMemcpyHostToDevice, c->stream));
+        CU_TRY(c, cudaMemsetAsync(d_best, 0, (size_t)n_fits * 8, c->stream));
+        CU_TRY(c, cudaMemsetAsync(d_count, 0, 8, c->stream));
+        for (size_t a0 = 0; a0 < args.size(); a0 += chunk) {
+            const uint32_t n = (uint32_t)std::min<size_t>(chunk, args.size() - a0);
+            const int r = W <= kScmCachedWords
+                              ? scm_launch_chunk<true>(c, d_args + a0, n, d_bl, d_masks, d_best, d_tile, d_list, d_count, cap)
+                              : scm_launch_chunk<false>(c, d_args + a0, n, d_bl, d_masks, d_best, d_tile, d_list, d_count, cap);
+            if (r) return r;
+        }
+        uint64_t count = 0;
+        CU_TRY(c, cudaMemcpyAsync(&count, d_count, 8, cudaMemcpyDeviceToHost, c->stream));
+        CU_TRY(c, cudaStreamSynchronize(c->stream));
+        if (count > cap) {              // the tie list overflowed: grow it and redo the step (nothing was updated)
+            cap = count + count / 4;
+            continue;
+        }
+        if (count) {
+            k_scm_gather<<<(uint32_t)std::min<uint64_t>((count + 255) / 256, (uint64_t)c->sm_count * 16), 256, 0, c->stream>>>(
+                (const unsigned long long*)c->matrix.p, U, c->pitch, W, d_masks, d_list, count, d_stats);
+            CU_TRY(c, cudaGetLastError());
+            c->stats.n_launches++;
+        }
+        h_list.resize(count); h_stats.resize(count * 3);
+        CU_TRY(c, cudaMemcpyAsync(h_list.data(), d_list, count * 8, cudaMemcpyDeviceToHost, c->stream));
+        CU_TRY(c, cudaMemcpyAsync(h_stats.data(), d_stats, count * 12, cudaMemcpyDeviceToHost, c->stream));
+        CU_TRY(c, cudaMemcpyAsync(h_best.data(), d_best, (size_t)n_fits * 8, cudaMemcpyDeviceToHost, c->stream));
+        CU_TRY(c, cudaStreamSynchronize(c->stream));
+        // the list comes in the order of the atomics: sort it by (fit, rule)
+        order.resize(count);
+        for (size_t i = 0; i < count; ++i) order[i] = i;
+        std::sort(order.begin(), order.end(), [&](size_t a, size_t b) { return h_list[a] < h_list[b]; });
+        sel.clear();
+        size_t i = 0;
+        for (const ScmFitArg& a : args) {
+            const uint32_t f = a.fit;
+            while (i < count && (h_list[order[i]] >> 32) < f) ++i;
+            size_t end = i;
+            while (end < count && (h_list[order[end]] >> 32) == f) ++end;
+            if (end == i) { done[f] = 1; continue; }        // no rule changes anything at u*, or every rule is blacklisted
+            uint32_t min_risk = UINT32_MAX;
+            if (jobs[f].tiebreak)
+                for (size_t t = i; t < end; ++t) min_risk = std::min(min_risk, h_stats[3 * order[t] + 2]);
+            std::vector<uint64_t>& eq = c->scm_equiv[f];
+            grmkm_scm_step st{};
+            st.utility = scm_unkey(h_best[f]);
+            st.equiv_offset = eq.size();
+            for (size_t t = i; t < end; ++t) {
+                const size_t o = order[t];
+                if (jobs[f].tiebreak && h_stats[3 * o + 2] != min_risk) continue;
+                if (eq.size() == st.equiv_offset) {
+                    st.rule = h_list[o] & 0xffffffffULL;
+                    st.positive_errors = h_stats[3 * o];
+                    st.negative_covers = h_stats[3 * o + 1];
+                }
+                eq.push_back(h_list[o] & 0xffffffffULL);
+            }
+            st.equiv_count = eq.size() - st.equiv_offset;
+            c->scm_steps[f].push_back(st);
+            n_pos[f] -= st.positive_errors;
+            n_neg[f] -= st.negative_covers;
+            if (n_neg[f] == 0 || ++n_rules[f] == jobs[f].max_rules) done[f] = 1;
+            sel.push_back(((uint64_t)f << 32) | st.rule);
+            i = end;
+        }
+        if (!sel.empty()) {
+            CU_TRY(c, cudaMemcpyAsync(d_sel, sel.data(), sel.size() * 8, cudaMemcpyHostToDevice, c->stream));
+            const uint64_t nw = (uint64_t)sel.size() * W;
+            k_scm_update<<<(uint32_t)std::min<uint64_t>((nw + 255) / 256, (uint64_t)c->sm_count * 8), 256, 0, c->stream>>>(
+                (const unsigned long long*)c->matrix.p, U, c->pitch, W, d_sel, (uint32_t)sel.size(), d_masks);
+            CU_TRY(c, cudaGetLastError());
+            c->stats.n_launches++;
+        }
+    }
+    CU_TRY(c, cudaStreamSynchronize(c->stream));
+    return GRMKM_OK;
+}
+
+int grmkm_scm_result(grmkm_ctx* c, uint32_t fit, grmkm_scm_step* steps, uint64_t steps_cap, uint64_t* n_steps,
+                     uint64_t* equivalent, uint64_t equiv_cap, uint64_t* n_equivalent) {
+    if (check_ctx(c)) return GRMKM_E_INVALID;
+    if (fit >= c->scm_steps.size()) return fail(c, GRMKM_E_INVALID, "no such fit in the last grmkm_scm_run");
+    const std::vector<grmkm_scm_step>& s = c->scm_steps[fit];
+    const std::vector<uint64_t>& e = c->scm_equiv[fit];
+    if (n_steps) *n_steps = s.size();
+    if (n_equivalent) *n_equivalent = e.size();
+    if ((!steps && !s.empty()) || steps_cap < s.size() || (!equivalent && !e.empty()) || equiv_cap < e.size())
+        return fail(c, GRMKM_E_CAPACITY, "scm result buffers too small");
+    if (!s.empty()) memcpy(steps, s.data(), s.size() * sizeof(grmkm_scm_step));
+    if (!e.empty()) memcpy(equivalent, e.data(), e.size() * 8);
     return GRMKM_OK;
 }
 

@@ -37,6 +37,7 @@ class KmerRuleClassifications:
         U, W, _ = builder.dims
         self._U, self._W = int(U), int(W)
         self._matrix = None
+        self._kmers = None                 # packed k-mers, fetched once the SCM names a rule (scm.fit_many)
 
     # -- row bookkeeping (rules.py:171-199): rows are numbered among the rows not removed yet ------------
     def _absolute_rows(self, rows) -> list[int]:
@@ -85,3 +86,30 @@ class KmerRuleClassifications:
         result = _unpack_binary_bytes_from_ints(self._matrix[:, cols])[row_mask]
         result[:, invert] = 1 - result[:, invert]
         return result.reshape(-1) if columns_is_int else result
+
+
+_BASE_CODE = np.full(256, 255, dtype=np.uint64)
+for _i, _b in enumerate(b"ACTG"):                       # the library's packing: A0 C1 T2 G3, first base most significant
+    _BASE_CODE[_b] = _i
+
+
+def load_kover(path: str, builder) -> KmerRuleClassifications:
+    """The k-mer matrix of a ``.kover`` dataset made the resident result of ``builder`` (a KmerMatrixBuilder whose k is
+    the dataset's k-mer length), for learning from an existing file.  Reads ``kmer_matrix``, ``kmer_sequences`` and
+    ``genome_identifiers`` with hdf5min."""
+    from . import hdf5min
+    r = hdf5min.H5Reader(path)
+    matrix = r["kmer_matrix"].read()
+    seqs = r["kmer_sequences"].read()
+    n_genomes = len(r["genome_identifiers"].read())
+    k = seqs.dtype.itemsize
+    if len(seqs) and k != builder.k:
+        raise ValueError(f"{path} holds {k}-mers, the builder counts {builder.k}-mers")
+    codes = _BASE_CODE[np.frombuffer(seqs.tobytes(), dtype=np.uint8).reshape(len(seqs), k)]
+    if (codes == 255).any():
+        raise ValueError(f"{path}: kmer_sequences holds a character other than A, C, G, T")
+    kmers = np.zeros(len(seqs), dtype=np.uint64)
+    for i in range(k):
+        kmers = (kmers << np.uint64(2)) | codes[:, i]
+    builder.load_result(kmers, matrix, n_genomes)
+    return KmerRuleClassifications(builder, n_genomes)

@@ -6,7 +6,7 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("GRMKM_LIB") or os.path.join(_HERE, "libgrmkm.so")   # GRMKM_LIB: another build of the same library (kernel experiments)
-ABI_VERSION = 10
+ABI_VERSION = 11
 
 OK = 0
 E_INVALID, E_UNSUPPORTED_K, E_NOMEM, E_CUDA, E_IO, E_CAPACITY, E_NO_DEVICE, E_UNSUPPORTED = -1, -2, -3, -4, -5, -6, -7, -8
@@ -22,7 +22,9 @@ SYMBOLS = [
     "grmkm_synth_fasta_device", "grmkm_build_partial", "grmkm_export_partials", "grmkm_export_partials_peers", "grmkm_merge_partials",
     "grmkm_plan_bucket_bits", "grmkm_set_bucket_bits", "grmkm_set_exchange_rank",
     "grmkm_result_checksum", "grmkm_sum_rows", "grmkm_gram", "grmkm_tsv_pack",
+    "grmkm_load_result", "grmkm_scm_run", "grmkm_scm_result",
 ]
+SCM_CONJUNCTION, SCM_DISJUNCTION = 0, 1
 
 
 class GrmkmError(RuntimeError):
@@ -56,6 +58,16 @@ class Times(C.Structure):
 
     def asdict(self):
         return {n: float(getattr(self, n)) for n, _ in self._fields_}
+
+
+class ScmJob(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("model_type", C.c_uint32), ("max_rules", C.c_uint32),
+                ("tiebreak", C.c_uint32), ("p", C.c_double), ("pos", C.c_void_p), ("neg", C.c_void_p)]
+
+
+class ScmStep(C.Structure):
+    _fields_ = [("rule", C.c_uint64), ("utility", C.c_double), ("positive_errors", C.c_uint32),
+                ("negative_covers", C.c_uint32), ("equiv_offset", C.c_uint64), ("equiv_count", C.c_uint64)]
 
 
 _lib = None
@@ -105,6 +117,9 @@ def load() -> C.CDLL:
         "grmkm_sum_rows": (i32, [vp, vp, u32, vp, u64]),
         "grmkm_gram": (i32, [vp, vp, u64]),
         "grmkm_tsv_pack": (i32, [vp, vp, u64, u32, u32, u32, u32, vp, vp, u64]),
+        "grmkm_load_result": (i32, [vp, vp, vp, u64, u32]),
+        "grmkm_scm_run": (i32, [vp, u32, vp, vp, u64]),
+        "grmkm_scm_result": (i32, [vp, u32, vp, u64, C.POINTER(u64), vp, u64, C.POINTER(u64)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)

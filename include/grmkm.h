@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define GRMKM_ABI_VERSION 10
+#define GRMKM_ABI_VERSION 11
 
 enum {
     GRMKM_OK = 0,
@@ -241,6 +241,53 @@ int grmkm_export_partials_peers(grmkm_ctx* ctx, uint32_t n_ranks, void* const* p
 int grmkm_set_exchange_rank(grmkm_ctx* ctx, uint32_t rank);
 int grmkm_merge_partials(grmkm_ctx* ctx, const void* dev_parts, uint32_t n_ranks, uint32_t rank,
                          const uint64_t* src_counts, const uint32_t* src_words, uint32_t total_genomes);
+
+/*
+ * An existing matrix as the context's result (a .kover file's kmer_matrix and its k-mers): kmers[n_kmers] packed as
+ * grmkm_copy_kmers_packed returns them, matrix row-major ceil(n_genomes / 64) x n_kmers (host memory).  Every result-side
+ * call then works on it as on a build.  Set bits at rows >= n_genomes: GRMKM_E_INVALID; n_genomes > 32768:
+ * GRMKM_E_UNSUPPORTED.
+ */
+int grmkm_load_result(grmkm_ctx* ctx, const uint64_t* kmers, const uint64_t* matrix, uint64_t n_kmers, uint32_t n_genomes);
+
+/*
+ * Set Covering Machine (kover learning/learners/scm.py) on the resident matrix, many fits at once.  Rule r < U is
+ * "k-mer r present", rule U + r its absence twin.  Per fit (disjunction: P0 and N0 swapped first), P = P0, N = N0;
+ * while |N| > 0 and fewer than max_rules rules: over the rules not blacklisted, e = #P examples the rule outputs 0 on,
+ * c = #N examples it outputs 0 on, u = (double)c - p * (double)e (product rounded, then difference); u* = max u;
+ * T = {u == u*, c > 0 or e > 0} (empty: stop); tiebreak: keep the T members of least risk (#P0 outputs 0 + #N0
+ * outputs 1); the rule is min T; P and N keep the examples it outputs 1 on.  Every greedy step of all fits is one
+ * pass over the matrix on the device; only the steps and the sets T cross PCIe.
+ */
+enum { GRMKM_SCM_CONJUNCTION = 0, GRMKM_SCM_DISJUNCTION = 1 };
+
+typedef struct grmkm_scm_job {
+    uint32_t struct_size;  /* = sizeof(grmkm_scm_job) */
+    uint32_t model_type;   /* GRMKM_SCM_CONJUNCTION / GRMKM_SCM_DISJUNCTION */
+    uint32_t max_rules;    /* >= 1 */
+    uint32_t tiebreak;     /* 1: risk tiebreaker (experiment_scm.py), 0: none */
+    double p;              /* >= 0, finite */
+    const uint64_t* pos;   /* P0: n_words words, genome g at bit 63 - g % 64 of word g / 64 */
+    const uint64_t* neg;   /* N0: disjoint from P0 */
+} grmkm_scm_job;
+
+typedef struct grmkm_scm_step {
+    uint64_t rule;             /* < 2U */
+    double utility;            /* u* */
+    uint32_t positive_errors;  /* e of the rule */
+    uint32_t negative_covers;  /* c of the rule */
+    uint64_t equiv_offset;     /* T of this step: equivalent[equiv_offset .. + equiv_count), ascending */
+    uint64_t equiv_count;
+} grmkm_scm_step;
+
+/* Runs every fit to completion; the results stay in the context until the next run / build / load / reset.  Refuses
+ * (GRMKM_E_UNSUPPORTED) a result that is one owner's slice of a multi-GPU merge. */
+int grmkm_scm_run(grmkm_ctx* ctx, uint32_t n_fits, const grmkm_scm_job* jobs, const uint64_t* blacklist,
+                  uint64_t n_blacklist);
+/* Steps and equivalent rules of fit `fit`.  *n_steps / *n_equivalent receive the sizes; NULL or short buffers:
+ * GRMKM_E_CAPACITY (sizes still written). */
+int grmkm_scm_result(grmkm_ctx* ctx, uint32_t fit, grmkm_scm_step* steps, uint64_t steps_cap, uint64_t* n_steps,
+                     uint64_t* equivalent, uint64_t equiv_cap, uint64_t* n_equivalent);
 
 #ifdef __cplusplus
 }
