@@ -249,6 +249,40 @@ class KmerMatrixBuilder:
             out.append((steps, eq))
         return out
 
+    CART_NODE_DTYPE = np.dtype([("rule", np.uint64), ("score", np.float64), ("depth", np.uint32), ("n_pos", np.uint32),
+                                ("n_neg", np.uint32), ("present_child", np.uint32), ("absent_child", np.uint32),
+                                ("prediction", np.uint32), ("equiv_offset", np.uint64), ("equiv_count", np.uint64),
+                                ("equiv_total", np.uint64)])
+
+    def cart_run(self, jobs, blacklist=()) -> list[tuple[np.ndarray, np.ndarray]]:
+        """CART trees on the resident matrix, all in one grmkm_cart_run.  jobs: (max_depth, min_samples_split,
+        equiv_cap, w_neg, w_pos, pos_mask, neg_mask) with masks of ceil(G/64) uint64 words.  -> per tree (nodes,
+        equivalent rules): nodes is a structured array with the fields of grmkm_cart_node, in breadth-first order."""
+        _, W, _ = self.dims
+        masks, arr = [], (native.CartJob * max(1, len(jobs)))()
+        for i, (max_depth, min_samples_split, equiv_cap, w_neg, w_pos, pos, neg) in enumerate(jobs):
+            pos = np.ascontiguousarray(pos, dtype=np.uint64)
+            neg = np.ascontiguousarray(neg, dtype=np.uint64)
+            if pos.shape != (W,) or neg.shape != (W,):
+                raise ValueError(f"example masks of {pos.shape} / {neg.shape} words for {W} matrix word rows")
+            masks += [pos, neg]
+            arr[i] = native.CartJob(C.sizeof(native.CartJob), int(max_depth), int(min_samples_split), 0, int(equiv_cap),
+                                    float(w_neg), float(w_pos), pos.ctypes.data, neg.ctypes.data)
+        bl = np.ascontiguousarray(blacklist if blacklist is not None else (), dtype=np.uint64).reshape(-1)
+        self._check(self._lib.grmkm_cart_run(self._ctx, len(jobs), arr, C.c_void_p(bl.ctypes.data), bl.size))
+        out = []
+        for t in range(len(jobs)):
+            nn, ne = C.c_uint64(), C.c_uint64()
+            rc = self._lib.grmkm_cart_result(self._ctx, t, None, 0, C.byref(nn), None, 0, C.byref(ne))
+            if rc not in (native.OK, native.E_CAPACITY):
+                self._check(rc)
+            nodes = np.zeros(nn.value, dtype=self.CART_NODE_DTYPE)
+            eq = np.zeros(ne.value, dtype=np.uint64)
+            self._check(self._lib.grmkm_cart_result(self._ctx, t, C.c_void_p(nodes.ctypes.data), nodes.size, C.byref(nn),
+                                                    C.c_void_p(eq.ctypes.data), eq.size, C.byref(ne)))
+            out.append((nodes, eq))
+        return out
+
     def device_result(self) -> tuple[int, int, int]:
         """(device pointer of kmers[U], device pointer of the matrix, row pitch in words): word row w of the matrix
         starts at pointer + 8 * w * pitch."""

@@ -6,6 +6,7 @@
 #include "grmkm_result.cuh"
 #include "grmkm_synth.cuh"
 #include "grmkm_scm.cuh"
+#include "grmkm_cart.cuh"
 
 #include <nvtx3/nvToolsExt.h>      // header-only; the ranges cost nothing until a tool (nsys, ncu --nvtx) attaches
 #include <zlib.h>
@@ -15,6 +16,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <functional>
+#include <map>
 #include <mutex>
 #include <string>
 #include <vector>
@@ -98,7 +100,11 @@ struct grmkm_ctx {
         racc,            // abundance builds: the solid presence records of the rounds done so far
         aux,             // result-side kernels: row mask / per-column sums / checksum / bit rows / Gram matrix
         scm,             // grmkm_scm_run: masks, bests, blacklist bits, per-CTA bests, selections
-        scm_list;        // grmkm_scm_run: the tie list and the statistics of its rules
+        scm_list,        // grmkm_scm_run: the tie list and the statistics of its rules
+        cart,            // grmkm_cart_run: per-level node arguments, bests, tie totals, per-CTA bests and tie counts, splits
+        cart_bl,         // grmkm_cart_run: blacklist bits (one per k-mer)
+        cart_masks[2],   // grmkm_cart_run: P and N of the open nodes of this level / of the next level
+        cart_list;       // grmkm_cart_run: the tie list
     uint64_t racc_hint = 0;        // records of the previous abundance build + headroom
     uint32_t pack_ctas[2] = {0, 0};      // resident CTAs of the persistent k_pack (FASTA / FASTQ)
     std::vector<uint64_t> merge_h_off;   // row-block merge of a partial build: chunk offsets of the merge buckets
@@ -140,6 +146,9 @@ struct grmkm_ctx {
     // grmkm_scm_run results: per fit, its steps and their equivalent rules
     std::vector<std::vector<grmkm_scm_step>> scm_steps;
     std::vector<std::vector<uint64_t>> scm_equiv;
+    // grmkm_cart_run results: per tree, its nodes and their recorded equivalent rules
+    std::vector<std::vector<grmkm_cart_node>> cart_nodes;
+    std::vector<std::vector<uint64_t>> cart_equiv;
 };
 
 namespace {
@@ -1291,6 +1300,7 @@ static int build_guarded(grmkm_ctx* c, uint32_t mode, uint32_t n_ranges) {
     NvtxRange nv(mode == 0 ? "grmkm_build" : "grmkm_build_partial");
     c->slice = false;
     c->scm_steps.clear(); c->scm_equiv.clear();
+    c->cart_nodes.clear(); c->cart_equiv.clear();
     const int r = build_impl(c, mode, n_ranges);
     if (r != GRMKM_OK) {
         const std::string msg = c->err;
@@ -1381,7 +1391,8 @@ void grmkm_destroy(grmkm_ctx* c) {
                      &c->fss, &c->codes, &c->valid, &c->hist, &c->offsets, &c->offsets2,
                      &c->bcounts, &c->ukeys, &c->uwords, &c->kmers, &c->matrix, &c->scalars, &c->fmt, &c->synth, &c->refs,
                      &c->stile_file, &c->bbase, &c->apub, &c->masks, &c->units, &c->ucur, &c->ubeg, &c->wu, &c->wide,
-                     &c->racc, &c->aux, &c->scm, &c->scm_list};
+                     &c->racc, &c->aux, &c->scm, &c->scm_list, &c->cart, &c->cart_bl,
+                     &c->cart_masks[0], &c->cart_masks[1], &c->cart_list};
     for (DevBuf* b : all) release(c, *b);
     if (c->ev_ok) for (int i = 0; i < T_N; ++i) cudaEventDestroy(c->ev[i]);
     if (c->host_res) cudaFreeHost(c->host_res);
@@ -1409,6 +1420,7 @@ int grmkm_reset(grmkm_ctx* c) {
     c->part_ranks = 0;
     c->slice = false;
     c->scm_steps.clear(); c->scm_equiv.clear();
+    c->cart_nodes.clear(); c->cart_equiv.clear();
     return GRMKM_OK;
 }
 
@@ -1877,6 +1889,7 @@ int grmkm_merge_partials(grmkm_ctx* c, const void* dev_parts, uint32_t n_ranks, 
     const uint32_t ob = n_ranks > 1 ? std::min(kUnitMaxBucketBits, c->cfg.bucket_bits) : 0u;
     const uint64_t own_lo = ((1ULL << ob) * rank) / n_ranks, own_hi = ((1ULL << ob) * (rank + 1)) / n_ranks;
     c->scm_steps.clear(); c->scm_equiv.clear();
+    c->cart_nodes.clear(); c->cart_equiv.clear();
     const int r = merge_sources(c, dev_parts, n_ranks, src_counts, src_words, total_genomes, ob, own_lo, own_hi, n_ranks, false, false);
     c->slice = r == GRMKM_OK && n_ranks > 1;
     return r;
@@ -2011,6 +2024,7 @@ int grmkm_load_result(grmkm_ctx* c, const uint64_t* kmers, const uint64_t* matri
     c->U = n_kmers; c->W = W; c->G = n_genomes; c->pitch = n_kmers;
     c->built = true; c->slice = false; c->part_ranks = 0;
     c->scm_steps.clear(); c->scm_equiv.clear();
+    c->cart_nodes.clear(); c->cart_equiv.clear();
     c->stats = grmkm_stats{};
     c->stats.n_kmers = c->stats.n_distinct = n_kmers;
     c->stats.n_words = W; c->stats.n_genomes = n_genomes;
@@ -2241,6 +2255,275 @@ int grmkm_scm_result(grmkm_ctx* c, uint32_t fit, grmkm_scm_step* steps, uint64_t
     if ((!steps && !s.empty()) || steps_cap < s.size() || (!equivalent && !e.empty()) || equiv_cap < e.size())
         return fail(c, GRMKM_E_CAPACITY, "scm result buffers too small");
     if (!s.empty()) memcpy(steps, s.data(), s.size() * sizeof(grmkm_scm_step));
+    if (!e.empty()) memcpy(equivalent, e.data(), e.size() * 8);
+    return GRMKM_OK;
+}
+
+}  // extern "C"
+
+namespace {
+
+// the largest dynamic shared memory any chunk of this run asks for, set once per run
+template <bool CACHED>
+int cart_allow_smem(grmkm_ctx* c, size_t smem) {
+    CU_TRY(c, cudaFuncSetAttribute(k_cart_scan<CACHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CU_TRY(c, cudaFuncSetAttribute(k_cart_ties<CACHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    return GRMKM_OK;
+}
+
+// the scan and both tie passes of one chunk of open nodes; CTA b covers the tiles [b tpc, (b + 1) tpc).  occ: resident
+// CTAs per SM by chunk size, filled on first use (a run sees few sizes: full chunks and the tails of its levels)
+template <bool CACHED>
+int cart_launch_chunk(grmkm_ctx* c, const CartNodeArg* d_args, uint32_t n, const uint32_t* d_bl, const unsigned long long* d_masks,
+                      unsigned long long* d_best, unsigned long long* d_tile, uint32_t* d_tcnt, unsigned long long* d_total,
+                      unsigned long long* d_list, unsigned long long* d_count, uint64_t cap, uint64_t max_grid,
+                      std::map<uint32_t, int>& occ_of) {
+    const size_t smem = cart_smem_bytes(n, c->W);
+    auto it = occ_of.find(n);
+    if (it == occ_of.end()) {
+        int occ = 0;
+        CU_TRY(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_cart_scan<CACHED>, kScmThreads, smem));
+        it = occ_of.emplace(n, occ).first;
+    }
+    const int occ = it->second;
+    const uint64_t n_tiles = (c->U + kScmThreads - 1) / kScmThreads;
+    const uint64_t grid0 = std::min<uint64_t>({n_tiles, (uint64_t)c->sm_count * std::max(1, occ), max_grid});
+    const uint64_t tpc = (n_tiles + grid0 - 1) / grid0;
+    const uint32_t grid = (uint32_t)((n_tiles + tpc - 1) / tpc);
+    const unsigned long long* m = (const unsigned long long*)c->matrix.p;
+    k_cart_scan<CACHED><<<grid, kScmThreads, smem, c->stream>>>(m, c->U, c->pitch, c->W, d_bl, d_args, n, d_masks, tpc, d_best, d_tile);
+    for (int append = 0; append < 2; ++append)
+        k_cart_ties<CACHED><<<grid, kScmThreads, smem, c->stream>>>(m, c->U, c->pitch, c->W, d_bl, d_args, n, d_masks, tpc, d_best,
+                                                                    d_tile, d_tcnt, d_total, append, d_list, d_count, cap);
+    CU_TRY(c, cudaGetLastError());
+    c->stats.n_launches += 3;
+    return GRMKM_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int grmkm_cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const uint64_t* blacklist, uint64_t n_blacklist) {
+    if (check_ctx(c)) return GRMKM_E_INVALID;
+    if (!c->built) return fail(c, GRMKM_E_INVALID, "no result: call grmkm_build or grmkm_load_result first");
+    if (c->slice)
+        return fail(c, GRMKM_E_UNSUPPORTED, "the result is one owner's slice of a multi-GPU build: its best split is not the answer");
+    const uint64_t U = c->U;
+    const uint32_t W = c->W;
+    if (U >= (1ULL << 31)) return fail(c, GRMKM_E_UNSUPPORTED, "CART indexes k-mers with 32 bits: at most 2^31 - 1 k-mers");
+    if (n_trees && !jobs) return fail(c, GRMKM_E_INVALID, "null jobs");
+    if (n_blacklist && !blacklist) return fail(c, GRMKM_E_INVALID, "null blacklist");
+    for (uint32_t t = 0; t < n_trees; ++t) {
+        const grmkm_cart_job& j = jobs[t];
+        const std::string at = " (tree " + std::to_string(t) + ")";
+        if (j.struct_size != sizeof(grmkm_cart_job)) return fail(c, GRMKM_E_INVALID, "job struct_size is not sizeof(grmkm_cart_job)" + at);
+        if (j.reserved != 0) return fail(c, GRMKM_E_INVALID, "reserved must be 0" + at);
+        if (j.max_depth == 0) return fail(c, GRMKM_E_INVALID, "max_depth must be at least 1" + at);
+        if (j.min_samples_split < 2) return fail(c, GRMKM_E_INVALID, "min_samples_split must be at least 2" + at);
+        if (!(j.w_neg > 0.0 && j.w_neg <= 1e100) || !(j.w_pos > 0.0 && j.w_pos <= 1e100))
+            return fail(c, GRMKM_E_INVALID, "class importances must be finite, > 0 and <= 1e100" + at);
+        if (W) {
+            int r = scm_check_mask(c, j.pos, "positive");
+            if (!r) r = scm_check_mask(c, j.neg, "negative");
+            if (r) return r;
+            for (uint32_t w = 0; w < W; ++w)
+                if (j.pos[w] & j.neg[w]) return fail(c, GRMKM_E_INVALID, "positive and negative examples overlap" + at);
+        }
+    }
+    for (uint64_t i = 0; i < n_blacklist; ++i)
+        if (blacklist[i] >= 2 * U) return fail(c, GRMKM_E_INVALID, "blacklisted rule index >= 2 x n_kmers");
+
+    NvtxRange nv("grmkm_cart_run");
+    c->cart_nodes.assign(n_trees, {});
+    c->cart_equiv.assign(n_trees, {});
+    struct Open { uint32_t tree, node; };
+    std::vector<Open> open, next;
+    auto add_node = [&](uint32_t t, uint32_t depth, uint32_t a, uint32_t b) -> uint32_t {
+        grmkm_cart_node nd{};
+        nd.rule = UINT64_MAX;
+        nd.depth = depth; nd.n_pos = a; nd.n_neg = b;
+        nd.present_child = nd.absent_child = UINT32_MAX;
+        nd.prediction = jobs[t].w_pos * (double)a > jobs[t].w_neg * (double)b;
+        c->cart_nodes[t].push_back(nd);
+        return (uint32_t)(c->cart_nodes[t].size() - 1);
+    };
+    // a node is scanned unless a stop rule makes it a leaf first (T empty is only known after the scan)
+    auto opens = [&](uint32_t t, uint32_t depth, uint32_t a, uint32_t b) {
+        return U > 0 && depth < jobs[t].max_depth && (uint64_t)a + b >= jobs[t].min_samples_split && a > 0 && b > 0;
+    };
+    std::vector<uint64_t> h_masks;
+    for (uint32_t t = 0; t < n_trees; ++t) {
+        uint32_t a = 0, b = 0;
+        for (uint32_t w = 0; w < W; ++w) {
+            a += (uint32_t)__builtin_popcountll(jobs[t].pos[w]);
+            b += (uint32_t)__builtin_popcountll(jobs[t].neg[w]);
+        }
+        const uint32_t root = add_node(t, 0, a, b);
+        if (opens(t, 0, a, b)) {
+            open.push_back({t, root});
+            h_masks.insert(h_masks.end(), jobs[t].pos, jobs[t].pos + W);
+            h_masks.insert(h_masks.end(), jobs[t].neg, jobs[t].neg + W);
+        }
+    }
+    if (open.empty()) return GRMKM_OK;
+
+    CU_TRY(c, cudaSetDevice(c->device));
+    // chunk = open nodes whose masks share one CTA's shared memory; small enough for two CTAs per SM (as the SCM's)
+    const size_t smem_cap = (c->smem_optin ? c->smem_optin : 227 * 1024) - 1024;
+    const uint32_t chunk = (uint32_t)std::max<size_t>(1, std::min<size_t>(smem_cap / 2, 64 * 1024) / cart_smem_bytes(1, W));
+    const uint64_t max_grid = (uint64_t)c->sm_count * 8;
+    const uint64_t bl_words = (U + 31) / 32;
+    std::vector<uint32_t> h_bl(bl_words, 0);
+    for (uint64_t i = 0; i < n_blacklist; ++i) {
+        const uint64_t j = blacklist[i] % U;
+        h_bl[j >> 5] |= 1u << (j & 31);
+    }
+    ENSURE(c, c->cart_bl, bl_words * 4);
+    ENSURE(c, c->cart_masks[0], h_masks.size() * 8);
+    CU_TRY(c, cudaMemcpyAsync(c->cart_bl.p, h_bl.data(), bl_words * 4, cudaMemcpyHostToDevice, c->stream));
+    CU_TRY(c, cudaMemcpyAsync(c->cart_masks[0].p, h_masks.data(), h_masks.size() * 8, cudaMemcpyHostToDevice, c->stream));
+    int cur = 0;
+    {
+        const int r = W <= kScmCachedWords ? cart_allow_smem<true>(c, cart_smem_bytes(chunk, W))
+                                           : cart_allow_smem<false>(c, cart_smem_bytes(chunk, W));
+        if (r) return r;
+    }
+    std::map<uint32_t, int> occ_of;
+
+    const unsigned long long* mat = (const unsigned long long*)c->matrix.p;
+    uint64_t cap = std::max<uint64_t>(1024, c->cart_list.cap / 8);      // tie list entries
+    std::vector<CartNodeArg> args;
+    std::vector<CartSplit> splits;
+    std::vector<uint64_t> h_best, h_total, h_list;
+    std::vector<uint32_t> h_stats;
+    auto al = [](size_t b) { return (b + 255) & ~size_t(255); };
+    while (!open.empty()) {
+        const uint32_t n_open = (uint32_t)open.size();
+        const uint32_t cw = std::min(chunk, n_open);            // the widest chunk of this level
+        args.resize(n_open);
+        for (uint32_t i = 0; i < n_open; ++i) {
+            const grmkm_cart_job& j = jobs[open[i].tree];
+            const grmkm_cart_node& nd = c->cart_nodes[open[i].tree][open[i].node];
+            args[i] = CartNodeArg{j.w_pos, j.w_neg, std::max<uint64_t>(1, j.equiv_cap), i, nd.n_pos, nd.n_neg, 0};
+        }
+        const size_t o_args = 0, o_best = o_args + al((size_t)n_open * sizeof(CartNodeArg)), o_total = o_best + al((size_t)n_open * 8),
+                     o_tile = o_total + al((size_t)n_open * 8), o_tcnt = o_tile + al((size_t)cw * max_grid * 8),
+                     o_split = o_tcnt + al((size_t)cw * max_grid * 4), o_stats = o_split + al((size_t)n_open * sizeof(CartSplit)),
+                     o_count = o_stats + al((size_t)n_open * 8), total = o_count + 256;
+        ENSURE(c, c->cart, total);
+        uint8_t* base = (uint8_t*)c->cart.p;
+        CartNodeArg* d_args = (CartNodeArg*)(base + o_args);
+        unsigned long long* d_best = (unsigned long long*)(base + o_best);
+        unsigned long long* d_total = (unsigned long long*)(base + o_total);
+        unsigned long long* d_tile = (unsigned long long*)(base + o_tile);
+        uint32_t* d_tcnt = (uint32_t*)(base + o_tcnt);
+        CartSplit* d_split = (CartSplit*)(base + o_split);
+        uint32_t* d_stats = (uint32_t*)(base + o_stats);
+        unsigned long long* d_count = (unsigned long long*)(base + o_count);
+        const unsigned long long* d_masks = (const unsigned long long*)c->cart_masks[cur].p;
+        CU_TRY(c, cudaMemcpyAsync(d_args, args.data(), (size_t)n_open * sizeof(CartNodeArg), cudaMemcpyHostToDevice, c->stream));
+        uint64_t count = 0;
+        for (;;) {
+            ENSURE(c, c->cart_list, cap * 8);
+            unsigned long long* d_list = (unsigned long long*)c->cart_list.p;
+            CU_TRY(c, cudaMemsetAsync(d_best, 0, (size_t)n_open * 8, c->stream));
+            CU_TRY(c, cudaMemsetAsync(d_total, 0, (size_t)n_open * 8, c->stream));
+            CU_TRY(c, cudaMemsetAsync(d_count, 0, 8, c->stream));
+            for (uint32_t a0 = 0; a0 < n_open; a0 += chunk) {
+                const uint32_t n = std::min(chunk, n_open - a0);
+                const int r = W <= kScmCachedWords
+                                  ? cart_launch_chunk<true>(c, d_args + a0, n, (const uint32_t*)c->cart_bl.p, d_masks, d_best, d_tile,
+                                                            d_tcnt, d_total, d_list, d_count, cap, max_grid, occ_of)
+                                  : cart_launch_chunk<false>(c, d_args + a0, n, (const uint32_t*)c->cart_bl.p, d_masks, d_best, d_tile,
+                                                             d_tcnt, d_total, d_list, d_count, cap, max_grid, occ_of);
+                if (r) return r;
+            }
+            CU_TRY(c, cudaMemcpyAsync(&count, d_count, 8, cudaMemcpyDeviceToHost, c->stream));
+            CU_TRY(c, cudaStreamSynchronize(c->stream));
+            if (count <= cap) break;
+            cap = count + count / 4;    // the tie list overflowed: grow it and redo the level (nothing was updated)
+        }
+        h_best.resize(n_open); h_total.resize(n_open); h_list.resize(count);
+        CU_TRY(c, cudaMemcpyAsync(h_best.data(), d_best, (size_t)n_open * 8, cudaMemcpyDeviceToHost, c->stream));
+        CU_TRY(c, cudaMemcpyAsync(h_total.data(), d_total, (size_t)n_open * 8, cudaMemcpyDeviceToHost, c->stream));
+        CU_TRY(c, cudaMemcpyAsync(h_list.data(), c->cart_list.p, count * 8, cudaMemcpyDeviceToHost, c->stream));
+        CU_TRY(c, cudaStreamSynchronize(c->stream));
+        // the list comes in the order of the atomics: sorted, each node's entries are its ties in ascending column order
+        std::sort(h_list.begin(), h_list.end());
+        splits.clear();
+        size_t p = 0;
+        for (uint32_t i = 0; i < n_open; ++i) {
+            size_t e = p;
+            while (e < count && (h_list[e] >> 32) == i) ++e;
+            if (h_best[i]) {            // else no admissible split: the node stays a leaf
+                const grmkm_cart_job& j = jobs[open[i].tree];
+                const uint64_t keep = std::min<uint64_t>(h_total[i], j.equiv_cap);
+                if (e - p < std::max<uint64_t>(1, keep))
+                    return fail(c, GRMKM_E_CUDA, "grmkm_cart_run: the tie list of a node misses members of T");
+                std::vector<uint64_t>& eq = c->cart_equiv[open[i].tree];
+                grmkm_cart_node& nd = c->cart_nodes[open[i].tree][open[i].node];
+                nd.rule = h_list[p] & 0xffffffffULL;
+                nd.score = scm_unkey(~h_best[i]);
+                nd.equiv_offset = eq.size();
+                nd.equiv_count = keep;
+                nd.equiv_total = h_total[i];
+                for (uint64_t k = 0; k < keep; ++k) eq.push_back(h_list[p + k] & 0xffffffffULL);
+                splits.push_back(CartSplit{i, (uint32_t)nd.rule, UINT32_MAX, UINT32_MAX});
+            }
+            p = e;
+        }
+        next.clear();
+        if (!splits.empty()) {
+            const uint32_t n_split = (uint32_t)splits.size();
+            CU_TRY(c, cudaMemcpyAsync(d_split, splits.data(), n_split * sizeof(CartSplit), cudaMemcpyHostToDevice, c->stream));
+            k_cart_gather<<<(uint32_t)std::min<uint64_t>((n_split + 7) / 8, (uint64_t)c->sm_count * 16), 256, 0, c->stream>>>(
+                mat, c->pitch, W, d_masks, d_split, n_split, d_stats);
+            CU_TRY(c, cudaGetLastError());
+            c->stats.n_launches++;
+            h_stats.resize(2 * (size_t)n_split);
+            CU_TRY(c, cudaMemcpyAsync(h_stats.data(), d_stats, n_split * 8, cudaMemcpyDeviceToHost, c->stream));
+            CU_TRY(c, cudaStreamSynchronize(c->stream));
+            // children in their parents' order, the present child first: breadth-first numbering
+            for (uint32_t k = 0; k < n_split; ++k) {
+                const Open o = open[splits[k].src];
+                const uint32_t depth = c->cart_nodes[o.tree][o.node].depth + 1;
+                const uint32_t a = c->cart_nodes[o.tree][o.node].n_pos, b = c->cart_nodes[o.tree][o.node].n_neg;
+                const uint32_t pl = h_stats[2 * k], nl = h_stats[2 * k + 1];
+                const uint32_t pc = add_node(o.tree, depth, pl, nl), ac = add_node(o.tree, depth, a - pl, b - nl);
+                c->cart_nodes[o.tree][o.node].present_child = pc;
+                c->cart_nodes[o.tree][o.node].absent_child = ac;
+                if (opens(o.tree, depth, pl, nl)) { splits[k].dst_present = (uint32_t)next.size(); next.push_back({o.tree, pc}); }
+                if (opens(o.tree, depth, a - pl, b - nl)) { splits[k].dst_absent = (uint32_t)next.size(); next.push_back({o.tree, ac}); }
+            }
+            if (!next.empty()) {
+                ENSURE(c, c->cart_masks[cur ^ 1], next.size() * 2 * W * 8);
+                CU_TRY(c, cudaMemcpyAsync(d_split, splits.data(), n_split * sizeof(CartSplit), cudaMemcpyHostToDevice, c->stream));
+                const uint64_t nw = (uint64_t)n_split * W;
+                k_cart_split<<<(uint32_t)std::min<uint64_t>((nw + 255) / 256, (uint64_t)c->sm_count * 8), 256, 0, c->stream>>>(
+                    mat, c->pitch, W, d_masks, d_split, n_split, (unsigned long long*)c->cart_masks[cur ^ 1].p);
+                CU_TRY(c, cudaGetLastError());
+                c->stats.n_launches++;
+                cur ^= 1;
+            }
+        }
+        open.swap(next);
+    }
+    CU_TRY(c, cudaStreamSynchronize(c->stream));
+    return GRMKM_OK;
+}
+
+int grmkm_cart_result(grmkm_ctx* c, uint32_t tree, grmkm_cart_node* nodes, uint64_t nodes_cap, uint64_t* n_nodes,
+                      uint64_t* equivalent, uint64_t equiv_cap, uint64_t* n_equivalent) {
+    if (check_ctx(c)) return GRMKM_E_INVALID;
+    if (tree >= c->cart_nodes.size()) return fail(c, GRMKM_E_INVALID, "no such tree in the last grmkm_cart_run");
+    const std::vector<grmkm_cart_node>& s = c->cart_nodes[tree];
+    const std::vector<uint64_t>& e = c->cart_equiv[tree];
+    if (n_nodes) *n_nodes = s.size();
+    if (n_equivalent) *n_equivalent = e.size();
+    if ((!nodes && !s.empty()) || nodes_cap < s.size() || (!equivalent && !e.empty()) || equiv_cap < e.size())
+        return fail(c, GRMKM_E_CAPACITY, "cart result buffers too small");
+    if (!s.empty()) memcpy(nodes, s.data(), s.size() * sizeof(grmkm_cart_node));
     if (!e.empty()) memcpy(equivalent, e.data(), e.size() * 8);
     return GRMKM_OK;
 }

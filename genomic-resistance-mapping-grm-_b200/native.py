@@ -6,7 +6,7 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("GRMKM_LIB") or os.path.join(_HERE, "libgrmkm.so")   # GRMKM_LIB: another build of the same library (kernel experiments)
-ABI_VERSION = 11
+ABI_VERSION = 12
 
 OK = 0
 E_INVALID, E_UNSUPPORTED_K, E_NOMEM, E_CUDA, E_IO, E_CAPACITY, E_NO_DEVICE, E_UNSUPPORTED = -1, -2, -3, -4, -5, -6, -7, -8
@@ -23,6 +23,7 @@ SYMBOLS = [
     "grmkm_plan_bucket_bits", "grmkm_set_bucket_bits", "grmkm_set_exchange_rank",
     "grmkm_result_checksum", "grmkm_sum_rows", "grmkm_gram", "grmkm_tsv_pack",
     "grmkm_load_result", "grmkm_scm_run", "grmkm_scm_result",
+    "grmkm_cart_run", "grmkm_cart_result",
 ]
 SCM_CONJUNCTION, SCM_DISJUNCTION = 0, 1
 
@@ -68,6 +69,19 @@ class ScmJob(C.Structure):
 class ScmStep(C.Structure):
     _fields_ = [("rule", C.c_uint64), ("utility", C.c_double), ("positive_errors", C.c_uint32),
                 ("negative_covers", C.c_uint32), ("equiv_offset", C.c_uint64), ("equiv_count", C.c_uint64)]
+
+
+class CartJob(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("max_depth", C.c_uint32), ("min_samples_split", C.c_uint32),
+                ("reserved", C.c_uint32), ("equiv_cap", C.c_uint64), ("w_neg", C.c_double), ("w_pos", C.c_double),
+                ("pos", C.c_void_p), ("neg", C.c_void_p)]
+
+
+class CartNode(C.Structure):
+    _fields_ = [("rule", C.c_uint64), ("score", C.c_double), ("depth", C.c_uint32), ("n_pos", C.c_uint32),
+                ("n_neg", C.c_uint32), ("present_child", C.c_uint32), ("absent_child", C.c_uint32),
+                ("prediction", C.c_uint32), ("equiv_offset", C.c_uint64), ("equiv_count", C.c_uint64),
+                ("equiv_total", C.c_uint64)]
 
 
 _lib = None
@@ -120,6 +134,8 @@ def load() -> C.CDLL:
         "grmkm_load_result": (i32, [vp, vp, vp, u64, u32]),
         "grmkm_scm_run": (i32, [vp, u32, vp, vp, u64]),
         "grmkm_scm_result": (i32, [vp, u32, vp, u64, C.POINTER(u64), vp, u64, C.POINTER(u64)]),
+        "grmkm_cart_run": (i32, [vp, u32, vp, vp, u64]),
+        "grmkm_cart_result": (i32, [vp, u32, vp, u64, C.POINTER(u64), vp, u64, C.POINTER(u64)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)

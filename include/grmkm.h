@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define GRMKM_ABI_VERSION 11
+#define GRMKM_ABI_VERSION 12
 
 enum {
     GRMKM_OK = 0,
@@ -288,6 +288,54 @@ int grmkm_scm_run(grmkm_ctx* ctx, uint32_t n_fits, const grmkm_scm_job* jobs, co
  * GRMKM_E_CAPACITY (sizes still written). */
 int grmkm_scm_result(grmkm_ctx* ctx, uint32_t fit, grmkm_scm_step* steps, uint64_t steps_cap, uint64_t* n_steps,
                      uint64_t* equivalent, uint64_t equiv_cap, uint64_t* n_equivalent);
+
+/*
+ * CART decision trees (kover learning/learners/cart.py, gini criterion) on the resident matrix, many trees at once.
+ * A node splits on k-mer j < U: the examples holding it go to the present child, the others to the absent child (rule
+ * U + j is the same split, so only j < U is considered; a blacklist entry j or U + j removes k-mer j).  For a child
+ * with a positive and b negative examples, A = w_pos * a, B = w_neg * b, S = A + B, term = (A * B) / S, each a
+ * correctly rounded double operation in this order; score = term_present + term_absent (half the weighted Gini
+ * impurity sum).  Admissible: both children non-empty, k-mer not blacklisted.  s* = min score over admissible splits,
+ * T = {admissible j : score == s*}, the node's rule is min T.  A node is a leaf when depth == max_depth (root: 0),
+ * a + b < min_samples_split, a == 0 or b == 0, or T is empty.  prediction = 1 iff A > B of the node's own counts.
+ * Nodes are numbered breadth-first: level by level, in their parents' order, the present child before the absent
+ * child; the root is 0.  Every level of all trees is one pass over the matrix on the device; only the best scores,
+ * the tie list and the chosen rules' counts cross PCIe.
+ */
+typedef struct grmkm_cart_job {
+    uint32_t struct_size;        /* = sizeof(grmkm_cart_job) */
+    uint32_t max_depth;          /* >= 1 */
+    uint32_t min_samples_split;  /* >= 2 */
+    uint32_t reserved;           /* 0 */
+    uint64_t equiv_cap;          /* per node, at most this many (the smallest) members of T are recorded */
+    double w_neg;                /* class importance of the negatives: finite, > 0, <= 1e100 (no product overflows) */
+    double w_pos;                /* the same for the positives */
+    const uint64_t* pos;         /* n_words words, genome g at bit 63 - g % 64 of word g / 64 */
+    const uint64_t* neg;         /* disjoint from pos */
+} grmkm_cart_job;
+
+typedef struct grmkm_cart_node {
+    uint64_t rule;               /* k-mer index of the split (< U), UINT64_MAX: leaf */
+    double score;                /* s* of the split; leaf: 0 */
+    uint32_t depth;              /* root: 0 */
+    uint32_t n_pos;              /* a: positive examples of the node */
+    uint32_t n_neg;              /* b: negative examples of the node */
+    uint32_t present_child;      /* node index, UINT32_MAX: leaf */
+    uint32_t absent_child;
+    uint32_t prediction;         /* 1 iff w_pos * a > w_neg * b (the leaf's output) */
+    uint64_t equiv_offset;       /* the recorded members of T: equivalent[equiv_offset .. + equiv_count), ascending */
+    uint64_t equiv_count;        /* min(|T|, equiv_cap) */
+    uint64_t equiv_total;        /* |T| */
+} grmkm_cart_node;
+
+/* Grows every tree to completion; the results stay in the context until the next run / build / load / reset.  Refuses
+ * (GRMKM_E_UNSUPPORTED) a result that is one owner's slice of a multi-GPU merge. */
+int grmkm_cart_run(grmkm_ctx* ctx, uint32_t n_trees, const grmkm_cart_job* jobs, const uint64_t* blacklist,
+                   uint64_t n_blacklist);
+/* Nodes and equivalent rules of tree `tree`.  *n_nodes / *n_equivalent receive the sizes; NULL or short buffers:
+ * GRMKM_E_CAPACITY (sizes still written). */
+int grmkm_cart_result(grmkm_ctx* ctx, uint32_t tree, grmkm_cart_node* nodes, uint64_t nodes_cap, uint64_t* n_nodes,
+                      uint64_t* equivalent, uint64_t equiv_cap, uint64_t* n_equivalent);
 
 #ifdef __cplusplus
 }
