@@ -22,6 +22,8 @@ class KmerMatrixBuilder:
         self._lib = native.load()
         self._ctx = C.c_void_p()
         self._keep = []          # borrowed host buffers must outlive build()
+        self._rows = 0           # max genome row + 1 of the inputs added since the last reset
+        self._declared = 0       # set_genome_count
         self.k = int(k)
         cfg = native.Config(C.sizeof(native.Config), int(k), int(min_abundance), int(bool(keep_singletons)),
                             int(input_kind), int(device), int(bucket_bits), int(flags),
@@ -59,6 +61,7 @@ class KmerMatrixBuilder:
     def reset(self):
         self._check(self._lib.grmkm_reset(self._ctx))
         self._keep = []
+        self._rows = self._declared = 0
 
     def add_genome_bytes(self, row: int, data) -> None:
         """data: bytes / bytearray / memoryview / uint8 ndarray (borrowed until build returns)."""
@@ -68,9 +71,11 @@ class KmerMatrixBuilder:
             arr = np.frombuffer(data, dtype=np.uint8)
         self._keep.append(arr)
         self._check(self._lib.grmkm_add_genome_bytes(self._ctx, int(row), C.c_void_p(arr.ctypes.data), arr.size))
+        self._rows = max(self._rows, int(row) + 1)
 
     def add_genome_device(self, row: int, dev_ptr: int, n_bytes: int) -> None:
         self._check(self._lib.grmkm_add_genome_device(self._ctx, int(row), C.c_void_p(int(dev_ptr)), int(n_bytes)))
+        self._rows = max(self._rows, int(row) + 1)
 
     def add_genomes(self, rows, data, lens=None, on_device: bool = False) -> None:
         """Every input of the build in one call.  rows[i] = genome row of input i; data = device pointers (ints,
@@ -89,14 +94,18 @@ class KmerMatrixBuilder:
             raise ValueError("rows, data and lens differ in length")
         self._check(self._lib.grmkm_add_genomes(self._ctx, len(rows), C.c_void_p(rows.ctypes.data), C.c_void_p(ptrs.ctypes.data),
                                                 C.c_void_p(lens.ctypes.data), int(bool(on_device))))
+        if len(rows):
+            self._rows = max(self._rows, int(rows.max()) + 1)
 
     def add_genome_files(self, row: int, paths: Sequence[str]) -> None:
         paths = [paths] if isinstance(paths, (str, bytes)) else list(paths)
         arr = (C.c_char_p * max(len(paths), 1))(*[p.encode() if isinstance(p, str) else p for p in paths])
         self._check(self._lib.grmkm_add_genome_files(self._ctx, int(row), arr, len(paths)))
+        self._rows = max(self._rows, int(row) + 1)
 
     def set_genome_count(self, n: int) -> None:
         self._check(self._lib.grmkm_set_genome_count(self._ctx, int(n)))
+        self._declared = int(n)
 
     # -- build + results ----------------------------------------------------------------------
     def build(self) -> "KmerMatrixBuilder":
@@ -282,6 +291,26 @@ class KmerMatrixBuilder:
                                                     C.c_void_p(eq.ctypes.data), eq.size, C.byref(ne)))
             out.append((nodes, eq))
         return out
+
+    @property
+    def query_genome_count(self) -> int:
+        """G of a build of the inputs added since the last reset: max row + 1, or set_genome_count when larger."""
+        return max(self._rows, self._declared)
+
+    def query(self, kmers, with_stats: bool = False):
+        """Which genome rows of the inputs added since the last reset hold which k-mers, without a build: uint64
+        (ceil(G/64), len(kmers)), genome g at bit 63 - g % 64 of word row g // 64 (the matrix's layout).  kmers: packed
+        as ``kmers()`` returns them, either strand, duplicates allowed; column i is about the canonical form of
+        kmers[i], set for a genome whose windows hold it at least min_abundance times.  The resident result, stats and
+        fits are left as they are.  with_stats: also return the call's statistics as a dict."""
+        q = np.ascontiguousarray(np.asarray(kmers, dtype=np.uint64).reshape(-1))
+        G = self.query_genome_count
+        out = np.zeros(((G + 63) // 64, q.size), dtype=np.uint64)
+        st = native.QueryStats()
+        st.struct_size = C.sizeof(native.QueryStats)
+        self._check(self._lib.grmkm_query(self._ctx, C.c_void_p(q.ctypes.data), q.size, C.c_void_p(out.ctypes.data),
+                                          out.size, C.byref(st)))
+        return (out, st.asdict()) if with_stats else out
 
     def device_result(self) -> tuple[int, int, int]:
         """(device pointer of kmers[U], device pointer of the matrix, row pitch in words): word row w of the matrix

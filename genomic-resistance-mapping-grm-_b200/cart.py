@@ -72,23 +72,35 @@ class DecisionTreeClassifier:
         if not self.nodes:
             raise ValueError("the tree is not fitted")
         example_idx = np.asarray(example_idx, dtype=np.int64).reshape(-1)
-        n = len(self.nodes)
-        present = np.array([-1 if x.rule is None else x.present_child for x in self.nodes], dtype=np.int64)
-        absent = np.array([-1 if x.rule is None else x.absent_child for x in self.nodes], dtype=np.int64)
-        pred = np.array([x.prediction for x in self.nodes], dtype=np.uint8)
         kmers = sorted({x.rule.kmer_index for x in self.nodes if x.rule is not None})
-        at = np.zeros(len(example_idx), dtype=np.int64)
-        if kmers:
-            col_of = {j: i for i, j in enumerate(kmers)}
-            col = np.array([col_of[x.rule.kmer_index] if x.rule is not None else -1 for x in self.nodes], dtype=np.int64)
-            cols = rule_classifications.get_columns(kmers)[example_idx]
-            for _ in range(n):
-                inner = np.nonzero(col[at] >= 0)[0]
-                if not len(inner):
-                    break
-                here = at[inner]
-                at[inner] = np.where(cols[inner, col[here]] == 1, present[here], absent[here])
-        return pred[at]
+        col_of = {j: i for i, j in enumerate(kmers)}
+        col = np.array([col_of[x.rule.kmer_index] if x.rule is not None else -1 for x in self.nodes], dtype=np.int64)
+        cols = (rule_classifications.get_columns(kmers)[example_idx] if kmers
+                else np.zeros((len(example_idx), 0), dtype=np.uint8))
+        return _tree_output(self.nodes, col, cols)
+
+    def predict_genomes(self, builder) -> np.ndarray:
+        """0/1 per genome row of the inputs of ``builder`` (a KmerMatrixBuilder holding genomes that need not have
+        been in the training matrix): one ``builder.query`` of the split k-mers, no build (predict.predict_genomes)."""
+        from .predict import predict_genomes
+        return predict_genomes([self], builder)[0]
+
+
+def _tree_output(nodes, col: np.ndarray, cols: np.ndarray) -> np.ndarray:
+    """The leaf prediction of every example: cols = 0/1 (examples x columns), col[i] = the column of node i's split
+    k-mer (-1: a leaf).  The examples walk the tree from the root to their leaves."""
+    n = len(nodes)
+    present = np.array([-1 if x.rule is None else x.present_child for x in nodes], dtype=np.int64)
+    absent = np.array([-1 if x.rule is None else x.absent_child for x in nodes], dtype=np.int64)
+    pred = np.array([x.prediction for x in nodes], dtype=np.uint8)
+    at = np.zeros(len(cols), dtype=np.int64)
+    for _ in range(n):
+        inner = np.nonzero(col[at] >= 0)[0]
+        if not len(inner):
+            break
+        here = at[inner]
+        at[inner] = np.where(cols[inner, col[here]] == 1, present[here], absent[here])
+    return pred[at]
 
 
 def fit_many(rule_classifications, trees, rule_blacklist=None):

@@ -7,6 +7,7 @@
 #include "grmkm_synth.cuh"
 #include "grmkm_scm.cuh"
 #include "grmkm_cart.cuh"
+#include "grmkm_query.cuh"
 
 #include <nvtx3/nvToolsExt.h>      // header-only; the ranges cost nothing until a tool (nsys, ncu --nvtx) attaches
 #include <zlib.h>
@@ -104,7 +105,11 @@ struct grmkm_ctx {
         cart,            // grmkm_cart_run: per-level node arguments, bests, tie totals, per-CTA bests and tie counts, splits
         cart_bl,         // grmkm_cart_run: blacklist bits (one per k-mer)
         cart_masks[2],   // grmkm_cart_run: P and N of the open nodes of this level / of the next level
-        cart_list;       // grmkm_cart_run: the tie list
+        cart_list,       // grmkm_cart_run: the tie list
+        qry,             // grmkm_query: key table, slot -> key index, caller column -> key index, totals
+        qplane,          // grmkm_query: presence plane or counters of one row range
+        qout;            // grmkm_query: one row range's word rows in the caller's column order
+    cudaEvent_t ev_query[2] = {nullptr, nullptr};   // grmkm_query: device time of the call
     uint64_t racc_hint = 0;        // records of the previous abundance build + headroom
     uint32_t pack_ctas[2] = {0, 0};      // resident CTAs of the persistent k_pack (FASTA / FASTQ)
     std::vector<uint64_t> merge_h_off;   // row-block merge of a partial build: chunk offsets of the merge buckets
@@ -349,6 +354,8 @@ struct Geo {
     uint32_t B = 0, VB = 0;
 };
 
+struct QueryJob;
+
 struct Job {
     uint32_t f0 = 0, f1 = 0;        // inputs
     uint32_t row0 = 0, n_rows = 0;  // genome rows of the job (FileDesc.row = input row - row0)
@@ -357,7 +364,30 @@ struct Job {
     // AGG_ROUND: where the round's records go
     ulonglong2* round_out = nullptr;
     uint64_t round_cap = 0;
+    // a query job (grmkm_query): every batch's packed stream goes through k_query_scan instead of the unit path, and
+    // the job ends after the last batch
+    const QueryJob* query = nullptr;
 };
+
+struct QueryJob {
+    QueryScanParams sp;             // table, plane / counters, totals (the batch fields are filled per batch)
+    bool smem = false, count = false;
+    uint32_t ctas_per_sm = 1;
+    size_t smem_bytes = 0;
+};
+
+int launch_query_scan(grmkm_ctx* c, const QueryJob& q, const FileDesc* d_files, uint32_t n_files, uint64_t n_groups_max) {
+    QueryScanParams sp = q.sp;
+    sp.codes = (const unsigned long long*)c->codes.p; sp.valid = (const uint32_t*)c->valid.p;
+    sp.scalars = (const uint64_t*)c->scalars.p; sp.fss = (const uint64_t*)c->fss.p; sp.files = d_files; sp.n_files = n_files;
+    const uint32_t grid = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((n_groups_max + kQsThreads - 1) / kQsThreads,
+                                                                               (uint64_t)c->sm_count * q.ctas_per_sm));
+    void (*kern)(QueryScanParams) = q.smem ? (q.count ? k_query_scan<true, true> : k_query_scan<true, false>)
+                                           : (q.count ? k_query_scan<false, true> : k_query_scan<false, false>);
+    kern<<<grid, kQsThreads, q.smem_bytes, c->stream>>>(sp);
+    CU_TRY(c, cudaGetLastError());
+    return GRMKM_OK;
+}
 
 struct JobOut {
     uint64_t sc[S_COUNT] = {0};
@@ -510,7 +540,8 @@ int run_job(grmkm_ctx* c, const Geo& geo, const Job& job, JobOut& out) {
     uint64_t* d_scalars = (uint64_t*)c->scalars.p;
     const FileDesc* d_files = nullptr;
 
-    if (c->ev_ok) cudaEventRecord(c->ev[T_START], st);
+    const bool query = job.query != nullptr;
+    if (c->ev_ok && !query) cudaEventRecord(c->ev[T_START], st);
     CU_TRY(c, cudaMemsetAsync(c->scalars.p, 0, S_COUNT * 8, st));
 
     // parse + pack of one batch: leaves codes / valid / fss / S_STREAM_LEN of the batch
@@ -637,10 +668,10 @@ int run_job(grmkm_ctx* c, const Geo& geo, const Job& job, JobOut& out) {
     const uint32_t WB = counting ? 1u : unit_words_per_entry(geo.W);
     const uint32_t n_groups_w = counting ? std::max(1u, job.n_rows) : (geo.W + WB - 1) / WB;
     const uint32_t wbits = std::max(1u, ceil_log2(n_groups_w));
-    if (wbits > geo.bucket_bits) return fail(c, GRMKM_E_UNSUPPORTED, "more genome groups than hash buckets");
+    if (!query && wbits > geo.bucket_bits) return fail(c, GRMKM_E_UNSUPPORTED, "more genome groups than hash buckets");
     const uint32_t ES = 2 + WB, RS = unit_record_stride(WB);
     uint32_t MB = (uint32_t)c->sm_count;
-    {
+    if (!query) {
         // distinct (unit, genome group) entries of a bucket should fit the dedupe table about once
         const uint64_t entries = counting ? in_bytes / (ug.w + 1) / 2 + 1
                                           : (job.max_row_bytes * 19 / 10) * 2 / (ug.w + 1) * 13 / 10 * n_groups_w;
@@ -654,6 +685,26 @@ int run_job(grmkm_ctx* c, const Geo& geo, const Job& job, JobOut& out) {
     out.MB = MB;
     const bool try_regions = !getenv("GRMKM_EXACT_OFFSETS");
     uint64_t* sc = out.sc;
+    // codes / valid / tile words are dead once the last batch has been scattered (or scanned): clear them for the next
+    // build or query (or the next pass) on the side stream, under whatever the stream runs next
+    auto preclear = [&]() -> int {
+        if (!c->pass_groups || getenv("GRMKM_NO_PRECLEAR")) return GRMKM_OK;
+        if (!c->aux_stream) {
+            CU_TRY(c, cudaStreamCreateWithFlags(&c->aux_stream, cudaStreamNonBlocking));
+            CU_TRY(c, cudaEventCreateWithFlags(&c->ev_scattered, cudaEventDisableTiming));
+            CU_TRY(c, cudaEventCreateWithFlags(&c->ev_cleared, cudaEventDisableTiming));
+        }
+        CU_TRY(c, cudaEventRecord(c->ev_scattered, st));
+        CU_TRY(c, cudaStreamWaitEvent(c->aux_stream, c->ev_scattered, 0));
+        CU_TRY(c, cudaMemsetAsync(c->codes.p, 0, c->pass_groups * 8, c->aux_stream));
+        CU_TRY(c, cudaMemsetAsync(c->valid.p, 0, c->pass_groups * 4, c->aux_stream));
+        CU_TRY(c, cudaMemsetAsync(c->tile_pub.p, 0, c->pass_pub_bytes, c->aux_stream));
+        CU_TRY(c, cudaEventRecord(c->ev_cleared, c->aux_stream));
+        c->pre_pending = true;
+        c->pre_codes = c->codes.p; c->pre_valid = c->valid.p; c->pre_pub = c->tile_pub.p;
+        c->pre_groups = c->pass_groups; c->pre_pub_bytes = c->pass_pub_bytes;
+        return GRMKM_OK;
+    };
     for (int pass = try_regions ? 0 : 1; pass < 2; ++pass) {
         // Pass 0 scatters into over-provisioned bucket regions without a count pass; if a region overflows (heavily
         // skewed unit spectrum) pass 1 redoes the scatter with exact offsets from a count pass.
@@ -675,7 +726,9 @@ int run_job(grmkm_ctx* c, const Geo& geo, const Job& job, JobOut& out) {
             c->h_tab_used = 0;
         }
         uint64_t cap = 0;
-        if (regions) {
+        if (query) {
+            // (no unit regions: the scan writes the plane)
+        } else if (regions) {
             const double est_units = (double)max_stream * 2.0 / (ug.w + 1) * 1.15;
             cap = (uint64_t)(est_units / MB * 1.25) + 4096;
             cap = (cap + 15) & ~15ULL;
@@ -694,11 +747,11 @@ int run_job(grmkm_ctx* c, const Geo& geo, const Job& job, JobOut& out) {
             }
         }
         CU_TRY(c, cudaMemsetAsync(d_scalars, 0, S_COUNT * 8, st));
-        if (regions) {
+        if (regions && !query) {
             k_init_regions<<<(MB + 1 + 255) / 256, 256, 0, st>>>((unsigned long long*)c->ubeg.p, (unsigned long long*)c->ucur.p, MB, cap);
             out.launches++;
         }
-        if (pipelined && c->ev_ok)
+        if (pipelined && c->ev_ok && !query)
             for (int e : {T_H2D, T_PARSE, T_PACK, T_COUNT, T_BOUNDS}) cudaEventRecord(c->ev[e], st);   // stages interleave: only "scatter" is timed
         out.h2d = 0;
         NvtxRange nv_front("grmkm front: stage / pack / unit bounds / unit scatter");
@@ -741,9 +794,15 @@ int run_job(grmkm_ctx* c, const Geo& geo, const Job& job, JobOut& out) {
                 CU_TRY(c, cudaEventRecord(c->ev_copied[bi & 1], cs));
                 CU_TRY(c, cudaStreamWaitEvent(st, c->ev_copied[bi & 1], 0));
             }
-            int fr = front(bt, half, !pipelined);
+            int fr = front(bt, half, !pipelined && !query);
             if (fr) return fr;
             if (pipelined) CU_TRY(c, cudaEventRecord(c->ev_free[bi & 1], st));     // the staged text has been consumed
+            if (query) {
+                fr = launch_query_scan(c, *job.query, d_files, bt.f1 - bt.f0, bt.stream / 32 + 2);
+                if (fr) return fr;
+                out.launches++;
+                continue;
+            }
 
             const uint32_t F = bt.f1 - bt.f0;
             const uint64_t n_groups_max = bt.stream / 32 + 2;
@@ -796,30 +855,15 @@ int run_job(grmkm_ctx* c, const Geo& geo, const Job& job, JobOut& out) {
             CU_TRY(c, cudaEventRecord(*gate_ev, pipelined ? c->copy_stream : st));      // behind this build's last copy
             gate.unlock();
         }
+        if (query) return preclear();
         // bucket b = units[begin[b], end[b]): end = the cursors (clamped to the region)
         k_finish_unit_regions<<<1, 1024, 0, st>>>((const unsigned long long*)c->ubeg.p, (unsigned long long*)c->ucur.p, MB,
                                                   cap, (unsigned long long*)d_scalars, S_N_UNITS);
         out.launches++;
         CU_TRY(c, cudaGetLastError());
         if (c->ev_ok) cudaEventRecord(c->ev[T_SCATTER], st);
-        // codes / valid / tile words are dead from here on: clear them for the next build (or the next pass) on the side
-        // stream, under the dedupe / expand / aggregate kernels, which leave most of the HBM bandwidth unused
-        if (c->pass_groups && !getenv("GRMKM_NO_PRECLEAR")) {
-            if (!c->aux_stream) {
-                CU_TRY(c, cudaStreamCreateWithFlags(&c->aux_stream, cudaStreamNonBlocking));
-                CU_TRY(c, cudaEventCreateWithFlags(&c->ev_scattered, cudaEventDisableTiming));
-                CU_TRY(c, cudaEventCreateWithFlags(&c->ev_cleared, cudaEventDisableTiming));
-            }
-            CU_TRY(c, cudaEventRecord(c->ev_scattered, st));
-            CU_TRY(c, cudaStreamWaitEvent(c->aux_stream, c->ev_scattered, 0));
-            CU_TRY(c, cudaMemsetAsync(c->codes.p, 0, c->pass_groups * 8, c->aux_stream));
-            CU_TRY(c, cudaMemsetAsync(c->valid.p, 0, c->pass_groups * 4, c->aux_stream));
-            CU_TRY(c, cudaMemsetAsync(c->tile_pub.p, 0, c->pass_pub_bytes, c->aux_stream));
-            CU_TRY(c, cudaEventRecord(c->ev_cleared, c->aux_stream));
-            c->pre_pending = true;
-            c->pre_codes = c->codes.p; c->pre_valid = c->valid.p; c->pre_pub = c->tile_pub.p;
-            c->pre_groups = c->pass_groups; c->pre_pub_bytes = c->pass_pub_bytes;
-        }
+        // (under the dedupe / expand / aggregate kernels, which leave most of the HBM bandwidth unused)
+        { const int pr = preclear(); if (pr) return pr; }
 
         nv_front.end();
         NvtxRange nv_back("grmkm back: dedupe / expand / aggregate");
@@ -1392,9 +1436,10 @@ void grmkm_destroy(grmkm_ctx* c) {
                      &c->bcounts, &c->ukeys, &c->uwords, &c->kmers, &c->matrix, &c->scalars, &c->fmt, &c->synth, &c->refs,
                      &c->stile_file, &c->bbase, &c->apub, &c->masks, &c->units, &c->ucur, &c->ubeg, &c->wu, &c->wide,
                      &c->racc, &c->aux, &c->scm, &c->scm_list, &c->cart, &c->cart_bl,
-                     &c->cart_masks[0], &c->cart_masks[1], &c->cart_list};
+                     &c->cart_masks[0], &c->cart_masks[1], &c->cart_list, &c->qry, &c->qplane, &c->qout};
     for (DevBuf* b : all) release(c, *b);
     if (c->ev_ok) for (int i = 0; i < T_N; ++i) cudaEventDestroy(c->ev[i]);
+    for (cudaEvent_t e : c->ev_query) if (e) cudaEventDestroy(e);
     if (c->host_res) cudaFreeHost(c->host_res);
     if (c->aux_stream) {
         cudaEventDestroy(c->ev_scattered); cudaEventDestroy(c->ev_cleared);
@@ -2525,6 +2570,192 @@ int grmkm_cart_result(grmkm_ctx* c, uint32_t tree, grmkm_cart_node* nodes, uint6
         return fail(c, GRMKM_E_CAPACITY, "cart result buffers too small");
     if (!s.empty()) memcpy(nodes, s.data(), s.size() * sizeof(grmkm_cart_node));
     if (!e.empty()) memcpy(equivalent, e.data(), e.size() * 8);
+    return GRMKM_OK;
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------------
+// grmkm_query: the inputs' genome rows against a set of k-mers, without a build
+// ------------------------------------------------------------------------------------------------
+namespace {
+
+// device memory of one row range: its presence plane (or counters) and its word rows in the caller's column order.
+// Over this, the query runs as consecutive row ranges, each a pass over its own rows' inputs only.
+constexpr uint64_t kQueryBudget = 1ULL << 30;
+
+uint64_t canonical_kmer(uint64_t x, uint32_t k) {
+    uint64_t rc = 0, f = x;
+    for (uint32_t i = 0; i < k; ++i) { rc = (rc << 2) | ((f & 3) ^ 2); f >>= 2; }
+    return std::min(x, rc);
+}
+
+int query_impl(grmkm_ctx* c, const uint64_t* kmers, uint64_t n, uint64_t* dst, uint32_t G, grmkm_query_stats& qs) {
+    CU_TRY(c, cudaSetDevice(c->device));
+    cudaStream_t st = c->stream;
+    const uint32_t k = c->cfg.k;
+    for (cudaEvent_t& e : c->ev_query) if (!e) CU_TRY(c, cudaEventCreate(&e));
+    CU_TRY(c, cudaEventRecord(c->ev_query[0], st));
+
+    // ---- distinct canonical keys in ascending hash order (the build's column order) and the caller's column -> key
+    std::vector<std::pair<uint64_t, uint32_t>> hv(n);
+    for (uint64_t i = 0; i < n; ++i) hv[i] = {khash(canonical_kmer(kmers[i], k)), (uint32_t)i};
+    std::sort(hv.begin(), hv.end());
+    std::vector<uint64_t> keys;
+    std::vector<uint32_t> col(n);
+    for (uint64_t j = 0; j < n; ++j) {
+        if (j == 0 || hv[j].first != hv[j - 1].first) keys.push_back(kunhash(hv[j].first));
+        col[hv[j].second] = (uint32_t)(keys.size() - 1);
+    }
+    std::vector<std::pair<uint64_t, uint32_t>>().swap(hv);
+    const uint64_t Qd = keys.size();
+    qs.n_queries = Qd;
+    // ---- open addressing, linear probing, home slot = top bits of fmix64 (grmkm_query.cuh).  kEmptyKey (UINT64_MAX)
+    // is never a canonical k-mer: below k = 32 every k-mer is < 2^62, and at k = 32 UINT64_MAX is all-G, whose reverse
+    // complement all-C is smaller.
+    const uint32_t slot_bits = std::max(1u, ceil_log2(2 * Qd));
+    const uint64_t slots = 1ULL << slot_bits;
+    std::vector<uint64_t> tk(slots, kEmptyKey);
+    std::vector<uint32_t> ti(slots, 0);
+    for (uint64_t q = 0; q < Qd; ++q) {
+        uint64_t s = fmix64(keys[q]) >> (64 - slot_bits);
+        while (tk[s] != kEmptyKey) s = (s + 1) & (slots - 1);
+        tk[s] = keys[q]; ti[s] = (uint32_t)q;
+    }
+    const size_t tab_bytes = slots * 12 + n * 4 + 16;
+    ENSURE(c, c->qry, tab_bytes);
+    unsigned long long* d_keys = (unsigned long long*)c->qry.p;
+    unsigned long long* d_totals = d_keys + slots;
+    uint32_t* d_idx = (uint32_t*)(d_totals + 2);
+    uint32_t* d_col = d_idx + slots;
+    CU_TRY(c, cudaMemcpyAsync(d_keys, tk.data(), slots * 8, cudaMemcpyHostToDevice, st));
+    CU_TRY(c, cudaMemsetAsync(d_totals, 0, 16, st));
+    CU_TRY(c, cudaMemcpyAsync(d_idx, ti.data(), slots * 4, cudaMemcpyHostToDevice, st));
+    CU_TRY(c, cudaMemcpyAsync(d_col, col.data(), n * 4, cudaMemcpyHostToDevice, st));
+
+    QueryJob qj;
+    qj.count = c->cfg.min_abundance > 1;
+    qj.smem = Qd <= kQuerySmemKeys && !getenv("GRMKM_QUERY_GLOBAL");
+    qj.smem_bytes = qj.smem ? slots * 8 : 0;
+    {
+        void (*kern)(QueryScanParams) = qj.smem ? (qj.count ? k_query_scan<true, true> : k_query_scan<true, false>)
+                                                : (qj.count ? k_query_scan<false, true> : k_query_scan<false, false>);
+        if (qj.smem) CU_TRY(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)qj.smem_bytes));
+        int occ = 0;
+        CU_TRY(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kQsThreads, qj.smem_bytes));
+        qj.ctas_per_sm = (uint32_t)std::max(1, occ);
+    }
+    qj.sp.k = k; qj.sp.keys = d_keys; qj.sp.idx = d_idx; qj.sp.slot_bits = slot_bits; qj.sp.qd = Qd; qj.sp.totals = d_totals;
+
+    // ---- row ranges: the plane (or counters) and the gathered word rows of one range stay within kQueryBudget
+    uint64_t rows_per;
+    if (!qj.count) rows_per = 64 * std::max<uint64_t>(1, kQueryBudget / ((Qd + n) * 8));
+    else rows_per = kQueryBudget > 2 * n * 8 ? std::max<uint64_t>(1, (kQueryBudget - 2 * n * 8) / (Qd * 4 + n * 8 / 64 + 1)) : 1;
+    if (const char* e = getenv("GRMKM_QUERY_ROWS")) {
+        const uint64_t v = (uint64_t)std::max(1LL, atoll(e));
+        rows_per = qj.count ? v : (v + 63) / 64 * 64;          // presence ranges are whole word rows
+    }
+    rows_per = std::min<uint64_t>(rows_per, G);
+    const uint32_t n_ranges = (uint32_t)((G + rows_per - 1) / rows_per);
+    if (n_ranges > 1)
+        std::stable_sort(c->inputs.begin(), c->inputs.end(), [](const Input& a, const Input& b) { return a.row < b.row; });
+    const InputTable tab = tabulate_inputs(c);
+    const uint32_t F = (uint32_t)c->inputs.size();
+    Geo geo;
+    geo.G = G; geo.W = (G + 63) / 64;
+
+    std::vector<uint64_t> boundary(n);          // a word row shared by two counter ranges: ORed on the host
+    uint32_t next_word = 0;                     // word rows of dst below this have been written
+    uint64_t sc[S_COUNT];
+    for (uint32_t r0 = 0; r0 < G; r0 += (uint32_t)rows_per) {
+        const uint32_t nr = (uint32_t)std::min<uint64_t>(rows_per, G - r0);
+        const uint32_t w0 = r0 >> 6, w1 = ((r0 + nr - 1) >> 6) + 1, nw = w1 - w0;
+        const uint32_t f0 = n_ranges > 1 ? tab.first_file[r0] : 0, f1 = n_ranges > 1 ? tab.first_file[r0 + nr] : F;
+        if (f0 == f1) {                         // rows without input
+            if (w1 > next_word) { memset(dst + (uint64_t)std::max(w0, next_word) * n, 0, (uint64_t)(w1 - std::max(w0, next_word)) * n * 8); next_word = w1; }
+            continue;
+        }
+        const uint64_t plane_bytes = qj.count ? (uint64_t)nr * Qd * 4 : (uint64_t)nw * Qd * 8;
+        ENSURE(c, c->qplane, plane_bytes);
+        ENSURE(c, c->qout, (uint64_t)nw * n * 8);
+        CU_TRY(c, cudaMemsetAsync(c->qplane.p, 0, plane_bytes, st));
+        qj.sp.row0 = r0;
+        qj.sp.plane = (unsigned long long*)c->qplane.p; qj.sp.counts = (uint32_t*)c->qplane.p;
+        Job job; job.f0 = f0; job.f1 = f1; job.row0 = r0; job.n_rows = nr; job.query = &qj;
+        JobOut out;
+        int rc = run_job(c, geo, job, out);
+        if (rc) return rc;
+        QueryGatherParams gp{};
+        gp.plane = (const unsigned long long*)c->qplane.p; gp.counts = (const uint32_t*)c->qplane.p; gp.col = d_col;
+        gp.qd = Qd; gp.n = n; gp.n_words = nw; gp.row0 = r0; gp.n_rows = nr; gp.min_abundance = c->cfg.min_abundance;
+        gp.out = (unsigned long long*)c->qout.p;
+        const uint32_t ggrid = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(((uint64_t)nw * n + 255) / 256, (uint64_t)c->sm_count * 8));
+        if (qj.count) k_query_gather<true><<<ggrid, 256, 0, st>>>(gp);
+        else k_query_gather<false><<<ggrid, 256, 0, st>>>(gp);
+        CU_TRY(c, cudaGetLastError());
+        CU_TRY(c, cudaMemcpyAsync(sc, c->scalars.p, sizeof sc, cudaMemcpyDeviceToHost, st));
+        uint32_t wd = w0;
+        if (w0 < next_word) {                   // only counter ranges share a word row with the range before
+            CU_TRY(c, cudaMemcpyAsync(boundary.data(), c->qout.p, n * 8, cudaMemcpyDeviceToHost, st));
+            wd = w0 + 1;
+        }
+        if (w1 > wd) CU_TRY(c, cudaMemcpyAsync(dst + (uint64_t)wd * n, (const uint64_t*)c->qout.p + (uint64_t)(wd - w0) * n,
+                                               (uint64_t)(w1 - wd) * n * 8, cudaMemcpyDeviceToHost, st));
+        CU_TRY(c, cudaStreamSynchronize(st));
+        if (wd > w0) for (uint64_t i = 0; i < n; ++i) dst[(uint64_t)w0 * n + i] |= boundary[i];
+        next_word = w1;
+        qs.n_records += sc[S_N_RECORDS];
+        qs.n_bases += sc[S_STREAM_TOTAL] - sc[S_N_RECORDS];
+    }
+    uint64_t tot[2] = {0, 0};
+    CU_TRY(c, cudaMemcpyAsync(tot, d_totals, 16, cudaMemcpyDeviceToHost, st));
+    CU_TRY(c, cudaEventRecord(c->ev_query[1], st));
+    CU_TRY(c, cudaStreamSynchronize(st));
+    qs.n_windows = tot[0]; qs.n_hits = tot[1]; qs.n_jobs = n_ranges;
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, c->ev_query[0], c->ev_query[1]) == cudaSuccess) qs.ms = ms; else cudaGetLastError();
+    return GRMKM_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int grmkm_query(grmkm_ctx* c, const uint64_t* kmers, uint64_t n_kmers, uint64_t* dst, uint64_t cap, grmkm_query_stats* stats) {
+    if (check_ctx(c)) return GRMKM_E_INVALID;
+    if (stats && stats->struct_size != sizeof(grmkm_query_stats))
+        return fail(c, GRMKM_E_INVALID, "stats->struct_size must be sizeof(grmkm_query_stats)");
+    if (c->cfg.flags & GRMKM_FLAG_COUNTS) return fail(c, GRMKM_E_INVALID, "a pooled count table has no genome rows to query");
+    if (n_kmers && !kmers) return fail(c, GRMKM_E_INVALID, "null k-mer list");
+    if (n_kmers > 0xFFFFFFFFULL) return fail(c, GRMKM_E_INVALID, "at most 2^32 - 1 k-mers in one query");
+    const uint32_t k = c->cfg.k;
+    if (k < 32)
+        for (uint64_t i = 0; i < n_kmers; ++i)
+            if (kmers[i] >> (2 * k))
+                return fail(c, GRMKM_E_INVALID, "k-mer " + std::to_string(i) + " is not below 4^k (k = " + std::to_string(k) + ")");
+    uint32_t G = c->n_genomes_decl;
+    grmkm_query_stats qs{};
+    qs.struct_size = sizeof qs;
+    for (const Input& in : c->inputs) { G = std::max(G, in.row + 1); qs.n_input_bytes += in.len; }
+    const uint64_t need = (uint64_t)((G + 63) / 64) * n_kmers;
+    if (cap < need) return fail(c, GRMKM_E_CAPACITY, "dst holds fewer than ceil(G/64) x n_kmers words");
+    if (need && !dst) return fail(c, GRMKM_E_INVALID, "null dst");
+    if (need) {
+        NvtxRange nv("grmkm_query");
+        const int r = query_impl(c, kmers, n_kmers, dst, G, qs);
+        if (r != GRMKM_OK) {
+            // nothing in flight reads the caller's buffers any more, and no side-stream clear is counted on
+            const std::string msg = c->err;
+            cudaStreamSynchronize(c->stream);
+            if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
+            if (c->aux_stream) cudaStreamSynchronize(c->aux_stream);
+            cudaGetLastError();
+            c->pre_pending = false;
+            c->err = msg;
+            return r;
+        }
+    }
+    if (stats) *stats = qs;
     return GRMKM_OK;
 }
 

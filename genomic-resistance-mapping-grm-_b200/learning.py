@@ -91,6 +91,35 @@ class KmerRuleClassifications:
 _BASE_CODE = np.full(256, 255, dtype=np.uint64)
 for _i, _b in enumerate(b"ACTG"):                       # the library's packing: A0 C1 T2 G3, first base most significant
     _BASE_CODE[_b] = _i
+    _BASE_CODE[_b | 0x20] = _i                          # lower case: the same base
+
+
+def kmers_from_strings(seqs, k: int) -> np.ndarray:
+    """k-mer strings (str, bytes or a numpy bytes array) -> packed uint64, as ``KmerMatrixBuilder.kmers`` returns
+    them (A0 C1 T2 G3, first base most significant).  Upper and lower case are accepted; a string that is not k
+    characters long, or a character other than A, C, G, T, raises ValueError."""
+    k = int(k)
+    if not 1 <= k <= 32:
+        raise ValueError(f"k must be in 1..32, not {k}")
+    if isinstance(seqs, np.ndarray) and seqs.dtype.kind == "S":
+        n = len(seqs)
+        if n and (seqs.dtype.itemsize != k or (np.char.str_len(seqs) != k).any()):
+            raise ValueError(f"every k-mer must be {k} characters long")
+        raw = np.frombuffer(np.ascontiguousarray(seqs).tobytes(), dtype=np.uint8)
+    else:
+        items = [s.encode("latin-1", "replace") if isinstance(s, str) else bytes(s) for s in seqs]
+        n = len(items)
+        bad = next((s for s in items if len(s) != k), None)
+        if bad is not None:
+            raise ValueError(f"every k-mer must be {k} characters long, not {bad!r}")
+        raw = np.frombuffer(b"".join(items), dtype=np.uint8)
+    codes = _BASE_CODE[raw.reshape(n, k)]
+    if (codes == 255).any():
+        raise ValueError("a k-mer holds a character other than A, C, G, T")
+    kmers = np.zeros(n, dtype=np.uint64)
+    for i in range(k):
+        kmers = (kmers << np.uint64(2)) | codes[:, i]
+    return kmers
 
 
 def load_kover(path: str, builder) -> KmerRuleClassifications:
@@ -105,11 +134,8 @@ def load_kover(path: str, builder) -> KmerRuleClassifications:
     k = seqs.dtype.itemsize
     if len(seqs) and k != builder.k:
         raise ValueError(f"{path} holds {k}-mers, the builder counts {builder.k}-mers")
-    codes = _BASE_CODE[np.frombuffer(seqs.tobytes(), dtype=np.uint8).reshape(len(seqs), k)]
-    if (codes == 255).any():
+    if len(seqs) and not np.isin(np.frombuffer(seqs.tobytes(), dtype=np.uint8), np.frombuffer(b"ACGT", dtype=np.uint8)).all():
         raise ValueError(f"{path}: kmer_sequences holds a character other than A, C, G, T")
-    kmers = np.zeros(len(seqs), dtype=np.uint64)
-    for i in range(k):
-        kmers = (kmers << np.uint64(2)) | codes[:, i]
+    kmers = kmers_from_strings(seqs, k) if len(seqs) else np.zeros(0, dtype=np.uint64)
     builder.load_result(kmers, matrix, n_genomes)
     return KmerRuleClassifications(builder, n_genomes)

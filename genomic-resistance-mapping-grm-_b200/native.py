@@ -6,7 +6,7 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("GRMKM_LIB") or os.path.join(_HERE, "libgrmkm.so")   # GRMKM_LIB: another build of the same library (kernel experiments)
-ABI_VERSION = 12
+ABI_VERSION = 13
 
 OK = 0
 E_INVALID, E_UNSUPPORTED_K, E_NOMEM, E_CUDA, E_IO, E_CAPACITY, E_NO_DEVICE, E_UNSUPPORTED = -1, -2, -3, -4, -5, -6, -7, -8
@@ -23,7 +23,7 @@ SYMBOLS = [
     "grmkm_plan_bucket_bits", "grmkm_set_bucket_bits", "grmkm_set_exchange_rank",
     "grmkm_result_checksum", "grmkm_sum_rows", "grmkm_gram", "grmkm_tsv_pack",
     "grmkm_load_result", "grmkm_scm_run", "grmkm_scm_result",
-    "grmkm_cart_run", "grmkm_cart_result",
+    "grmkm_cart_run", "grmkm_cart_result", "grmkm_query",
 ]
 SCM_CONJUNCTION, SCM_DISJUNCTION = 0, 1
 
@@ -84,6 +84,15 @@ class CartNode(C.Structure):
                 ("equiv_total", C.c_uint64)]
 
 
+class QueryStats(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("n_jobs", C.c_uint32), ("n_queries", C.c_uint64),
+                ("n_bases", C.c_uint64), ("n_windows", C.c_uint64), ("n_records", C.c_uint64),
+                ("n_input_bytes", C.c_uint64), ("n_hits", C.c_uint64), ("ms", C.c_float)]
+
+    def asdict(self):
+        return {n: (float if n == "ms" else int)(getattr(self, n)) for n, _ in self._fields_ if n != "struct_size"}
+
+
 _lib = None
 
 
@@ -136,6 +145,7 @@ def load() -> C.CDLL:
         "grmkm_scm_result": (i32, [vp, u32, vp, u64, C.POINTER(u64), vp, u64, C.POINTER(u64)]),
         "grmkm_cart_run": (i32, [vp, u32, vp, vp, u64]),
         "grmkm_cart_result": (i32, [vp, u32, vp, u64, C.POINTER(u64), vp, u64, C.POINTER(u64)]),
+        "grmkm_query": (i32, [vp, vp, u64, vp, u64, C.POINTER(QueryStats)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)

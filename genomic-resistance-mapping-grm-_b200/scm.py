@@ -49,10 +49,21 @@ class SetCoveringMachine:
         """0/1 per example (row indices among the rows not removed), from the <= max_rules columns of the model."""
         example_idx = np.asarray(example_idx, dtype=np.int64)
         if not self.rule_indices:
-            return np.full(len(example_idx), 1 if self.model_type == "conjunction" else 0, dtype=np.uint8)
-        cols = rule_classifications.get_columns(self.rule_indices)[example_idx]
-        out = cols.all(axis=1) if self.model_type == "conjunction" else cols.any(axis=1)
-        return out.astype(np.uint8)
+            return _scm_output(self.model_type, np.zeros((len(example_idx), 0), dtype=np.uint8))
+        return _scm_output(self.model_type, rule_classifications.get_columns(self.rule_indices)[example_idx])
+
+    def predict_genomes(self, builder) -> np.ndarray:
+        """0/1 per genome row of the inputs of ``builder`` (a KmerMatrixBuilder holding genomes that need not have
+        been in the training matrix): one ``builder.query`` of the model's k-mers, no build (predict.predict_genomes)."""
+        from .predict import predict_genomes
+        return predict_genomes([self], builder)[0]
+
+
+def _scm_output(model_type: str, cols: np.ndarray) -> np.ndarray:
+    """The model's output from the 0/1 values of its rules (examples x rules, absence rules already inverted): all of
+    them for a conjunction, any of them for a disjunction (an empty model: 1 and 0)."""
+    out = cols.all(axis=1) if model_type == "conjunction" else cols.any(axis=1)
+    return out.astype(np.uint8)
 
 
 def _refuse_slices(rule_classifications):

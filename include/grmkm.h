@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define GRMKM_ABI_VERSION 12
+#define GRMKM_ABI_VERSION 13
 
 enum {
     GRMKM_OK = 0,
@@ -336,6 +336,40 @@ int grmkm_cart_run(grmkm_ctx* ctx, uint32_t n_trees, const grmkm_cart_job* jobs,
  * GRMKM_E_CAPACITY (sizes still written). */
 int grmkm_cart_result(grmkm_ctx* ctx, uint32_t tree, grmkm_cart_node* nodes, uint64_t nodes_cap, uint64_t* n_nodes,
                       uint64_t* equivalent, uint64_t equiv_cap, uint64_t* n_equivalent);
+
+/*
+ * Query: which genome rows of the inputs hold which k-mers, without building their matrix (a fitted model applied to
+ * new genomes: its rules' k-mers; a marker panel: the k-mers of known genes).
+ *
+ * kmers[i] is packed as grmkm_copy_kmers_packed returns it (A0 C1 T2 G3, first base most significant, < 4^k), on
+ * either strand; duplicates are allowed.  Column i of the answer is about canonical(kmers[i]) = min(forward, reverse
+ * complement), the complement of code c being c ^ 2.  Genome g has column i set iff, among the valid k-mer windows of
+ * g's inputs (the windows, records and FASTA/FASTQ rules of a build), at least min_abundance have the canonical k-mer
+ * canonical(kmers[i]): the per-genome solid set before the singleton filter, so keep_singletons plays no part.  For a
+ * k-mer that is a column of a build of the same inputs, the query column equals the matrix column bit for bit; every
+ * other k-mer gives zeros, except a k-mer of exactly one genome when the build drops singletons.
+ *
+ * dst: row-major ceil(G/64) x n_kmers words, genome g at bit 63 - g % 64 of word row g / 64 (the matrix's layout), G
+ * the genome count a build of these inputs would have (max row + 1, or grmkm_set_genome_count).
+ *
+ * The call reads the inputs added since the last reset, as grmkm_build does, and keeps them: a build or another query
+ * can follow.  It changes nothing else in the context: the resident result, grmkm_get_stats, grmkm_stage_times and the
+ * SCM and CART results stay as they are (grmkm_stats.device_bytes is the memory the context holds at the time of the
+ * call, and counts the buffers a query keeps for the next one).  Rejected before any device work: a k-mer >= 4^k and a bad
+ * stats->struct_size (GRMKM_E_INVALID), a GRMKM_FLAG_COUNTS context (GRMKM_E_INVALID: pooled counts have no genome
+ * rows), cap < ceil(G/64) * n_kmers (GRMKM_E_CAPACITY).  n_kmers = 0 or G = 0 is valid and writes nothing.
+ */
+typedef struct grmkm_query_stats {
+    uint32_t struct_size;     /* = sizeof(grmkm_query_stats) */
+    uint32_t n_jobs;          /* row ranges the call was split into (each a pass over its rows' inputs) */
+    uint64_t n_queries;       /* distinct canonical k-mers in the query */
+    uint64_t n_bases, n_windows, n_records, n_input_bytes;   /* as grmkm_stats, for the queried inputs */
+    uint64_t n_hits;          /* valid windows whose canonical k-mer is in the set */
+    float ms;                 /* device time of the call, CUDA events */
+} grmkm_query_stats;
+
+int grmkm_query(grmkm_ctx* ctx, const uint64_t* kmers, uint64_t n_kmers, uint64_t* dst, uint64_t cap,
+                grmkm_query_stats* stats /* may be NULL */);
 
 #ifdef __cplusplus
 }
