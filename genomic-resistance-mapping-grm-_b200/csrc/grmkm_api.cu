@@ -111,7 +111,6 @@ struct grmkm_ctx {
         qout;            // grmkm_query: one row range's word rows in the caller's column order
     cudaEvent_t ev_query[2] = {nullptr, nullptr};   // grmkm_query: device time of the call
     uint64_t racc_hint = 0;        // records of the previous abundance build + headroom
-    uint32_t pack_ctas[2] = {0, 0};      // resident CTAs of the persistent k_pack (FASTA / FASTQ)
     std::vector<uint64_t> merge_h_off;   // row-block merge of a partial build: chunk offsets of the merge buckets
     uint32_t merge_bits = 0;
     uint64_t merge_cap = 0;
@@ -623,39 +622,8 @@ int run_job(grmkm_ctx* c, const Geo& geo, const Job& job, JobOut& out) {
         pp.pub_a0 = (unsigned long long*)c->tile_pub.p; pp.pub_a1 = pp.pub_a0 + n_tiles; pp.pub_ps = pp.pub_a0 + 2 * n_tiles;
         pp.stream_len = bt.stream;
         pp.codes = (unsigned long long*)c->codes.p; pp.valid = (uint32_t*)c->valid.p; pp.scalars = d_scalars;
-        // files of very many tiles: summaries first, the chains resolved by a scan, so that the pack itself never waits
-        // (k_scan_tile_chains)
-        const bool two_pass = getenv("GRMKM_TWO_PASS") != nullptr;        // measured on 300 MB read sets: the second read of the text costs more than the chain (DESIGN.md 4a)
-        if (two_pass) {
-            if (c->cfg.input_kind == GRMKM_FASTA) {
-                k_pack<0, true><<<(uint32_t)n_tiles, kParseThreads, 0, st>>>(pp);
-                k_scan_tile_chains<0><<<(F * 32 + 127) / 128, 128, 0, st>>>(d_files, F, (const uint64_t*)c->fss.p, n_tiles, pp.pub_a0, pp.pub_a1, pp.pub_ps);
-            } else {
-                k_pack<1, true><<<(uint32_t)n_tiles, kParseThreads, 0, st>>>(pp);
-                k_scan_tile_chains<1><<<(F * 32 + 127) / 128, 128, 0, st>>>(d_files, F, (const uint64_t*)c->fss.p, n_tiles, pp.pub_a0, pp.pub_a1, pp.pub_ps);
-            }
-            CU_TRY(c, cudaMemsetAsync(pp.ticket, 0, 4, st));
-            out.launches += 2;
-        }
-        if (getenv("GRMKM_PACK_TMA")) {
-            // persistent CTAs (exactly what is resident at once), the next tile's text fetched by cp.async.bulk under the
-            // current tile's parse.  Measured against the one-tile-per-CTA kernel on C2 (profiles/r02_pack_tma_ab.txt):
-            // 0.85 ms instead of 0.63 ms -- the resident CTAs serialise on their own look-back waits, while the hardware
-            // scheduler refills an SM with a fresh tile as soon as any CTA exits -- so it is kept as an option, not the
-            // default.
-            const int kind = c->cfg.input_kind == GRMKM_FASTA ? 0 : 1;
-            if (!c->pack_ctas[kind]) {
-                int occ = 0;
-                CU_TRY(c, kind ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_pack<1, false, true>, kParseThreads, 0)
-                               : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_pack<0, false, true>, kParseThreads, 0));
-                if (occ < 1) return fail(c, GRMKM_E_CUDA, "k_pack does not fit an SM");
-                c->pack_ctas[kind] = (uint32_t)occ * (uint32_t)c->sm_count;
-            }
-            const uint32_t pgrid = (uint32_t)std::min<uint64_t>(n_tiles, c->pack_ctas[kind]);
-            if (kind) k_pack<1, false, true><<<pgrid, kParseThreads, 0, st>>>(pp);
-            else k_pack<0, false, true><<<pgrid, kParseThreads, 0, st>>>(pp);
-        } else if (c->cfg.input_kind == GRMKM_FASTA) k_pack<0><<<(uint32_t)n_tiles, kParseThreads, 0, st>>>(pp);
-        else k_pack<1><<<(uint32_t)n_tiles, kParseThreads, 0, st>>>(pp);
+        const auto pack = c->cfg.input_kind == GRMKM_FASTA ? k_pack<0> : k_pack<1>;
+        pack<<<(uint32_t)n_tiles, kParseThreads, 0, st>>>(pp);
         out.launches++;
         CU_TRY(c, cudaGetLastError());
         if (timed && c->ev_ok) cudaEventRecord(c->ev[T_PACK], st);
@@ -688,7 +656,7 @@ int run_job(grmkm_ctx* c, const Geo& geo, const Job& job, JobOut& out) {
     // codes / valid / tile words are dead once the last batch has been scattered (or scanned): clear them for the next
     // build or query (or the next pass) on the side stream, under whatever the stream runs next
     auto preclear = [&]() -> int {
-        if (!c->pass_groups || getenv("GRMKM_NO_PRECLEAR")) return GRMKM_OK;
+        if (!c->pass_groups) return GRMKM_OK;
         if (!c->aux_stream) {
             CU_TRY(c, cudaStreamCreateWithFlags(&c->aux_stream, cudaStreamNonBlocking));
             CU_TRY(c, cudaEventCreateWithFlags(&c->ev_scattered, cudaEventDisableTiming));
@@ -757,7 +725,7 @@ int run_job(grmkm_ctx* c, const Geo& geo, const Job& job, JobOut& out) {
         NvtxRange nv_front("grmkm front: stage / pack / unit bounds / unit scatter");
         std::unique_lock<std::mutex> gate;
         cudaEvent_t* gate_ev = nullptr;
-        if (any_host && c->device >= 0 && c->device < 64 && !getenv("GRMKM_NO_H2D_GATE")) {
+        if (any_host && c->device >= 0 && c->device < 64) {
             gate = std::unique_lock<std::mutex>(g_h2d.mu);
             gate_ev = &g_h2d.done[c->device];
             if (!*gate_ev) CU_TRY(c, cudaEventCreateWithFlags(gate_ev, cudaEventDisableTiming));

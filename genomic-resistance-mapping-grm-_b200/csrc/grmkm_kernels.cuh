@@ -278,46 +278,6 @@ __device__ __noinline__ void tile_lookback_fa(uint64_t tile, uint64_t first, uin
     }
 }
 
-// Two-pass parse for very long files.  The look-back resolves a file's tiles one after the other in the worst case,
-// and with a handful of files of tens of thousands of tiles each (a 300 MB read set is 19 k tiles) almost every tile
-// waits for its predecessor: 8.5 ms for 620 MB.  Such inputs get a first pass that only publishes the tile summaries
-// (k_pack<KIND, true>: the text is read once more, at HBM speed) and this scan -- one warp per file, 32 tiles per step --
-// which resolves every tile's incoming (state, position).  The real k_pack then finds its predecessor resolved at
-// its first poll.
-template <int KIND>
-__global__ void __launch_bounds__(128)
-k_scan_tile_chains(const FileDesc* __restrict__ files, uint32_t n_files, const uint64_t* __restrict__ fss, uint64_t n_tiles,
-                   const unsigned long long* __restrict__ a0, const unsigned long long* __restrict__ a1,
-                   unsigned long long* __restrict__ ps) {
-    const uint32_t f = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const int lane = threadIdx.x & 31;
-    if (f >= n_files) return;
-    const uint64_t t0 = files[f].tile_begin, t1 = f + 1 < n_files ? files[f + 1].tile_begin : n_tiles;
-    uint32_t st = 0;                              // every file starts in state 0 at its own stream position
-    uint64_t pos = fss[f];
-    for (uint64_t base = t0; base < t1; base += 32) {
-        const uint64_t t = base + lane;
-        Sum mine = sum_identity();
-        if (t < t1) mine = pub_sum(a0[t], KIND == 1 ? a1[t] : kPubValid);
-        Sum inc = mine;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            const Sum o = sum_shfl_up(inc, d);
-            if (lane >= d) inc = sum_comb<KIND == 1>(o, inc);
-        }
-        Sum excl = sum_shfl_up(inc, 1);
-        if (lane == 0) excl = sum_identity();
-        if (t < t1) ps[t] = kPubValid | ((unsigned long long)sum_end(excl, st) << 61) | (pos + sum_cnt(excl, st));
-        const uint32_t e_all = __shfl_sync(0xffffffffu, inc.e, 31);
-        Sum all;
-        all.e = e_all;
-        all.c0 = __shfl_sync(0xffffffffu, inc.c0, 31); all.c1 = __shfl_sync(0xffffffffu, inc.c1, 31);
-        all.c2 = __shfl_sync(0xffffffffu, inc.c2, 31); all.c3 = __shfl_sync(0xffffffffu, inc.c3, 31);
-        pos += sum_cnt(all, st);
-        st = sum_end(all, st);
-    }
-}
-
 // text tile -> packed stream: codes64[g] holds entries 32g..32g+31 (entry j at bits 2j), valid32[g] bit j.
 // Every thread turns its 64 bytes into at most 64 entries (register accumulator), the block scan of the
 // thread summaries gives each thread its entry offset inside the tile, the look-back gives the tile its state and
@@ -338,39 +298,7 @@ struct PackParams {
     uint64_t* scalars;
 };
 
-// ---- bulk asynchronous copies (TMA, 1-D): global -> shared, completion counted in bytes on an mbarrier -----------
-// SASS: UBLKCP.S.G / SYNCS.ARRIVE.TRANS64 / SYNCS.PHASECHK.  Source, destination and size are multiples of 16 bytes.
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t mbar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(mbar), "r"(count) : "memory");
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t mbar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mbar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t mbar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(mbar) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t mbar, uint32_t parity) {
-    uint32_t ok;
-    do {
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(ok) : "r"(mbar), "r"(parity) : "memory");
-    } while (!ok);
-}
-// generic-proxy reads of a shared buffer are ordered before the async proxy overwrites it
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
-// TMA: persistent variant.  The grid is what is resident at once (4 CTAs per SM), CTA b takes tickets b, b + grid, ... and
-// the 16 KiB text tile of its NEXT ticket is fetched by one cp.async.bulk into shared memory while the current tile is
-// parsed: the ticket record, the text and its HBM latency are off the tile's critical path, and the text is read with
-// LDS.128 instead of LDG.128.  (Tickets are still started in order -- every CTA is resident and works through its
-// tickets in ascending order, so the smallest unfinished ticket is always being worked on: the look-back cannot
-// deadlock.)
-// SUMMARY_ONLY: publish the tile's summary and stop (first pass of the two-pass parse of very long files, see
-// k_scan_tile_chains).
-template <int KIND, bool SUMMARY_ONLY = false, bool TMA = false>
+template <int KIND>
 #ifndef GRMKM_PACK_CTAS
 #define GRMKM_PACK_CTAS (1024 / kParseThreads)      // resident CTAs per SM the register budget is cut for (A/B: profiles/r02_pack_occupancy_ab.txt)
 #endif
@@ -388,19 +316,30 @@ k_pack(const PackParams p) {
     uint32_t* const s_valid = s_cv + kCodeWords;
     __shared__ uint32_t s_nrec, s_st;
     __shared__ uint64_t s_pos;
-    __shared__ uint4 s_tk[TMA ? 8 : 4];                                 // this CTA's TileTicket (TMA: and the next one)
-    __shared__ __align__(128) uint8_t s_text[TMA ? kTileBytes : 16];    // TMA: the tile's text
-    __shared__ __align__(8) unsigned long long s_mbar;
-    static_assert(!(TMA && SUMMARY_ONLY), "the summary pass is not persistent");
-    auto make_ctx = [&](const TileTicket& tk) {
-        TileCtx t;
-        t.f = tk.f; t.fd = tk.fd; t.hdr0 = tk.hdr0;
-        t.first_tile = (tk.tile == t.fd.tile_begin);
-        t.off = (tk.tile - t.fd.tile_begin) * (uint64_t)kTileBytes + (uint64_t)threadIdx.x * (16 * kChunksPerThread);
-        return t;
-    };
+    __shared__ uint4 s_tk[4];                                           // this CTA's TileTicket
+    // ---- one tile per CTA, tickets from the counter
+    if (threadIdx.x == 0) {
+        const uint32_t ticket = atomicAdd(p.ticket, 1u);
+        s_nrec = 0;
+        if (ticket == 0) p.scalars[S_STREAM_LEN] = p.stream_len;
+        if (ticket < p.n_tiles) {
+            const uint4* src = reinterpret_cast<const uint4*>(p.tickets + ticket);
+            const uint4 a = src[0], b = src[1], c = src[2], d = src[3];
+            s_tk[0] = a; s_tk[1] = b; s_tk[2] = c; s_tk[3] = d;
+        } else {
+            s_tk[3] = make_uint4(0xFFFFFFFFu, 0u, 0u, 0u);                 // no tile left
+        }
+    }
+    for (int i = threadIdx.x; i < kCvVec; i += kParseThreads) reinterpret_cast<uint4*>(s_cv)[i] = make_uint4(0u, 0u, 0u, 0u);
+    __syncthreads();
+    const TileTicket& tk = *reinterpret_cast<const TileTicket*>(s_tk);
+    if (tk.tile == 0xFFFFFFFFu) return;
+    TileCtx t;
+    t.f = tk.f; t.fd = tk.fd; t.hdr0 = tk.hdr0;
+    t.first_tile = (tk.tile == t.fd.tile_begin);
+    t.off = (tk.tile - t.fd.tile_begin) * (uint64_t)kTileBytes + (uint64_t)threadIdx.x * (16 * kChunksPerThread);
+    const ThreadText x = load_thread_text(t);
     // ---- everything after the thread's 64 bytes are in registers
-    auto tile_body = [&](const TileTicket& tk, const TileCtx& t, const ThreadText& x) {
     const uint64_t tile = tk.tile;
     unsigned long long* __restrict__ codes = p.codes;
     uint32_t* __restrict__ valid = p.valid;
@@ -440,7 +379,6 @@ k_pack(const PackParams p) {
         uint32_t ex, tot;
         block_scan_fa(mine, ex, tot, reinterpret_cast<uint32_t*>(s_w));
         publish(fa_to_sum(tot));
-        if (SUMMARY_ONLY) return;
         // The entries are accumulated while the look-back is still in flight, as if the tile started inside a sequence
         // line; the few threads in front of the tile's first line start redo it when it started inside a header.
         const uint32_t ex_t = ex >> kFaT;
@@ -487,7 +425,6 @@ k_pack(const PackParams p) {
         }
         block_scan_sum<true>(mine, excl, total, s_w);
         publish(total);
-        if (SUMMARY_ONLY) return;
         resolve(st_in, tpos);
         uint32_t st = sum_end(excl, st_in);
         local = sum_cnt(excl, st_in);
@@ -584,109 +521,6 @@ k_pack(const PackParams p) {
     if (threadIdx.x == 0) {
         if (s_nrec) atomicAdd((unsigned long long*)&p.scalars[S_N_RECORDS], (unsigned long long)s_nrec);
         if (e_total) atomicAdd((unsigned long long*)&p.scalars[S_STREAM_TOTAL], (unsigned long long)e_total);
-    }
-    };  // tile_body
-
-    if (!TMA) {
-        // ---- one tile per CTA, tickets from the counter
-        if (threadIdx.x == 0) {
-            const uint32_t ticket = atomicAdd(p.ticket, 1u);
-            s_nrec = 0;
-            if (ticket == 0) p.scalars[S_STREAM_LEN] = p.stream_len;
-            if (ticket < p.n_tiles) {
-                const uint4* src = reinterpret_cast<const uint4*>(p.tickets + ticket);
-                const uint4 a = src[0], b = src[1], c = src[2], d = src[3];
-                s_tk[0] = a; s_tk[1] = b; s_tk[2] = c; s_tk[3] = d;
-            } else {
-                s_tk[3] = make_uint4(0xFFFFFFFFu, 0u, 0u, 0u);                 // no tile left
-            }
-        }
-        for (int i = threadIdx.x; i < kCvVec; i += kParseThreads) reinterpret_cast<uint4*>(s_cv)[i] = make_uint4(0u, 0u, 0u, 0u);
-        __syncthreads();
-        const TileTicket& tk = *reinterpret_cast<const TileTicket*>(s_tk);
-        if (tk.tile == 0xFFFFFFFFu) return;
-        const TileCtx t = make_ctx(tk);
-        const ThreadText x = load_thread_text(t);
-        tile_body(tk, t, x);
-        return;
-    }
-
-    // ---- persistent: the next ticket's text travels while this tile is parsed.  Tickets still come from the counter (a
-    // statically dealt tile could start later than a tile that waits for it): the ticket NUMBER is taken two tiles ahead,
-    // its record is loaded one tile ahead, so neither latency is on a tile's critical path.
-    const uint32_t mbar = smem_u32(&s_mbar), text = smem_u32(s_text);
-    auto issue = [&](const uint4 (&rec)[4]) {                 // thread 0: arm the barrier, start the bulk copy
-        const TileTicket& k = *reinterpret_cast<const TileTicket*>(rec);
-        const uint64_t off = (uint64_t)(k.tile - k.fd.tile_begin) * kTileBytes;
-        const uint64_t avail = k.fd.len > off ? k.fd.len - off : 0;
-        const uint32_t nb = (uint32_t)(avail < (uint64_t)kTileBytes ? avail : (uint64_t)kTileBytes) & ~15u;   // whole 16-byte chunks
-        fence_proxy_async();
-        mbar_expect_tx(mbar, nb);
-        if (nb) bulk_g2s(text, k.fd.ptr + off, nb, mbar);
-    };
-    const uint64_t n_tiles = p.n_tiles;
-    uint32_t tk1 = 0xFFFFFFFFu;                               // thread 0: ticket number of the next iteration
-    if (threadIdx.x == 0) {
-        mbar_init(mbar, 1);
-        const uint32_t t0 = atomicAdd(p.ticket, 1u);
-        tk1 = atomicAdd(p.ticket, 1u);
-        if (t0 == 0) p.scalars[S_STREAM_LEN] = p.stream_len;
-        if (t0 < n_tiles) {
-            const uint4* src = reinterpret_cast<const uint4*>(p.tickets + t0);
-            uint4 rec[4] = {src[0], src[1], src[2], src[3]};
-            s_tk[0] = rec[0]; s_tk[1] = rec[1]; s_tk[2] = rec[2]; s_tk[3] = rec[3];
-            issue(rec);
-        } else {
-            s_tk[3] = make_uint4(0xFFFFFFFFu, 0u, 0u, 0u);     // no tile at all for this CTA
-        }
-    }
-    __syncthreads();
-    for (uint32_t it = 0;; ++it) {
-        const uint32_t cur = (it & 1u) * 4u;
-        const TileTicket& tk = *reinterpret_cast<const TileTicket*>(s_tk + cur);
-        if (tk.tile == 0xFFFFFFFFu) break;
-        uint4 nxt[4];
-        uint32_t tk2 = 0xFFFFFFFFu;
-        const bool more = threadIdx.x == 0 && tk1 < n_tiles;
-        if (more) {                                            // record of the next ticket, number of the one after: both in flight
-            const uint4* src = reinterpret_cast<const uint4*>(p.tickets + tk1);
-            nxt[0] = src[0]; nxt[1] = src[1]; nxt[2] = src[2]; nxt[3] = src[3];
-            tk2 = atomicAdd(p.ticket, 1u);
-        }
-        for (int i = threadIdx.x; i < kCvVec; i += kParseThreads) reinterpret_cast<uint4*>(s_cv)[i] = make_uint4(0u, 0u, 0u, 0u);
-        if (threadIdx.x == 0) s_nrec = 0;
-        const TileCtx t = make_ctx(tk);
-        mbar_wait(mbar, it & 1u);
-        ThreadText x;
-#pragma unroll
-        for (int c = 0; c < kChunksPerThread; ++c) {
-            const uint64_t off = t.off + 16 * c;
-            if (off + 16 <= t.fd.len) {
-                const uint4 v = *reinterpret_cast<const uint4*>(s_text + threadIdx.x * (16 * kChunksPerThread) + 16 * c);
-                x.ch[c].w[0] = v.x; x.ch[c].w[1] = v.y; x.ch[c].w[2] = v.z; x.ch[c].w[3] = v.w;
-            } else {
-                x.ch[c] = load_chunk(t.fd.ptr, off, t.fd.len);           // the file's last, partial chunk (or nothing)
-            }
-        }
-        {
-            uint32_t pb = __shfl_up_sync(0xffffffffu, x.ch[kChunksPerThread - 1].byte(15), 1);
-            if ((threadIdx.x & 31) == 0) pb = (t.off > 0 && t.off - 1 < t.fd.len) ? t.fd.ptr[t.off - 1] : (uint32_t)'\n';
-            x.prev[0] = pb;
-#pragma unroll
-            for (int c = 1; c < kChunksPerThread; ++c) x.prev[c] = x.ch[c - 1].byte(15);
-        }
-        __syncthreads();                                       // the text is in registers, the tile arrays are clear
-        if (threadIdx.x == 0) {
-            if (more) {
-                s_tk[(cur ^ 4u) + 0] = nxt[0]; s_tk[(cur ^ 4u) + 1] = nxt[1]; s_tk[(cur ^ 4u) + 2] = nxt[2]; s_tk[(cur ^ 4u) + 3] = nxt[3];
-                issue(nxt);
-            } else {
-                s_tk[(cur ^ 4u) + 3] = make_uint4(0xFFFFFFFFu, 0u, 0u, 0u);
-            }
-            tk1 = tk2;
-        }
-        tile_body(tk, t, x);
-        __syncthreads();                                       // the tile arrays are free again, the next ticket is visible
     }
 }
 

@@ -540,11 +540,10 @@ def test_row_blocks_in_partial_builds(gpu):
     _emulated_ranks(3, 1000, True)
 
 
-def test_two_pass_parse_of_long_files(gpu, monkeypatch):
-    """Files of very many tiles are parsed in two passes (tile summaries, a chain scan, then the pack finds every
-    predecessor resolved); GRMKM_TWO_PASS=1 forces it on inputs of a few tiles per file, FASTA and FASTQ, with the
-    quirks that change the parser state across tile borders."""
-    monkeypatch.setenv("GRMKM_TWO_PASS", "1")
+def test_parse_quirks_of_long_files(gpu):
+    """Files of several tiles each, FASTA and FASTQ, with the quirks that change the parser state across tile borders
+    (CR-LF, blank lines, a junk prefix, no final newline, a header longer than two tiles): every tile's incoming state
+    and stream position come from the look-back over its file's earlier tiles."""
     rng = np.random.default_rng(99)
     shared = [inputs.rand_seq(rng, 90_000)]
     genomes = [[inputs.fasta(rng, n_records=4, min_len=30_000, max_len=70_000, shared=shared, crlf=(g == 1), blank=(g == 2),
