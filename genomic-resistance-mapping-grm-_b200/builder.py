@@ -292,6 +292,36 @@ class KmerMatrixBuilder:
             out.append((nodes, eq))
         return out
 
+    EVAL_NODE_DTYPE = np.dtype([("kmer", np.uint64), ("present_child", np.uint32), ("absent_child", np.uint32)])
+
+    def eval_run(self, jobs) -> list[np.ndarray]:
+        """Fitted models scored on example sets of the resident matrix, all in one grmkm_eval_run (one launch, one copy
+        of the counts).  jobs: (kind, model_type, items, pos_mask, neg_mask) with masks of ceil(G/64) uint64 words.
+        kind native.EVAL_SCM: items = the model's rule indices (< 2U), model_type native.SCM_CONJUNCTION / _DISJUNCTION
+        -> (R + 1, 2) counts (fn, fp) of the prefixes of 0..R rules.  kind native.EVAL_CART: model_type 0, items = nodes
+        with the fields of EVAL_NODE_DTYPE (kmer UINT64_MAX: leaf) -> (n, 2) counts (pos, neg) of the examples reaching
+        each node."""
+        _, W, _ = self.dims
+        keep, arr, sizes = [], (native.EvalJob * max(1, len(jobs)))(), []
+        for i, (kind, model_type, items, pos, neg) in enumerate(jobs):
+            pos = np.ascontiguousarray(pos, dtype=np.uint64)
+            neg = np.ascontiguousarray(neg, dtype=np.uint64)
+            if pos.shape != (W,) or neg.shape != (W,):
+                raise ValueError(f"example masks of {pos.shape} / {neg.shape} words for {W} matrix word rows")
+            if kind == native.EVAL_SCM:
+                items = np.ascontiguousarray(np.asarray(items, dtype=np.uint64).reshape(-1))
+                rules, nodes, pairs = items.ctypes.data, None, items.size + 1
+            else:
+                items = np.ascontiguousarray(items, dtype=self.EVAL_NODE_DTYPE).reshape(-1)
+                rules, nodes, pairs = None, items.ctypes.data, items.size
+            keep += [pos, neg, items]
+            sizes.append(pairs)
+            arr[i] = native.EvalJob(C.sizeof(native.EvalJob), int(kind), int(model_type), 0, items.size, rules, nodes,
+                                    pos.ctypes.data, neg.ctypes.data)
+        counts = np.zeros((sum(sizes), 2), dtype=np.uint32)
+        self._check(self._lib.grmkm_eval_run(self._ctx, len(jobs), arr, C.c_void_p(counts.ctypes.data), counts.size))
+        return np.split(counts, np.cumsum(sizes)[:-1]) if sizes else []
+
     @property
     def query_genome_count(self) -> int:
         """G of a build of the inputs added since the last reset: max row + 1, or set_genome_count when larger."""

@@ -13,8 +13,8 @@ do not depend on the GPU, the batch or the grid.
 
 The tree fitted with ``max_depth = d`` is the depth-d truncation of the tree fitted with any larger ``max_depth``, and
 a larger ``min_samples_split`` only turns internal nodes into leaves, so a max-depth or min-samples grid needs one tree
-per fold and class weighting.  Cost-complexity pruning and hyperparameter selection are the caller's: CV composes from
-``fit_many`` and ``predict``.
+per fold and class weighting; ``model_selection.cross_validate_cart`` scores such a grid from one tree per fold and
+picks its hyperparameters.  Cost-complexity pruning is the caller's.
 """
 from __future__ import annotations
 

@@ -8,6 +8,7 @@
 #include "grmkm_scm.cuh"
 #include "grmkm_cart.cuh"
 #include "grmkm_query.cuh"
+#include "grmkm_eval.cuh"
 
 #include <nvtx3/nvToolsExt.h>      // header-only; the ranges cost nothing until a tool (nsys, ncu --nvtx) attaches
 #include <zlib.h>
@@ -108,7 +109,8 @@ struct grmkm_ctx {
         cart_list,       // grmkm_cart_run: the tie list
         qry,             // grmkm_query: key table, slot -> key index, caller column -> key index, totals
         qplane,          // grmkm_query: presence plane or counters of one row range
-        qout;            // grmkm_query: one row range's word rows in the caller's column order
+        qout,            // grmkm_query: one row range's word rows in the caller's column order
+        eval;            // grmkm_eval_run: job arguments, rules, nodes, example masks, counts
     cudaEvent_t ev_query[2] = {nullptr, nullptr};   // grmkm_query: device time of the call
     uint64_t racc_hint = 0;        // records of the previous abundance build + headroom
     std::vector<uint64_t> merge_h_off;   // row-block merge of a partial build: chunk offsets of the merge buckets
@@ -1404,7 +1406,7 @@ void grmkm_destroy(grmkm_ctx* c) {
                      &c->bcounts, &c->ukeys, &c->uwords, &c->kmers, &c->matrix, &c->scalars, &c->fmt, &c->synth, &c->refs,
                      &c->stile_file, &c->bbase, &c->apub, &c->masks, &c->units, &c->ucur, &c->ubeg, &c->wu, &c->wide,
                      &c->racc, &c->aux, &c->scm, &c->scm_list, &c->cart, &c->cart_bl,
-                     &c->cart_masks[0], &c->cart_masks[1], &c->cart_list, &c->qry, &c->qplane, &c->qout};
+                     &c->cart_masks[0], &c->cart_masks[1], &c->cart_list, &c->qry, &c->qplane, &c->qout, &c->eval};
     for (DevBuf* b : all) release(c, *b);
     if (c->ev_ok) for (int i = 0; i < T_N; ++i) cudaEventDestroy(c->ev[i]);
     for (cudaEvent_t e : c->ev_query) if (e) cudaEventDestroy(e);
@@ -2724,6 +2726,117 @@ int grmkm_query(grmkm_ctx* c, const uint64_t* kmers, uint64_t n_kmers, uint64_t*
         }
     }
     if (stats) *stats = qs;
+    return GRMKM_OK;
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------------
+// grmkm_eval_run: fitted models scored on example sets, counts only
+// ------------------------------------------------------------------------------------------------
+static_assert(sizeof(EvalNode) == sizeof(grmkm_eval_node), "EvalNode mirrors grmkm_eval_node");
+
+extern "C" {
+
+int grmkm_eval_run(grmkm_ctx* c, uint32_t n_jobs, const grmkm_eval_job* jobs, uint32_t* counts, uint64_t cap) {
+    if (check_ctx(c)) return GRMKM_E_INVALID;
+    if (!c->built) return fail(c, GRMKM_E_INVALID, "no result: call grmkm_build or grmkm_load_result first");
+    if (c->slice)
+        return fail(c, GRMKM_E_UNSUPPORTED, "the result is one owner's slice of a multi-GPU build: it holds some k-mers only");
+    const uint64_t U = c->U;
+    const uint32_t W = c->W;
+    if (n_jobs && !jobs) return fail(c, GRMKM_E_INVALID, "null jobs");
+    uint64_t pairs = 0, n_rules = 0, n_nodes = 0;
+    std::vector<uint8_t> has_parent;
+    for (uint32_t i = 0; i < n_jobs; ++i) {
+        const grmkm_eval_job& j = jobs[i];
+        const std::string at = " (job " + std::to_string(i) + ")";
+        if (j.struct_size != sizeof(grmkm_eval_job)) return fail(c, GRMKM_E_INVALID, "job struct_size is not sizeof(grmkm_eval_job)" + at);
+        if (j.reserved != 0) return fail(c, GRMKM_E_INVALID, "reserved must be 0" + at);
+        if (j.kind > GRMKM_EVAL_CART) return fail(c, GRMKM_E_INVALID, "unknown job kind" + at);
+        if (j.n_items >= 0xFFFFFFFFULL) return fail(c, GRMKM_E_INVALID, "at most 2^32 - 2 rules or nodes per job" + at);
+        if (j.kind == GRMKM_EVAL_SCM) {
+            if (j.model_type > GRMKM_SCM_DISJUNCTION) return fail(c, GRMKM_E_INVALID, "unknown model type" + at);
+            if (j.n_items && !j.rules) return fail(c, GRMKM_E_INVALID, "null rules" + at);
+            for (uint64_t r = 0; r < j.n_items; ++r)
+                if (j.rules[r] >= 2 * U) return fail(c, GRMKM_E_INVALID, "rule index >= 2 x n_kmers" + at);
+            n_rules += j.n_items;
+            pairs += j.n_items + 1;
+        } else {
+            if (j.model_type != 0) return fail(c, GRMKM_E_INVALID, "model_type of a tree must be 0" + at);
+            if (j.n_items == 0) return fail(c, GRMKM_E_INVALID, "a tree has at least its root node" + at);
+            if (!j.nodes) return fail(c, GRMKM_E_INVALID, "null nodes" + at);
+            const uint64_t n = j.n_items;
+            has_parent.assign(n, 0);
+            for (uint64_t k = 0; k < n; ++k) {
+                const grmkm_eval_node& e = j.nodes[k];
+                if (e.kmer == UINT64_MAX) continue;
+                const std::string nat = " (job " + std::to_string(i) + ", node " + std::to_string(k) + ")";
+                if (e.kmer >= U) return fail(c, GRMKM_E_INVALID, "split k-mer >= n_kmers" + nat);
+                for (uint32_t ch : {e.present_child, e.absent_child}) {
+                    if (ch <= k || ch >= n) return fail(c, GRMKM_E_INVALID, "a child index must be above its parent's and below n" + nat);
+                    if (has_parent[ch]) return fail(c, GRMKM_E_INVALID, "node " + std::to_string(ch) + " has two parents" + at);
+                    has_parent[ch] = 1;
+                }
+            }
+            n_nodes += n;
+            pairs += n;
+        }
+        if (W) {
+            int r = scm_check_mask(c, j.pos, "positive");
+            if (!r) r = scm_check_mask(c, j.neg, "negative");
+            if (r) return r;
+            for (uint32_t w = 0; w < W; ++w)
+                if (j.pos[w] & j.neg[w]) return fail(c, GRMKM_E_INVALID, "positive and negative examples overlap" + at);
+        }
+    }
+    if (cap < 2 * pairs) return fail(c, GRMKM_E_CAPACITY, "counts holds fewer than 2 x the count pairs of the jobs");
+    if (pairs && !counts) return fail(c, GRMKM_E_INVALID, "null counts");
+    if (!pairs) return GRMKM_OK;
+
+    NvtxRange nv("grmkm_eval_run");
+    std::vector<EvalJobArg> args(n_jobs);
+    std::vector<uint64_t> h_rules, h_masks((size_t)n_jobs * 2 * W);
+    std::vector<grmkm_eval_node> h_nodes;
+    h_rules.reserve(n_rules);
+    h_nodes.reserve(n_nodes);
+    uint64_t out = 0;
+    for (uint32_t i = 0; i < n_jobs; ++i) {
+        const grmkm_eval_job& j = jobs[i];
+        const bool scm = j.kind == GRMKM_EVAL_SCM;
+        args[i] = EvalJobArg{scm ? EVAL_SCM : EVAL_CART, (uint32_t)(scm && j.model_type == GRMKM_SCM_CONJUNCTION),
+                             (uint32_t)j.n_items, 0, scm ? h_rules.size() : h_nodes.size(), out};
+        if (scm) h_rules.insert(h_rules.end(), j.rules, j.rules + j.n_items);
+        else h_nodes.insert(h_nodes.end(), j.nodes, j.nodes + j.n_items);
+        out += scm ? j.n_items + 1 : j.n_items;
+        if (W) {
+            memcpy(h_masks.data() + (size_t)i * 2 * W, j.pos, (size_t)W * 8);
+            memcpy(h_masks.data() + (size_t)i * 2 * W + W, j.neg, (size_t)W * 8);
+        }
+    }
+    CU_TRY(c, cudaSetDevice(c->device));
+    auto al = [](size_t b) { return (b + 255) & ~size_t(255); };
+    const size_t o_args = 0, o_rules = al((size_t)n_jobs * sizeof(EvalJobArg)), o_nodes = o_rules + al(n_rules * 8),
+                 o_masks = o_nodes + al(n_nodes * sizeof(EvalNode)), o_cnt = o_masks + al(h_masks.size() * 8),
+                 total = o_cnt + pairs * 8;
+    ENSURE(c, c->eval, total);
+    uint8_t* base = (uint8_t*)c->eval.p;
+    cudaStream_t st = c->stream;
+    CU_TRY(c, cudaMemcpyAsync(base + o_args, args.data(), (size_t)n_jobs * sizeof(EvalJobArg), cudaMemcpyHostToDevice, st));
+    if (n_rules) CU_TRY(c, cudaMemcpyAsync(base + o_rules, h_rules.data(), n_rules * 8, cudaMemcpyHostToDevice, st));
+    if (n_nodes) CU_TRY(c, cudaMemcpyAsync(base + o_nodes, h_nodes.data(), n_nodes * sizeof(EvalNode), cudaMemcpyHostToDevice, st));
+    if (!h_masks.empty()) CU_TRY(c, cudaMemcpyAsync(base + o_masks, h_masks.data(), h_masks.size() * 8, cudaMemcpyHostToDevice, st));
+    CU_TRY(c, cudaMemsetAsync(base + o_cnt, 0, pairs * 8, st));
+    const uint32_t warps_per_cta = kEvalThreads / 32;
+    const uint32_t grid = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((n_jobs + warps_per_cta - 1) / warps_per_cta,
+                                                                              (uint64_t)c->sm_count * 8));
+    k_eval<<<grid, kEvalThreads, 0, st>>>((const unsigned long long*)c->matrix.p, U, c->pitch, W, (const EvalJobArg*)(base + o_args),
+                                          n_jobs, (const unsigned long long*)(base + o_rules), (const EvalNode*)(base + o_nodes),
+                                          (const unsigned long long*)(base + o_masks), (uint32_t*)(base + o_cnt));
+    CU_TRY(c, cudaGetLastError());
+    c->stats.n_launches++;
+    CU_TRY(c, cudaMemcpyAsync(counts, base + o_cnt, pairs * 8, cudaMemcpyDeviceToHost, st));
+    CU_TRY(c, cudaStreamSynchronize(st));
     return GRMKM_OK;
 }
 

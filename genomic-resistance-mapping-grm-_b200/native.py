@@ -6,7 +6,7 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("GRMKM_LIB") or os.path.join(_HERE, "libgrmkm.so")   # GRMKM_LIB: another build of the same library (kernel experiments)
-ABI_VERSION = 13
+ABI_VERSION = 14
 
 OK = 0
 E_INVALID, E_UNSUPPORTED_K, E_NOMEM, E_CUDA, E_IO, E_CAPACITY, E_NO_DEVICE, E_UNSUPPORTED = -1, -2, -3, -4, -5, -6, -7, -8
@@ -23,9 +23,10 @@ SYMBOLS = [
     "grmkm_plan_bucket_bits", "grmkm_set_bucket_bits", "grmkm_set_exchange_rank",
     "grmkm_result_checksum", "grmkm_sum_rows", "grmkm_gram", "grmkm_tsv_pack",
     "grmkm_load_result", "grmkm_scm_run", "grmkm_scm_result",
-    "grmkm_cart_run", "grmkm_cart_result", "grmkm_query",
+    "grmkm_cart_run", "grmkm_cart_result", "grmkm_query", "grmkm_eval_run",
 ]
 SCM_CONJUNCTION, SCM_DISJUNCTION = 0, 1
+EVAL_SCM, EVAL_CART = 0, 1
 
 
 class GrmkmError(RuntimeError):
@@ -93,6 +94,16 @@ class QueryStats(C.Structure):
         return {n: (float if n == "ms" else int)(getattr(self, n)) for n, _ in self._fields_ if n != "struct_size"}
 
 
+class EvalNode(C.Structure):
+    _fields_ = [("kmer", C.c_uint64), ("present_child", C.c_uint32), ("absent_child", C.c_uint32)]
+
+
+class EvalJob(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("kind", C.c_uint32), ("model_type", C.c_uint32), ("reserved", C.c_uint32),
+                ("n_items", C.c_uint64), ("rules", C.c_void_p), ("nodes", C.c_void_p), ("pos", C.c_void_p),
+                ("neg", C.c_void_p)]
+
+
 _lib = None
 
 
@@ -146,6 +157,7 @@ def load() -> C.CDLL:
         "grmkm_cart_run": (i32, [vp, u32, vp, vp, u64]),
         "grmkm_cart_result": (i32, [vp, u32, vp, u64, C.POINTER(u64), vp, u64, C.POINTER(u64)]),
         "grmkm_query": (i32, [vp, vp, u64, vp, u64, C.POINTER(QueryStats)]),
+        "grmkm_eval_run": (i32, [vp, u32, vp, vp, u64]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)

@@ -9,7 +9,8 @@ The rule a step chooses is the one the greedy search scored: for a disjunction, 
 swapped first, so the model itself holds the chosen rules' complements (absence for presence and vice versa) and
 predicts 1 when any of them does; a conjunction holds the chosen rules and predicts 1 when all of them do.
 
-A cross-validation or p grid is one ``fit_many`` call; its predictions come from ``predict``.
+A cross-validation or p grid is one ``fit_many`` call; ``model_selection.cross_validate_scm`` scores such a grid on
+the held-out examples and picks its hyperparameters.
 """
 from __future__ import annotations
 

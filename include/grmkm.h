@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define GRMKM_ABI_VERSION 13
+#define GRMKM_ABI_VERSION 14
 
 enum {
     GRMKM_OK = 0,
@@ -370,6 +370,47 @@ typedef struct grmkm_query_stats {
 
 int grmkm_query(grmkm_ctx* ctx, const uint64_t* kmers, uint64_t n_kmers, uint64_t* dst, uint64_t cap,
                 grmkm_query_stats* stats /* may be NULL */);
+
+/*
+ * Evaluation: fitted models scored on example sets of the resident matrix, many at once (the held-out side of
+ * cross-validation).  A job is one model and a pair of disjoint example masks pos / neg (n_words words, genome g at
+ * bit 63 - g % 64 of word g / 64).  Only counts come back, as uint32 pairs, job after job in the order of the jobs:
+ *
+ *   GRMKM_EVAL_SCM   items = R rule indices < 2U, the model's own rules (a disjunction's absence twins already
+ *                    applied: SetCoveringMachine.rule_indices).  R + 1 pairs (fn_r, fp_r), r = 0..R: fn_r = #pos the
+ *                    model of the first r rules outputs 0 on, fp_r = #neg it outputs 1 on.  A conjunction outputs 1
+ *                    iff all its rules do, a disjunction iff any does; the empty prefix outputs 1 / 0.
+ *   GRMKM_EVAL_CART  items = n >= 1 nodes (root 0).  n pairs (p_i, q_i): the pos / neg examples that reach node i.
+ *                    An example at split node i goes to present_child iff its bit in column kmer is set; a leaf
+ *                    (kmer = UINT64_MAX) ends its walk, and its children are not read.
+ *
+ * Rejected before any device work (GRMKM_E_INVALID): a bad struct_size or kind, reserved != 0, an SCM rule >= 2U, a
+ * CART job without nodes, a split k-mer >= U, a child index not greater than its parent's or >= n, a node with two
+ * parents, overlapping masks, mask bits at rows >= n_genomes.  cap (in uint32 elements) below 2 x the pairs of all
+ * jobs: GRMKM_E_CAPACITY.  A result that is one owner's slice of a multi-GPU merge: GRMKM_E_UNSUPPORTED.  One launch
+ * (one warp per job) and one device->host copy of the counts; the context's SCM and CART results are left as they are.
+ */
+enum { GRMKM_EVAL_SCM = 0, GRMKM_EVAL_CART = 1 };
+
+typedef struct grmkm_eval_node {
+    uint64_t kmer;               /* split k-mer (< U), UINT64_MAX: leaf */
+    uint32_t present_child;      /* node index (> this node's), read for a split node only */
+    uint32_t absent_child;
+} grmkm_eval_node;
+
+typedef struct grmkm_eval_job {
+    uint32_t struct_size;        /* = sizeof(grmkm_eval_job) */
+    uint32_t kind;               /* GRMKM_EVAL_SCM / GRMKM_EVAL_CART */
+    uint32_t model_type;         /* SCM: GRMKM_SCM_CONJUNCTION / GRMKM_SCM_DISJUNCTION; CART: 0 */
+    uint32_t reserved;           /* 0 */
+    uint64_t n_items;            /* SCM: R rules (0 allowed); CART: n nodes (>= 1) */
+    const uint64_t* rules;       /* SCM: R rule indices */
+    const grmkm_eval_node* nodes; /* CART: n nodes */
+    const uint64_t* pos;         /* n_words words */
+    const uint64_t* neg;         /* disjoint from pos */
+} grmkm_eval_job;
+
+int grmkm_eval_run(grmkm_ctx* ctx, uint32_t n_jobs, const grmkm_eval_job* jobs, uint32_t* counts, uint64_t cap);
 
 #ifdef __cplusplus
 }
