@@ -142,6 +142,16 @@ class KmerMatrixBuilder:
         self._check(self._lib.grmkm_copy_matrix(self._ctx, C.c_void_p(out.ctypes.data), U * W))
         return out
 
+    def columns(self, idx) -> np.ndarray:
+        """The (ceil(G/64) x len(idx)) words of columns ``idx``, packed on the device (grmkm_copy_columns): a few columns
+        without copying the whole matrix."""
+        _, W, _ = self.dims
+        idx = np.ascontiguousarray(np.asarray(idx, dtype=np.uint64).reshape(-1))
+        out = np.empty((W, idx.size), dtype=np.uint64)
+        self._check(self._lib.grmkm_copy_columns(self._ctx, C.c_void_p(idx.ctypes.data), idx.size,
+                                                 C.c_void_p(out.ctypes.data), out.size))
+        return out
+
     def result_host(self) -> tuple[np.ndarray, np.ndarray]:
         """(kmers[U], matrix[W][U]) as views of the context's page-locked result buffer: one device->host
         copy at PCIe speed.  The views are valid until the next build / reset / close; copy them to keep them."""
@@ -227,10 +237,43 @@ class KmerMatrixBuilder:
                                                 kmers.size, int(n_genomes)))
         return self
 
-    def scm_run(self, jobs, blacklist=()) -> list[tuple[np.ndarray, np.ndarray]]:
+    def _sharded(self, fn: str, shard, *args):
+        """Call grmkm_<fn> (shard None), or grmkm_<fn>_sharded on this context's slice of the columns.  shard: rank,
+        world, col_offset, n_kmers_total and exchange, whose allgather(bytes) returns every rank's bytes in rank order
+        (learning.ShardedRuleClassifications).  The ctypes callback and the last received bytes live until the call
+        returns."""
+        if shard is None:
+            return self._check(getattr(self._lib, "grmkm_" + fn)(self._ctx, *args))
+        keep = {}
+
+        def exchange(user, send, n, recv, sizes):
+            try:
+                blocks = shard.exchange.allgather(C.string_at(send, n) if n else b"")
+                if len(blocks) != shard.world:
+                    raise RuntimeError(f"the exchange returned {len(blocks)} blocks for {shard.world} ranks")
+                keep["recv"] = C.create_string_buffer(b"".join(blocks), max(1, sum(map(len, blocks))))
+                recv[0] = C.cast(keep["recv"], C.c_void_p)
+                for r, b in enumerate(blocks):
+                    sizes[r] = len(b)
+                return 0
+            except BaseException as e:          # an exception must not cross the C frames
+                keep["error"] = e
+                return 1
+
+        cb = native.EXCHANGE_FN(exchange)
+        sh = native.Shard(C.sizeof(native.Shard), int(shard.rank), int(shard.world), 0, int(shard.col_offset),
+                          int(shard.n_kmers_total), cb, None)
+        rc = getattr(self._lib, "grmkm_" + fn + "_sharded")(self._ctx, *args, C.byref(sh))
+        if rc != native.OK and "error" in keep:
+            msg = self._lib.grmkm_last_error(self._ctx)
+            raise GrmkmError(rc, msg.decode() if msg else "") from keep["error"]
+        self._check(rc)
+
+    def scm_run(self, jobs, blacklist=(), shard=None) -> list[tuple[np.ndarray, np.ndarray]]:
         """Set Covering Machine fits on the resident matrix, all in one grmkm_scm_run.  jobs: (model_type, p, max_rules,
         tiebreak, pos_mask, neg_mask) with masks of ceil(G/64) uint64 words.  -> per fit (steps, equivalent rules):
-        steps is a structured array with the fields of grmkm_scm_step."""
+        steps is a structured array with the fields of grmkm_scm_step.  shard: this context holds one slice of the
+        columns (see _sharded); every rank gets the global result, rule indices global."""
         _, W, _ = self.dims
         masks, arr = [], (native.ScmJob * max(1, len(jobs)))()
         for i, (model_type, p, max_rules, tiebreak, pos, neg) in enumerate(jobs):
@@ -242,7 +285,7 @@ class KmerMatrixBuilder:
             arr[i] = native.ScmJob(C.sizeof(native.ScmJob), int(model_type), int(max_rules), int(bool(tiebreak)), float(p),
                                    pos.ctypes.data, neg.ctypes.data)
         bl = np.ascontiguousarray(blacklist if blacklist is not None else (), dtype=np.uint64).reshape(-1)
-        self._check(self._lib.grmkm_scm_run(self._ctx, len(jobs), arr, C.c_void_p(bl.ctypes.data), bl.size))
+        self._sharded("scm_run", shard, len(jobs), arr, C.c_void_p(bl.ctypes.data), bl.size)
         out = []
         step_dtype = np.dtype([("rule", np.uint64), ("utility", np.float64), ("positive_errors", np.uint32),
                                ("negative_covers", np.uint32), ("equiv_offset", np.uint64), ("equiv_count", np.uint64)])
@@ -263,10 +306,11 @@ class KmerMatrixBuilder:
                                 ("prediction", np.uint32), ("equiv_offset", np.uint64), ("equiv_count", np.uint64),
                                 ("equiv_total", np.uint64)])
 
-    def cart_run(self, jobs, blacklist=()) -> list[tuple[np.ndarray, np.ndarray]]:
+    def cart_run(self, jobs, blacklist=(), shard=None) -> list[tuple[np.ndarray, np.ndarray]]:
         """CART trees on the resident matrix, all in one grmkm_cart_run.  jobs: (max_depth, min_samples_split,
         equiv_cap, w_neg, w_pos, pos_mask, neg_mask) with masks of ceil(G/64) uint64 words.  -> per tree (nodes,
-        equivalent rules): nodes is a structured array with the fields of grmkm_cart_node, in breadth-first order."""
+        equivalent rules): nodes is a structured array with the fields of grmkm_cart_node, in breadth-first order.
+        shard: as for scm_run."""
         _, W, _ = self.dims
         masks, arr = [], (native.CartJob * max(1, len(jobs)))()
         for i, (max_depth, min_samples_split, equiv_cap, w_neg, w_pos, pos, neg) in enumerate(jobs):
@@ -278,7 +322,7 @@ class KmerMatrixBuilder:
             arr[i] = native.CartJob(C.sizeof(native.CartJob), int(max_depth), int(min_samples_split), 0, int(equiv_cap),
                                     float(w_neg), float(w_pos), pos.ctypes.data, neg.ctypes.data)
         bl = np.ascontiguousarray(blacklist if blacklist is not None else (), dtype=np.uint64).reshape(-1)
-        self._check(self._lib.grmkm_cart_run(self._ctx, len(jobs), arr, C.c_void_p(bl.ctypes.data), bl.size))
+        self._sharded("cart_run", shard, len(jobs), arr, C.c_void_p(bl.ctypes.data), bl.size)
         out = []
         for t in range(len(jobs)):
             nn, ne = C.c_uint64(), C.c_uint64()
@@ -294,13 +338,13 @@ class KmerMatrixBuilder:
 
     EVAL_NODE_DTYPE = np.dtype([("kmer", np.uint64), ("present_child", np.uint32), ("absent_child", np.uint32)])
 
-    def eval_run(self, jobs) -> list[np.ndarray]:
+    def eval_run(self, jobs, shard=None) -> list[np.ndarray]:
         """Fitted models scored on example sets of the resident matrix, all in one grmkm_eval_run (one launch, one copy
         of the counts).  jobs: (kind, model_type, items, pos_mask, neg_mask) with masks of ceil(G/64) uint64 words.
         kind native.EVAL_SCM: items = the model's rule indices (< 2U), model_type native.SCM_CONJUNCTION / _DISJUNCTION
         -> (R + 1, 2) counts (fn, fp) of the prefixes of 0..R rules.  kind native.EVAL_CART: model_type 0, items = nodes
         with the fields of EVAL_NODE_DTYPE (kmer UINT64_MAX: leaf) -> (n, 2) counts (pos, neg) of the examples reaching
-        each node."""
+        each node.  shard: as for scm_run (rule and k-mer indices global)."""
         _, W, _ = self.dims
         keep, arr, sizes = [], (native.EvalJob * max(1, len(jobs)))(), []
         for i, (kind, model_type, items, pos, neg) in enumerate(jobs):
@@ -319,7 +363,7 @@ class KmerMatrixBuilder:
             arr[i] = native.EvalJob(C.sizeof(native.EvalJob), int(kind), int(model_type), 0, items.size, rules, nodes,
                                     pos.ctypes.data, neg.ctypes.data)
         counts = np.zeros((sum(sizes), 2), dtype=np.uint32)
-        self._check(self._lib.grmkm_eval_run(self._ctx, len(jobs), arr, C.c_void_p(counts.ctypes.data), counts.size))
+        self._sharded("eval_run", shard, len(jobs), arr, C.c_void_p(counts.ctypes.data), counts.size)
         return np.split(counts, np.cumsum(sizes)[:-1]) if sizes else []
 
     @property

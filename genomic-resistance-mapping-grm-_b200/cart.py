@@ -116,18 +116,15 @@ def fit_many(rule_classifications, trees, rule_blacklist=None):
                      _ALL_EQUIVALENT if t.max_equivalent_rules is None else t.max_equivalent_rules,
                      t.class_importance[0], t.class_importance[1], _row_mask(rc, pos, W), _row_mask(rc, neg, W)))
     blacklist = np.asarray(rule_blacklist if rule_blacklist is not None else [], dtype=np.uint64).reshape(-1)
-    results = b.cart_run(jobs, blacklist)
-    if rc._kmers is None and any((nodes["present_child"] != 0xFFFFFFFF).any() for nodes, _ in results):
-        rc._kmers = b.kmers()
-    seqs = {}
+    results = b.cart_run(jobs, blacklist, shard=rc.shard)
+    needed = sorted({int(x["rule"]) for nodes, _ in results for x in nodes if int(x["present_child"]) != 0xFFFFFFFF})
+    seqs = dict(zip(needed, (_kmer_string(int(x), b.k) for x in rc.kmers_at(needed)))) if needed else {}
     for (t, _, _), (nodes, eq) in zip(trees, results):
         t.nodes = []
         for x in nodes:
             rule = None
             if int(x["present_child"]) != 0xFFFFFFFF:
                 j = int(x["rule"])
-                if j not in seqs:
-                    seqs[j] = _kmer_string(int(rc._kmers[j]), b.k)
                 rule = KmerRule(j, seqs[j], "presence")
             o, c = int(x["equiv_offset"]), int(x["equiv_count"])
             t.nodes.append(Node(rule, float(x["score"]), int(x["depth"]), int(x["n_pos"]), int(x["n_neg"]),

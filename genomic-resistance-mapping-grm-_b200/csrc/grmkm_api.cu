@@ -9,6 +9,7 @@
 #include "grmkm_cart.cuh"
 #include "grmkm_query.cuh"
 #include "grmkm_eval.cuh"
+#include "grmkm_shard.cuh"
 
 #include <nvtx3/nvToolsExt.h>      // header-only; the ranges cost nothing until a tool (nsys, ncu --nvtx) attaches
 #include <zlib.h>
@@ -110,7 +111,9 @@ struct grmkm_ctx {
         qry,             // grmkm_query: key table, slot -> key index, caller column -> key index, totals
         qplane,          // grmkm_query: presence plane or counters of one row range
         qout,            // grmkm_query: one row range's word rows in the caller's column order
-        eval;            // grmkm_eval_run: job arguments, rules, nodes, example masks, counts
+        eval,            // grmkm_eval_run: job arguments, rules, nodes, example masks, counts
+        shard_idx,       // sharded runs: the local indices of the columns this rank sends, and their packed words
+        shard_cols;      // sharded runs: the compact matrix of the exchanged columns
     cudaEvent_t ev_query[2] = {nullptr, nullptr};   // grmkm_query: device time of the call
     uint64_t racc_hint = 0;        // records of the previous abundance build + headroom
     std::vector<uint64_t> merge_h_off;   // row-block merge of a partial build: chunk offsets of the merge buckets
@@ -1406,7 +1409,8 @@ void grmkm_destroy(grmkm_ctx* c) {
                      &c->bcounts, &c->ukeys, &c->uwords, &c->kmers, &c->matrix, &c->scalars, &c->fmt, &c->synth, &c->refs,
                      &c->stile_file, &c->bbase, &c->apub, &c->masks, &c->units, &c->ucur, &c->ubeg, &c->wu, &c->wide,
                      &c->racc, &c->aux, &c->scm, &c->scm_list, &c->cart, &c->cart_bl,
-                     &c->cart_masks[0], &c->cart_masks[1], &c->cart_list, &c->qry, &c->qplane, &c->qout, &c->eval};
+                     &c->cart_masks[0], &c->cart_masks[1], &c->cart_list, &c->qry, &c->qplane, &c->qout, &c->eval,
+                     &c->shard_idx, &c->shard_cols};
     for (DevBuf* b : all) release(c, *b);
     if (c->ev_ok) for (int i = 0; i < T_N; ++i) cudaEventDestroy(c->ev[i]);
     for (cudaEvent_t e : c->ev_query) if (e) cudaEventDestroy(e);
@@ -2059,10 +2063,158 @@ double scm_unkey(uint64_t k) {
     return u;
 }
 
+// ------------------------------------------------------------------------------------------------
+// sharded runs: one rank's slice of the global matrix and the all-gather the ranks talk through
+// ------------------------------------------------------------------------------------------------
+struct Shard {
+    uint32_t rank = 0, n_ranks = 1;
+    uint64_t off = 0, total = 0;            // this slice's first global column; U of the whole matrix
+    grmkm_exchange_fn fn = nullptr;         // nullptr: the whole matrix on one rank, nothing exchanged
+    void* user = nullptr;
+    std::vector<uint64_t> offs;             // every rank's first column and offs[n_ranks] = total (from the first exchange)
+    bool on() const { return fn != nullptr; }
+    uint32_t owner(uint64_t j) const { return (uint32_t)(std::upper_bound(offs.begin(), offs.end(), j) - offs.begin() - 1); }
+    bool mine(uint64_t j) const { return j >= offs[rank] && j < offs[rank + 1]; }
+    // a global rule (j or total + j) -> the local rule of this slice of U columns (j or U + j)
+    uint64_t local_rule(uint64_t r, uint64_t U) const { return r < total ? r - off : U + (r - total - off); }
+    uint64_t global_rule(uint64_t r, uint64_t U) const { return r < U ? off + r : total + off + (r - U); }
+};
+
+Shard whole_matrix(const grmkm_ctx* c) {
+    Shard s;
+    s.total = c->U;
+    s.offs = {0, c->U};
+    return s;
+}
+
+int shard_from(grmkm_ctx* c, const grmkm_shard* in, Shard& s) {
+    if (!in) return fail(c, GRMKM_E_INVALID, "null shard");
+    if (in->struct_size != sizeof(grmkm_shard)) return fail(c, GRMKM_E_INVALID, "shard struct_size is not sizeof(grmkm_shard)");
+    if (!in->exchange) return fail(c, GRMKM_E_INVALID, "null shard exchange");
+    if (in->n_ranks == 0 || in->rank >= in->n_ranks || in->reserved != 0)
+        return fail(c, GRMKM_E_INVALID, "shard rank must be below n_ranks, and reserved 0");
+    s.rank = in->rank; s.n_ranks = in->n_ranks;
+    s.off = in->col_offset; s.total = in->n_kmers_total;
+    s.fn = in->exchange; s.user = in->user;
+    return GRMKM_OK;
+}
+
+// one all-gather: blk[r] / len[r] = the bytes rank r sent
+struct Gathered {
+    std::vector<const uint8_t*> blk;
+    std::vector<uint64_t> len;
+};
+
+int shard_exchange(grmkm_ctx* c, const Shard& s, const void* send, uint64_t n, Gathered& g) {
+    const void* recv = nullptr;
+    g.len.assign(s.n_ranks, 0);
+    if (s.fn(s.user, send, n, &recv, g.len.data()) != 0)
+        return fail(c, GRMKM_E_INVALID, "the shard exchange failed on rank " + std::to_string(s.rank));
+    if (g.len[s.rank] != n) return fail(c, GRMKM_E_INVALID, "the shard exchange returned a block of another size for this rank");
+    g.blk.resize(s.n_ranks);
+    uint64_t o = 0;
+    for (uint32_t r = 0; r < s.n_ranks; ++r) { g.blk[r] = (const uint8_t*)recv + o; o += g.len[r]; }
+    return GRMKM_OK;
+}
+
+// The first exchange of a sharded run: every rank's validation status, column range and n_kmers_total.  If any rank
+// failed, every rank returns the code of the first failing one, before any device work; ranges that do not tile
+// [0, n_kmers_total), or ranks that disagree on n_kmers_total, fail every rank too.  Otherwise s.offs is filled.
+int shard_agree(grmkm_ctx* c, Shard& s, int status) {
+    if (!s.on()) return status;
+    struct Hello { int32_t status; uint32_t pad; uint64_t off, n, total; };
+    const Hello mine{status, 0, s.off, c->built ? c->U : 0, s.total};
+    const std::string own_err = c->err;
+    Gathered g;
+    if (int r = shard_exchange(c, s, &mine, sizeof mine, g)) return r;
+    s.offs.assign(s.n_ranks + 1, 0);
+    uint64_t next = 0;
+    bool tiled = true, same_total = true;
+    for (uint32_t r = 0; r < s.n_ranks; ++r) {
+        if (g.len[r] != sizeof(Hello)) return fail(c, GRMKM_E_INVALID, "rank " + std::to_string(r) + " is not in this run");
+        Hello h;
+        memcpy(&h, g.blk[r], sizeof h);
+        if (h.status) {
+            if (r == s.rank) { c->err = own_err; return h.status; }
+            return fail(c, h.status, "rank " + std::to_string(r) + " refused the run");
+        }
+        tiled = tiled && h.off == next;
+        same_total = same_total && h.total == s.total;
+        s.offs[r] = h.off;
+        next = h.off + h.n;
+    }
+    s.offs[s.n_ranks] = next;
+    if (!same_total) return fail(c, GRMKM_E_INVALID, "the ranks were given different n_kmers_total");
+    if (!tiled || next != s.total)
+        return fail(c, GRMKM_E_INVALID, "the column slices do not tile [0, n_kmers_total) in rank order");
+    return GRMKM_OK;
+}
+
+// dst[w][i] = the words of local columns idx[i], i < m (< 2^32), packed on the device by k_gather_columns
+int pack_columns(grmkm_ctx* c, const uint64_t* idx, uint64_t m, uint64_t* dst) {
+    const uint32_t W = c->W;
+    if (!m || !W) return GRMKM_OK;
+    ENSURE(c, c->shard_idx, m * 8 + m * W * 8);
+    unsigned long long* d_idx = (unsigned long long*)c->shard_idx.p;
+    CU_TRY(c, cudaMemcpyAsync(d_idx, idx, m * 8, cudaMemcpyHostToDevice, c->stream));
+    k_gather_columns<<<(uint32_t)std::min<uint64_t>((m + 7) / 8, (uint64_t)c->sm_count * 16), 256, 0, c->stream>>>(
+        (const unsigned long long*)c->matrix.p, c->pitch, W, d_idx, (uint32_t)m, d_idx + m);
+    CU_TRY(c, cudaGetLastError());
+    c->stats.n_launches++;
+    CU_TRY(c, cudaMemcpyAsync(dst, d_idx + m, m * W * 8, cudaMemcpyDeviceToHost, c->stream));
+    CU_TRY(c, cudaStreamSynchronize(c->stream));
+    return GRMKM_OK;
+}
+
+// The compact matrix [W][cols.size()] of the global columns `cols` (the same list on every rank), in c->shard_cols:
+// every rank packs the columns it owns (k_gather_columns), one exchange, every rank assembles and uploads the whole.
+int shard_columns(grmkm_ctx* c, const Shard& s, const std::vector<uint64_t>& cols, const unsigned long long** out) {
+    const uint32_t W = c->W;
+    const uint64_t n = cols.size();
+    std::vector<uint64_t> own, cnt(s.n_ranks, 0);
+    for (uint64_t j : cols) {
+        const uint32_t o = s.owner(j);
+        ++cnt[o];
+        if (o == s.rank) own.push_back(j - s.off);
+    }
+    const uint64_t m = own.size();
+    std::vector<uint64_t> packed(m * W);
+    if (int r = pack_columns(c, own.data(), m, packed.data())) return r;
+    Gathered g;
+    if (int r = shard_exchange(c, s, packed.data(), m * W * 8, g)) return r;
+    for (uint32_t r = 0; r < s.n_ranks; ++r)
+        if (g.len[r] != cnt[r] * W * 8) return fail(c, GRMKM_E_INVALID, "rank " + std::to_string(r) + " sent other columns");
+    std::vector<uint64_t> h(n * W), at(s.n_ranks, 0);
+    for (uint64_t i = 0; i < n; ++i) {
+        const uint32_t o = s.owner(cols[i]);
+        const uint64_t k = at[o]++;
+        for (uint32_t w = 0; w < W; ++w) memcpy(&h[(uint64_t)w * n + i], g.blk[o] + ((uint64_t)w * cnt[o] + k) * 8, 8);
+    }
+    ENSURE(c, c->shard_cols, n * W * 8);
+    CU_TRY(c, cudaMemcpyAsync(c->shard_cols.p, h.data(), n * W * 8, cudaMemcpyHostToDevice, c->stream));
+    CU_TRY(c, cudaStreamSynchronize(c->stream));
+    *out = (const unsigned long long*)c->shard_cols.p;
+    return GRMKM_OK;
+}
+
+// the position of every global column in the ascending list of the distinct ones
+std::vector<uint64_t> distinct(std::vector<uint64_t> v) {
+    std::sort(v.begin(), v.end());
+    v.erase(std::unique(v.begin(), v.end()), v.end());
+    return v;
+}
+uint64_t position(const std::vector<uint64_t>& cols, uint64_t j) {
+    return (uint64_t)(std::lower_bound(cols.begin(), cols.end(), j) - cols.begin());
+}
+
+// SCM passes over this rank's columns: bit 0 the scan, bit 1 the tie pass (the same grid in both)
+enum { SCM_SCAN = 1, SCM_TIES = 2 };
+
 template <bool CACHED>
-int scm_launch_chunk(grmkm_ctx* c, const ScmFitArg* d_args, uint32_t n, const uint32_t* d_bl, const unsigned long long* d_masks,
-                     unsigned long long* d_best, unsigned long long* d_tile, unsigned long long* d_list,
-                     unsigned long long* d_count, uint64_t cap) {
+int scm_launch_chunk(grmkm_ctx* c, int passes, const ScmFitArg* d_args, uint32_t n, const uint32_t* d_bl,
+                     const unsigned long long* d_masks, unsigned long long* d_best, unsigned long long* d_tile,
+                     unsigned long long* d_list, unsigned long long* d_count, uint64_t cap) {
+    if (c->U == 0) return GRMKM_OK;         // a rank without columns (sharded runs): a zero-size grid is a launch error
     const size_t smem = scm_smem_bytes(n, c->W);
     CU_TRY(c, cudaFuncSetAttribute(k_scm_scan<CACHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CU_TRY(c, cudaFuncSetAttribute(k_scm_ties<CACHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -2071,11 +2223,16 @@ int scm_launch_chunk(grmkm_ctx* c, const ScmFitArg* d_args, uint32_t n, const ui
     const uint64_t n_tiles = (c->U + kScmThreads - 1) / kScmThreads;
     const uint32_t grid = (uint32_t)std::min<uint64_t>(n_tiles, (uint64_t)c->sm_count * std::max(1, occ));
     const unsigned long long* m = (const unsigned long long*)c->matrix.p;
-    k_scm_scan<CACHED><<<grid, kScmThreads, smem, c->stream>>>(m, c->U, c->pitch, c->W, d_bl, d_args, n, d_masks, d_best, d_tile);
-    k_scm_ties<CACHED><<<grid, kScmThreads, smem, c->stream>>>(m, c->U, c->pitch, c->W, d_bl, d_args, n, d_masks, d_best, d_tile,
-                                                               d_list, d_count, cap);
+    if (passes & SCM_SCAN) {
+        k_scm_scan<CACHED><<<grid, kScmThreads, smem, c->stream>>>(m, c->U, c->pitch, c->W, d_bl, d_args, n, d_masks, d_best, d_tile);
+        c->stats.n_launches++;
+    }
+    if (passes & SCM_TIES) {
+        k_scm_ties<CACHED><<<grid, kScmThreads, smem, c->stream>>>(m, c->U, c->pitch, c->W, d_bl, d_args, n, d_masks, d_best, d_tile,
+                                                                   d_list, d_count, cap);
+        c->stats.n_launches++;
+    }
     CU_TRY(c, cudaGetLastError());
-    c->stats.n_launches += 2;
     return GRMKM_OK;
 }
 
@@ -2086,18 +2243,12 @@ int scm_check_mask(grmkm_ctx* c, const uint64_t* m, const char* what) {
     return GRMKM_OK;
 }
 
-}  // namespace
-
-extern "C" {
-
-int grmkm_scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, const uint64_t* blacklist, uint64_t n_blacklist) {
-    if (check_ctx(c)) return GRMKM_E_INVALID;
+int scm_validate(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, const uint64_t* blacklist, uint64_t n_blacklist,
+                 const Shard& sh) {
     if (!c->built) return fail(c, GRMKM_E_INVALID, "no result: call grmkm_build or grmkm_load_result first");
-    if (c->slice)
-        return fail(c, GRMKM_E_UNSUPPORTED, "the result is one owner's slice of a multi-GPU build: its best rule is not the answer");
-    const uint64_t U = c->U;
+    const uint64_t UG = sh.total;
     const uint32_t W = c->W;
-    if (U >= (1ULL << 31)) return fail(c, GRMKM_E_UNSUPPORTED, "the SCM indexes rules with 32 bits: at most 2^31 - 1 k-mers");
+    if (UG >= (1ULL << 31)) return fail(c, GRMKM_E_UNSUPPORTED, "the SCM indexes rules with 32 bits: at most 2^31 - 1 k-mers");
     if (n_fits && !jobs) return fail(c, GRMKM_E_INVALID, "null jobs");
     if (n_blacklist && !blacklist) return fail(c, GRMKM_E_INVALID, "null blacklist");
     for (uint32_t f = 0; f < n_fits; ++f) {
@@ -2117,7 +2268,18 @@ int grmkm_scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, cons
         }
     }
     for (uint64_t i = 0; i < n_blacklist; ++i)
-        if (blacklist[i] >= 2 * U) return fail(c, GRMKM_E_INVALID, "blacklisted rule index >= 2 x n_kmers");
+        if (blacklist[i] >= 2 * UG) return fail(c, GRMKM_E_INVALID, "blacklisted rule index >= 2 x n_kmers");
+    return GRMKM_OK;
+}
+
+// The greedy loop of a batch of fits on this rank's columns; sh: the whole matrix (no exchange) or one slice of it.
+// Sharded, each step is: scan -> exchange the best keys -> tie pass and statistics against the global keys -> exchange
+// the tie lists -> the same host selection on every rank -> exchange the chosen columns -> update the masks.
+int scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, const uint64_t* blacklist, uint64_t n_blacklist, Shard& sh) {
+    if (int r = shard_agree(c, sh, scm_validate(c, n_fits, jobs, blacklist, n_blacklist, sh))) return r;
+    const uint64_t U = c->U, UG = sh.total;
+    const uint32_t W = c->W;
+    const bool sharded = sh.on();
 
     NvtxRange nv("grmkm_scm_run");
     c->scm_steps.assign(n_fits, {});
@@ -2138,7 +2300,7 @@ int grmkm_scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, cons
             nn += (uint32_t)__builtin_popcountll(N0[w]);
         }
         n_pos[f] = np; n_neg[f] = nn;
-        done[f] = nn == 0 || U == 0;          // nothing to cover, or no rule at all
+        done[f] = nn == 0 || UG == 0;         // nothing to cover, or no rule at all
     }
     if (std::find(done.begin(), done.end(), 0) == done.end()) return GRMKM_OK;
 
@@ -2149,10 +2311,12 @@ int grmkm_scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, cons
     const uint32_t chunk = (uint32_t)std::max<size_t>(1, std::min<size_t>(smem_cap / 2, 64 * 1024) / per_fit);
     const uint64_t bl_words = (2 * U + 31) / 32;
     const uint64_t max_grid = (uint64_t)c->sm_count * 8;
+    // sharded, the tie pass runs after the exchange of the keys: every chunk keeps its per-CTA bests until then
+    const uint64_t tile_fits = sharded ? n_fits : chunk;
     auto al = [](size_t b) { return (b + 255) & ~size_t(255); };
     const size_t o_masks = 0, o_best = o_masks + al(h_masks.size() * 8), o_args = o_best + al((size_t)n_fits * 8),
                  o_bl = o_args + al((size_t)n_fits * sizeof(ScmFitArg)), o_tile = o_bl + al(bl_words * 4),
-                 o_sel = o_tile + al((size_t)chunk * max_grid * 8), o_count = o_sel + al((size_t)n_fits * 8),
+                 o_sel = o_tile + al((size_t)tile_fits * max_grid * 8), o_count = o_sel + al((size_t)n_fits * 8),
                  total = o_count + 256;
     ENSURE(c, c->scm, total);
     uint8_t* base = (uint8_t*)c->scm.p;
@@ -2164,15 +2328,33 @@ int grmkm_scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, cons
     unsigned long long* d_sel = (unsigned long long*)(base + o_sel);
     unsigned long long* d_count = (unsigned long long*)(base + o_count);
     std::vector<uint32_t> h_bl(bl_words, 0);
-    for (uint64_t i = 0; i < n_blacklist; ++i) h_bl[blacklist[i] >> 5] |= 1u << (blacklist[i] & 31);
+    for (uint64_t i = 0; i < n_blacklist; ++i) {
+        const uint64_t b = blacklist[i];
+        if (!sh.mine(b % UG)) continue;
+        const uint64_t r = sh.local_rule(b, U);
+        h_bl[r >> 5] |= 1u << (r & 31);
+    }
     CU_TRY(c, cudaMemcpyAsync(d_masks, h_masks.data(), h_masks.size() * 8, cudaMemcpyHostToDevice, c->stream));
     CU_TRY(c, cudaMemcpyAsync(d_bl, h_bl.data(), bl_words * 4, cudaMemcpyHostToDevice, c->stream));
 
     uint64_t cap = std::max<uint64_t>(1024, c->scm_list.cap / 20);      // tie list entries (8 bytes + 3 x 4 bytes of statistics)
     std::vector<ScmFitArg> args;
-    std::vector<uint64_t> h_list, h_best(n_fits), sel;
+    std::vector<uint64_t> h_list, h_best(n_fits), sel, keys, block, cols;
     std::vector<uint32_t> h_stats;
     std::vector<size_t> order;
+    Gathered g;
+    auto launch = [&](int passes) -> int {
+        for (size_t a0 = 0; a0 < args.size(); a0 += chunk) {
+            const uint32_t n = (uint32_t)std::min<size_t>(chunk, args.size() - a0);
+            unsigned long long* tile = d_tile + (sharded ? a0 * max_grid : 0);
+            unsigned long long* d_list = (unsigned long long*)c->scm_list.p;
+            const int r = W <= kScmCachedWords
+                              ? scm_launch_chunk<true>(c, passes, d_args + a0, n, d_bl, d_masks, d_best, tile, d_list, d_count, cap)
+                              : scm_launch_chunk<false>(c, passes, d_args + a0, n, d_bl, d_masks, d_best, tile, d_list, d_count, cap);
+            if (r) return r;
+        }
+        return GRMKM_OK;
+    };
     for (;;) {
         args.clear();
         for (uint32_t f = 0; f < n_fits; ++f)
@@ -2184,31 +2366,75 @@ int grmkm_scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, cons
         CU_TRY(c, cudaMemcpyAsync(d_args, args.data(), args.size() * sizeof(ScmFitArg), cudaMemcpyHostToDevice, c->stream));
         CU_TRY(c, cudaMemsetAsync(d_best, 0, (size_t)n_fits * 8, c->stream));
         CU_TRY(c, cudaMemsetAsync(d_count, 0, 8, c->stream));
-        for (size_t a0 = 0; a0 < args.size(); a0 += chunk) {
-            const uint32_t n = (uint32_t)std::min<size_t>(chunk, args.size() - a0);
-            const int r = W <= kScmCachedWords
-                              ? scm_launch_chunk<true>(c, d_args + a0, n, d_bl, d_masks, d_best, d_tile, d_list, d_count, cap)
-                              : scm_launch_chunk<false>(c, d_args + a0, n, d_bl, d_masks, d_best, d_tile, d_list, d_count, cap);
-            if (r) return r;
+        if (!sharded) {
+            if (int r = launch(SCM_SCAN | SCM_TIES)) return r;
+        } else {
+            // exchange 1: the best key of every pending fit, the max over the ranks is the global u*
+            if (int r = launch(SCM_SCAN)) return r;
+            CU_TRY(c, cudaMemcpyAsync(h_best.data(), d_best, (size_t)n_fits * 8, cudaMemcpyDeviceToHost, c->stream));
+            CU_TRY(c, cudaStreamSynchronize(c->stream));
+            keys.resize(args.size());
+            for (size_t a = 0; a < args.size(); ++a) keys[a] = h_best[args[a].fit];
+            if (int r = shard_exchange(c, sh, keys.data(), keys.size() * 8, g)) return r;
+            for (size_t a = 0; a < args.size(); ++a) {
+                uint64_t k = 0;
+                for (uint32_t q = 0; q < sh.n_ranks; ++q) {
+                    if (g.len[q] != keys.size() * 8) return fail(c, GRMKM_E_INVALID, "a rank sent keys of other fits");
+                    uint64_t x;
+                    memcpy(&x, g.blk[q] + a * 8, 8);
+                    k = std::max(k, x);
+                }
+                h_best[args[a].fit] = k;
+            }
+            CU_TRY(c, cudaMemcpyAsync(d_best, h_best.data(), (size_t)n_fits * 8, cudaMemcpyHostToDevice, c->stream));
+            if (int r = launch(SCM_TIES)) return r;
         }
         uint64_t count = 0;
         CU_TRY(c, cudaMemcpyAsync(&count, d_count, 8, cudaMemcpyDeviceToHost, c->stream));
         CU_TRY(c, cudaStreamSynchronize(c->stream));
-        if (count > cap) {              // the tie list overflowed: grow it and redo the step (nothing was updated)
+        const bool over = count > cap;
+        if (over && !sharded) {         // the tie list overflowed: grow it and redo the step (nothing was updated)
             cap = count + count / 4;
             continue;
         }
-        if (count) {
+        const uint64_t n_local = over ? 0 : count;
+        if (n_local) {
             k_scm_gather<<<(uint32_t)std::min<uint64_t>((count + 255) / 256, (uint64_t)c->sm_count * 16), 256, 0, c->stream>>>(
                 (const unsigned long long*)c->matrix.p, U, c->pitch, W, d_masks, d_list, count, d_stats);
             CU_TRY(c, cudaGetLastError());
             c->stats.n_launches++;
         }
-        h_list.resize(count); h_stats.resize(count * 3);
-        CU_TRY(c, cudaMemcpyAsync(h_list.data(), d_list, count * 8, cudaMemcpyDeviceToHost, c->stream));
-        CU_TRY(c, cudaMemcpyAsync(h_stats.data(), d_stats, count * 12, cudaMemcpyDeviceToHost, c->stream));
-        CU_TRY(c, cudaMemcpyAsync(h_best.data(), d_best, (size_t)n_fits * 8, cudaMemcpyDeviceToHost, c->stream));
+        h_list.resize(n_local); h_stats.resize(n_local * 3);
+        CU_TRY(c, cudaMemcpyAsync(h_list.data(), d_list, n_local * 8, cudaMemcpyDeviceToHost, c->stream));
+        CU_TRY(c, cudaMemcpyAsync(h_stats.data(), d_stats, n_local * 12, cudaMemcpyDeviceToHost, c->stream));
+        if (!sharded) CU_TRY(c, cudaMemcpyAsync(h_best.data(), d_best, (size_t)n_fits * 8, cudaMemcpyDeviceToHost, c->stream));
         CU_TRY(c, cudaStreamSynchronize(c->stream));
+        if (sharded) {
+            // exchange 2: [count][list, global rules][statistics]; an overflow anywhere redoes the step on every rank
+            block.assign(1 + n_local + (n_local * 3 + 1) / 2, 0);
+            block[0] = count;
+            for (uint64_t i = 0; i < n_local; ++i)
+                block[1 + i] = (h_list[i] & ~0xffffffffULL) | sh.global_rule(h_list[i] & 0xffffffffULL, U);
+            if (n_local) memcpy(block.data() + 1 + n_local, h_stats.data(), n_local * 12);
+            if (int r = shard_exchange(c, sh, block.data(), block.size() * 8, g)) return r;
+            bool any_over = false;
+            h_list.clear(); h_stats.clear();
+            for (uint32_t q = 0; q < sh.n_ranks; ++q) {
+                uint64_t nq = 0;
+                if (g.len[q] < 8) return fail(c, GRMKM_E_INVALID, "a rank sent no tie list");
+                memcpy(&nq, g.blk[q], 8);
+                if (g.len[q] == 8) { any_over |= nq > 0; continue; }       // no ties, or an overflow: the count only
+                const uint64_t n = nq;
+                if (g.len[q] != 8 * (1 + n + (n * 3 + 1) / 2)) return fail(c, GRMKM_E_INVALID, "a rank sent a malformed tie list");
+                const size_t l0 = h_list.size();
+                h_list.resize(l0 + n); h_stats.resize((l0 + n) * 3);
+                memcpy(h_list.data() + l0, g.blk[q] + 8, n * 8);
+                memcpy(h_stats.data() + l0 * 3, g.blk[q] + 8 + n * 8, n * 12);
+            }
+            if (over) cap = count + count / 4;
+            if (any_over) continue;
+            count = h_list.size();
+        }
         // the list comes in the order of the atomics: sort it by (fit, rule)
         order.resize(count);
         for (size_t i = 0; i < count; ++i) order[i] = i;
@@ -2247,16 +2473,50 @@ int grmkm_scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, cons
             i = end;
         }
         if (!sel.empty()) {
+            const unsigned long long* mat = (const unsigned long long*)c->matrix.p;
+            uint64_t mU = U, mpitch = c->pitch;
+            if (sharded) {
+                // exchange 3: the chosen columns from their owners; the update runs on their compact matrix
+                cols.clear();
+                for (uint64_t e : sel) cols.push_back((e & 0xffffffffULL) % UG);
+                cols = distinct(cols);
+                if (int r = shard_columns(c, sh, cols, &mat)) return r;
+                mU = mpitch = cols.size();
+                for (uint64_t& e : sel) {
+                    const uint64_t r = e & 0xffffffffULL;
+                    e = (e & ~0xffffffffULL) | (position(cols, r % UG) + (r >= UG ? mU : 0));
+                }
+            }
             CU_TRY(c, cudaMemcpyAsync(d_sel, sel.data(), sel.size() * 8, cudaMemcpyHostToDevice, c->stream));
             const uint64_t nw = (uint64_t)sel.size() * W;
             k_scm_update<<<(uint32_t)std::min<uint64_t>((nw + 255) / 256, (uint64_t)c->sm_count * 8), 256, 0, c->stream>>>(
-                (const unsigned long long*)c->matrix.p, U, c->pitch, W, d_sel, (uint32_t)sel.size(), d_masks);
+                mat, mU, mpitch, W, d_sel, (uint32_t)sel.size(), d_masks);
             CU_TRY(c, cudaGetLastError());
             c->stats.n_launches++;
         }
     }
     CU_TRY(c, cudaStreamSynchronize(c->stream));
     return GRMKM_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int grmkm_scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, const uint64_t* blacklist, uint64_t n_blacklist) {
+    if (check_ctx(c)) return GRMKM_E_INVALID;
+    if (c->built && c->slice)
+        return fail(c, GRMKM_E_UNSUPPORTED, "the result is one owner's slice of a multi-GPU build: its best rule is not the answer");
+    Shard sh = whole_matrix(c);
+    return scm_run(c, n_fits, jobs, blacklist, n_blacklist, sh);
+}
+
+int grmkm_scm_run_sharded(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, const uint64_t* blacklist,
+                          uint64_t n_blacklist, const grmkm_shard* shard) {
+    if (check_ctx(c)) return GRMKM_E_INVALID;
+    Shard sh;
+    if (int r = shard_from(c, shard, sh)) return r;
+    return scm_run(c, n_fits, jobs, blacklist, n_blacklist, sh);
 }
 
 int grmkm_scm_result(grmkm_ctx* c, uint32_t fit, grmkm_scm_step* steps, uint64_t steps_cap, uint64_t* n_steps,
@@ -2286,13 +2546,15 @@ int cart_allow_smem(grmkm_ctx* c, size_t smem) {
     return GRMKM_OK;
 }
 
-// the scan and both tie passes of one chunk of open nodes; CTA b covers the tiles [b tpc, (b + 1) tpc).  occ: resident
-// CTAs per SM by chunk size, filled on first use (a run sees few sizes: full chunks and the tails of its levels)
+// the scan (passes bit 0) and both tie passes (bit 1) of one chunk of open nodes; CTA b covers the tiles
+// [b tpc, (b + 1) tpc).  occ: resident CTAs per SM by chunk size, filled on first use (a run sees few sizes: full chunks
+// and the tails of its levels)
 template <bool CACHED>
-int cart_launch_chunk(grmkm_ctx* c, const CartNodeArg* d_args, uint32_t n, const uint32_t* d_bl, const unsigned long long* d_masks,
-                      unsigned long long* d_best, unsigned long long* d_tile, uint32_t* d_tcnt, unsigned long long* d_total,
-                      unsigned long long* d_list, unsigned long long* d_count, uint64_t cap, uint64_t max_grid,
-                      std::map<uint32_t, int>& occ_of) {
+int cart_launch_chunk(grmkm_ctx* c, int passes, const CartNodeArg* d_args, uint32_t n, const uint32_t* d_bl,
+                      const unsigned long long* d_masks, unsigned long long* d_best, unsigned long long* d_tile, uint32_t* d_tcnt,
+                      unsigned long long* d_total, unsigned long long* d_list, unsigned long long* d_count, uint64_t cap,
+                      uint64_t max_grid, std::map<uint32_t, int>& occ_of) {
+    if (c->U == 0) return GRMKM_OK;         // a rank without columns (sharded runs): a zero-size grid is a launch error
     const size_t smem = cart_smem_bytes(n, c->W);
     auto it = occ_of.find(n);
     if (it == occ_of.end()) {
@@ -2306,27 +2568,26 @@ int cart_launch_chunk(grmkm_ctx* c, const CartNodeArg* d_args, uint32_t n, const
     const uint64_t tpc = (n_tiles + grid0 - 1) / grid0;
     const uint32_t grid = (uint32_t)((n_tiles + tpc - 1) / tpc);
     const unsigned long long* m = (const unsigned long long*)c->matrix.p;
-    k_cart_scan<CACHED><<<grid, kScmThreads, smem, c->stream>>>(m, c->U, c->pitch, c->W, d_bl, d_args, n, d_masks, tpc, d_best, d_tile);
-    for (int append = 0; append < 2; ++append)
-        k_cart_ties<CACHED><<<grid, kScmThreads, smem, c->stream>>>(m, c->U, c->pitch, c->W, d_bl, d_args, n, d_masks, tpc, d_best,
-                                                                    d_tile, d_tcnt, d_total, append, d_list, d_count, cap);
+    if (passes & SCM_SCAN) {
+        k_cart_scan<CACHED><<<grid, kScmThreads, smem, c->stream>>>(m, c->U, c->pitch, c->W, d_bl, d_args, n, d_masks, tpc, d_best, d_tile);
+        c->stats.n_launches++;
+    }
+    if (passes & SCM_TIES) {
+        for (int append = 0; append < 2; ++append)
+            k_cart_ties<CACHED><<<grid, kScmThreads, smem, c->stream>>>(m, c->U, c->pitch, c->W, d_bl, d_args, n, d_masks, tpc, d_best,
+                                                                        d_tile, d_tcnt, d_total, append, d_list, d_count, cap);
+        c->stats.n_launches += 2;
+    }
     CU_TRY(c, cudaGetLastError());
-    c->stats.n_launches += 3;
     return GRMKM_OK;
 }
 
-}  // namespace
-
-extern "C" {
-
-int grmkm_cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const uint64_t* blacklist, uint64_t n_blacklist) {
-    if (check_ctx(c)) return GRMKM_E_INVALID;
+int cart_validate(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const uint64_t* blacklist, uint64_t n_blacklist,
+                  const Shard& sh) {
     if (!c->built) return fail(c, GRMKM_E_INVALID, "no result: call grmkm_build or grmkm_load_result first");
-    if (c->slice)
-        return fail(c, GRMKM_E_UNSUPPORTED, "the result is one owner's slice of a multi-GPU build: its best split is not the answer");
-    const uint64_t U = c->U;
+    const uint64_t UG = sh.total;
     const uint32_t W = c->W;
-    if (U >= (1ULL << 31)) return fail(c, GRMKM_E_UNSUPPORTED, "CART indexes k-mers with 32 bits: at most 2^31 - 1 k-mers");
+    if (UG >= (1ULL << 31)) return fail(c, GRMKM_E_UNSUPPORTED, "CART indexes k-mers with 32 bits: at most 2^31 - 1 k-mers");
     if (n_trees && !jobs) return fail(c, GRMKM_E_INVALID, "null jobs");
     if (n_blacklist && !blacklist) return fail(c, GRMKM_E_INVALID, "null blacklist");
     for (uint32_t t = 0; t < n_trees; ++t) {
@@ -2347,7 +2608,18 @@ int grmkm_cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, c
         }
     }
     for (uint64_t i = 0; i < n_blacklist; ++i)
-        if (blacklist[i] >= 2 * U) return fail(c, GRMKM_E_INVALID, "blacklisted rule index >= 2 x n_kmers");
+        if (blacklist[i] >= 2 * UG) return fail(c, GRMKM_E_INVALID, "blacklisted rule index >= 2 x n_kmers");
+    return GRMKM_OK;
+}
+
+// The level loop of a batch of trees on this rank's columns; sh: the whole matrix (no exchange) or one slice of it.
+// Sharded, each level is: scan -> exchange the best keys -> both tie passes against the global keys -> exchange the
+// tie totals and lists -> the same host selection on every rank -> exchange the split columns -> gather and split.
+int cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const uint64_t* blacklist, uint64_t n_blacklist, Shard& sh) {
+    if (int r = shard_agree(c, sh, cart_validate(c, n_trees, jobs, blacklist, n_blacklist, sh))) return r;
+    const uint64_t U = c->U, UG = sh.total;
+    const uint32_t W = c->W;
+    const bool sharded = sh.on();
 
     NvtxRange nv("grmkm_cart_run");
     c->cart_nodes.assign(n_trees, {});
@@ -2365,7 +2637,7 @@ int grmkm_cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, c
     };
     // a node is scanned unless a stop rule makes it a leaf first (T empty is only known after the scan)
     auto opens = [&](uint32_t t, uint32_t depth, uint32_t a, uint32_t b) {
-        return U > 0 && depth < jobs[t].max_depth && (uint64_t)a + b >= jobs[t].min_samples_split && a > 0 && b > 0;
+        return UG > 0 && depth < jobs[t].max_depth && (uint64_t)a + b >= jobs[t].min_samples_split && a > 0 && b > 0;
     };
     std::vector<uint64_t> h_masks;
     for (uint32_t t = 0; t < n_trees; ++t) {
@@ -2391,8 +2663,9 @@ int grmkm_cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, c
     const uint64_t bl_words = (U + 31) / 32;
     std::vector<uint32_t> h_bl(bl_words, 0);
     for (uint64_t i = 0; i < n_blacklist; ++i) {
-        const uint64_t j = blacklist[i] % U;
-        h_bl[j >> 5] |= 1u << (j & 31);
+        const uint64_t j = blacklist[i] % UG;
+        if (!sh.mine(j)) continue;
+        h_bl[(j - sh.off) >> 5] |= 1u << ((j - sh.off) & 31);
     }
     ENSURE(c, c->cart_bl, bl_words * 4);
     ENSURE(c, c->cart_masks[0], h_masks.size() * 8);
@@ -2406,16 +2679,18 @@ int grmkm_cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, c
     }
     std::map<uint32_t, int> occ_of;
 
-    const unsigned long long* mat = (const unsigned long long*)c->matrix.p;
     uint64_t cap = std::max<uint64_t>(1024, c->cart_list.cap / 8);      // tie list entries
     std::vector<CartNodeArg> args;
     std::vector<CartSplit> splits;
-    std::vector<uint64_t> h_best, h_total, h_list;
+    std::vector<uint64_t> h_best, h_total, h_list, block, cols;
     std::vector<uint32_t> h_stats;
+    Gathered g;
     auto al = [](size_t b) { return (b + 255) & ~size_t(255); };
     while (!open.empty()) {
         const uint32_t n_open = (uint32_t)open.size();
-        const uint32_t cw = std::min(chunk, n_open);            // the widest chunk of this level
+        // the widest chunk of this level; sharded, the tie passes run after the exchange of the keys, so every chunk
+        // keeps its per-CTA bests until then
+        const uint32_t cw = std::min(chunk, n_open), tile_nodes = sharded ? n_open : cw;
         args.resize(n_open);
         for (uint32_t i = 0; i < n_open; ++i) {
             const grmkm_cart_job& j = jobs[open[i].tree];
@@ -2423,7 +2698,7 @@ int grmkm_cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, c
             args[i] = CartNodeArg{j.w_pos, j.w_neg, std::max<uint64_t>(1, j.equiv_cap), i, nd.n_pos, nd.n_neg, 0};
         }
         const size_t o_args = 0, o_best = o_args + al((size_t)n_open * sizeof(CartNodeArg)), o_total = o_best + al((size_t)n_open * 8),
-                     o_tile = o_total + al((size_t)n_open * 8), o_tcnt = o_tile + al((size_t)cw * max_grid * 8),
+                     o_tile = o_total + al((size_t)n_open * 8), o_tcnt = o_tile + al((size_t)tile_nodes * max_grid * 8),
                      o_split = o_tcnt + al((size_t)cw * max_grid * 4), o_stats = o_split + al((size_t)n_open * sizeof(CartSplit)),
                      o_count = o_stats + al((size_t)n_open * 8), total = o_count + 256;
         ENSURE(c, c->cart, total);
@@ -2438,32 +2713,92 @@ int grmkm_cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, c
         unsigned long long* d_count = (unsigned long long*)(base + o_count);
         const unsigned long long* d_masks = (const unsigned long long*)c->cart_masks[cur].p;
         CU_TRY(c, cudaMemcpyAsync(d_args, args.data(), (size_t)n_open * sizeof(CartNodeArg), cudaMemcpyHostToDevice, c->stream));
+        auto launch = [&](int passes) -> int {
+            for (uint32_t a0 = 0; a0 < n_open; a0 += chunk) {
+                const uint32_t n = std::min(chunk, n_open - a0);
+                unsigned long long* tile = d_tile + (sharded ? (uint64_t)a0 * max_grid : 0);
+                unsigned long long* d_list = (unsigned long long*)c->cart_list.p;
+                const int r = W <= kScmCachedWords
+                                  ? cart_launch_chunk<true>(c, passes, d_args + a0, n, (const uint32_t*)c->cart_bl.p, d_masks, d_best,
+                                                            tile, d_tcnt, d_total, d_list, d_count, cap, max_grid, occ_of)
+                                  : cart_launch_chunk<false>(c, passes, d_args + a0, n, (const uint32_t*)c->cart_bl.p, d_masks, d_best,
+                                                             tile, d_tcnt, d_total, d_list, d_count, cap, max_grid, occ_of);
+                if (r) return r;
+            }
+            return GRMKM_OK;
+        };
         uint64_t count = 0;
         for (;;) {
             ENSURE(c, c->cart_list, cap * 8);
-            unsigned long long* d_list = (unsigned long long*)c->cart_list.p;
             CU_TRY(c, cudaMemsetAsync(d_best, 0, (size_t)n_open * 8, c->stream));
             CU_TRY(c, cudaMemsetAsync(d_total, 0, (size_t)n_open * 8, c->stream));
             CU_TRY(c, cudaMemsetAsync(d_count, 0, 8, c->stream));
-            for (uint32_t a0 = 0; a0 < n_open; a0 += chunk) {
-                const uint32_t n = std::min(chunk, n_open - a0);
-                const int r = W <= kScmCachedWords
-                                  ? cart_launch_chunk<true>(c, d_args + a0, n, (const uint32_t*)c->cart_bl.p, d_masks, d_best, d_tile,
-                                                            d_tcnt, d_total, d_list, d_count, cap, max_grid, occ_of)
-                                  : cart_launch_chunk<false>(c, d_args + a0, n, (const uint32_t*)c->cart_bl.p, d_masks, d_best, d_tile,
-                                                             d_tcnt, d_total, d_list, d_count, cap, max_grid, occ_of);
-                if (r) return r;
+            if (!sharded) {
+                if (int r = launch(SCM_SCAN | SCM_TIES)) return r;
+            } else {
+                // exchange 1: every open node's best key, the max over the ranks is the global one
+                if (int r = launch(SCM_SCAN)) return r;
+                h_best.resize(n_open);
+                CU_TRY(c, cudaMemcpyAsync(h_best.data(), d_best, (size_t)n_open * 8, cudaMemcpyDeviceToHost, c->stream));
+                CU_TRY(c, cudaStreamSynchronize(c->stream));
+                if (int r = shard_exchange(c, sh, h_best.data(), (uint64_t)n_open * 8, g)) return r;
+                for (uint32_t q = 0; q < sh.n_ranks; ++q) {
+                    if (g.len[q] != (uint64_t)n_open * 8) return fail(c, GRMKM_E_INVALID, "a rank sent keys of other nodes");
+                    for (uint32_t i = 0; i < n_open; ++i) {
+                        uint64_t x;
+                        memcpy(&x, g.blk[q] + (size_t)i * 8, 8);
+                        h_best[i] = std::max(h_best[i], x);
+                    }
+                }
+                CU_TRY(c, cudaMemcpyAsync(d_best, h_best.data(), (size_t)n_open * 8, cudaMemcpyHostToDevice, c->stream));
+                if (int r = launch(SCM_TIES)) return r;
             }
             CU_TRY(c, cudaMemcpyAsync(&count, d_count, 8, cudaMemcpyDeviceToHost, c->stream));
             CU_TRY(c, cudaStreamSynchronize(c->stream));
-            if (count <= cap) break;
+            const bool over = count > cap;
+            if (sharded) {
+                // exchange 2: [count][tie totals][list, global columns]; an overflow anywhere redoes the level on every rank
+                const uint64_t n_local = over ? 0 : count;
+                block.assign(1 + n_open + n_local, 0);
+                block[0] = count;
+                CU_TRY(c, cudaMemcpyAsync(block.data() + 1, d_total, (size_t)n_open * 8, cudaMemcpyDeviceToHost, c->stream));
+                CU_TRY(c, cudaMemcpyAsync(block.data() + 1 + n_open, c->cart_list.p, n_local * 8, cudaMemcpyDeviceToHost, c->stream));
+                CU_TRY(c, cudaStreamSynchronize(c->stream));
+                for (uint64_t i = 0; i < n_local; ++i) block[1 + n_open + i] += sh.off;
+                if (int r = shard_exchange(c, sh, block.data(), block.size() * 8, g)) return r;
+                bool any_over = false;
+                h_total.assign(n_open, 0);
+                h_list.clear();
+                for (uint32_t q = 0; q < sh.n_ranks; ++q) {
+                    uint64_t nq = 0;
+                    if (g.len[q] < 8 * (1 + (uint64_t)n_open)) return fail(c, GRMKM_E_INVALID, "a rank sent no tie list");
+                    memcpy(&nq, g.blk[q], 8);
+                    const uint64_t n = g.len[q] / 8 - 1 - n_open;
+                    if (n != nq) { if (n == 0) { any_over = true; continue; } return fail(c, GRMKM_E_INVALID, "a rank sent a malformed tie list"); }
+                    for (uint32_t i = 0; i < n_open; ++i) {
+                        uint64_t x;
+                        memcpy(&x, g.blk[q] + 8 + (size_t)i * 8, 8);
+                        h_total[i] += x;
+                    }
+                    const size_t l0 = h_list.size();
+                    h_list.resize(l0 + n);
+                    memcpy(h_list.data() + l0, g.blk[q] + 8 * (1 + (uint64_t)n_open), n * 8);
+                }
+                if (over) cap = count + count / 4;
+                if (any_over) continue;
+                count = h_list.size();
+                break;
+            }
+            if (!over) break;
             cap = count + count / 4;    // the tie list overflowed: grow it and redo the level (nothing was updated)
         }
-        h_best.resize(n_open); h_total.resize(n_open); h_list.resize(count);
-        CU_TRY(c, cudaMemcpyAsync(h_best.data(), d_best, (size_t)n_open * 8, cudaMemcpyDeviceToHost, c->stream));
-        CU_TRY(c, cudaMemcpyAsync(h_total.data(), d_total, (size_t)n_open * 8, cudaMemcpyDeviceToHost, c->stream));
-        CU_TRY(c, cudaMemcpyAsync(h_list.data(), c->cart_list.p, count * 8, cudaMemcpyDeviceToHost, c->stream));
-        CU_TRY(c, cudaStreamSynchronize(c->stream));
+        if (!sharded) {
+            h_best.resize(n_open); h_total.resize(n_open); h_list.resize(count);
+            CU_TRY(c, cudaMemcpyAsync(h_best.data(), d_best, (size_t)n_open * 8, cudaMemcpyDeviceToHost, c->stream));
+            CU_TRY(c, cudaMemcpyAsync(h_total.data(), d_total, (size_t)n_open * 8, cudaMemcpyDeviceToHost, c->stream));
+            CU_TRY(c, cudaMemcpyAsync(h_list.data(), c->cart_list.p, count * 8, cudaMemcpyDeviceToHost, c->stream));
+            CU_TRY(c, cudaStreamSynchronize(c->stream));
+        }
         // the list comes in the order of the atomics: sorted, each node's entries are its ties in ascending column order
         std::sort(h_list.begin(), h_list.end());
         splits.clear();
@@ -2491,9 +2826,20 @@ int grmkm_cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, c
         next.clear();
         if (!splits.empty()) {
             const uint32_t n_split = (uint32_t)splits.size();
+            const unsigned long long* mat = (const unsigned long long*)c->matrix.p;
+            uint64_t mpitch = c->pitch;
+            if (sharded) {
+                // exchange 3: the split columns from their owners; gather and split run on their compact matrix
+                cols.clear();
+                for (const CartSplit& s : splits) cols.push_back(s.j);
+                cols = distinct(cols);
+                if (int r = shard_columns(c, sh, cols, &mat)) return r;
+                mpitch = cols.size();
+                for (CartSplit& s : splits) s.j = (uint32_t)position(cols, s.j);
+            }
             CU_TRY(c, cudaMemcpyAsync(d_split, splits.data(), n_split * sizeof(CartSplit), cudaMemcpyHostToDevice, c->stream));
             k_cart_gather<<<(uint32_t)std::min<uint64_t>((n_split + 7) / 8, (uint64_t)c->sm_count * 16), 256, 0, c->stream>>>(
-                mat, c->pitch, W, d_masks, d_split, n_split, d_stats);
+                mat, mpitch, W, d_masks, d_split, n_split, d_stats);
             CU_TRY(c, cudaGetLastError());
             c->stats.n_launches++;
             h_stats.resize(2 * (size_t)n_split);
@@ -2516,7 +2862,7 @@ int grmkm_cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, c
                 CU_TRY(c, cudaMemcpyAsync(d_split, splits.data(), n_split * sizeof(CartSplit), cudaMemcpyHostToDevice, c->stream));
                 const uint64_t nw = (uint64_t)n_split * W;
                 k_cart_split<<<(uint32_t)std::min<uint64_t>((nw + 255) / 256, (uint64_t)c->sm_count * 8), 256, 0, c->stream>>>(
-                    mat, c->pitch, W, d_masks, d_split, n_split, (unsigned long long*)c->cart_masks[cur ^ 1].p);
+                    mat, mpitch, W, d_masks, d_split, n_split, (unsigned long long*)c->cart_masks[cur ^ 1].p);
                 CU_TRY(c, cudaGetLastError());
                 c->stats.n_launches++;
                 cur ^= 1;
@@ -2526,6 +2872,26 @@ int grmkm_cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, c
     }
     CU_TRY(c, cudaStreamSynchronize(c->stream));
     return GRMKM_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int grmkm_cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const uint64_t* blacklist, uint64_t n_blacklist) {
+    if (check_ctx(c)) return GRMKM_E_INVALID;
+    if (c->built && c->slice)
+        return fail(c, GRMKM_E_UNSUPPORTED, "the result is one owner's slice of a multi-GPU build: its best split is not the answer");
+    Shard sh = whole_matrix(c);
+    return cart_run(c, n_trees, jobs, blacklist, n_blacklist, sh);
+}
+
+int grmkm_cart_run_sharded(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const uint64_t* blacklist,
+                           uint64_t n_blacklist, const grmkm_shard* shard) {
+    if (check_ctx(c)) return GRMKM_E_INVALID;
+    Shard sh;
+    if (int r = shard_from(c, shard, sh)) return r;
+    return cart_run(c, n_trees, jobs, blacklist, n_blacklist, sh);
 }
 
 int grmkm_cart_result(grmkm_ctx* c, uint32_t tree, grmkm_cart_node* nodes, uint64_t nodes_cap, uint64_t* n_nodes,
@@ -2736,62 +3102,65 @@ int grmkm_query(grmkm_ctx* c, const uint64_t* kmers, uint64_t n_kmers, uint64_t*
 // ------------------------------------------------------------------------------------------------
 static_assert(sizeof(EvalNode) == sizeof(grmkm_eval_node), "EvalNode mirrors grmkm_eval_node");
 
-extern "C" {
+namespace {
 
-int grmkm_eval_run(grmkm_ctx* c, uint32_t n_jobs, const grmkm_eval_job* jobs, uint32_t* counts, uint64_t cap) {
-    if (check_ctx(c)) return GRMKM_E_INVALID;
-    if (!c->built) return fail(c, GRMKM_E_INVALID, "no result: call grmkm_build or grmkm_load_result first");
-    if (c->slice)
-        return fail(c, GRMKM_E_UNSUPPORTED, "the result is one owner's slice of a multi-GPU build: it holds some k-mers only");
-    const uint64_t U = c->U;
+// The jobs scored on this rank's matrix; sh: the whole matrix (no exchange) or one slice of it.  Sharded, the columns
+// of the jobs' rules and split k-mers are exchanged once and every rank scores all jobs on their compact matrix.
+int eval_run(grmkm_ctx* c, uint32_t n_jobs, const grmkm_eval_job* jobs, uint32_t* counts, uint64_t cap, Shard& sh) {
+    const uint64_t UG = sh.total;
     const uint32_t W = c->W;
-    if (n_jobs && !jobs) return fail(c, GRMKM_E_INVALID, "null jobs");
     uint64_t pairs = 0, n_rules = 0, n_nodes = 0;
-    std::vector<uint8_t> has_parent;
-    for (uint32_t i = 0; i < n_jobs; ++i) {
-        const grmkm_eval_job& j = jobs[i];
-        const std::string at = " (job " + std::to_string(i) + ")";
-        if (j.struct_size != sizeof(grmkm_eval_job)) return fail(c, GRMKM_E_INVALID, "job struct_size is not sizeof(grmkm_eval_job)" + at);
-        if (j.reserved != 0) return fail(c, GRMKM_E_INVALID, "reserved must be 0" + at);
-        if (j.kind > GRMKM_EVAL_CART) return fail(c, GRMKM_E_INVALID, "unknown job kind" + at);
-        if (j.n_items >= 0xFFFFFFFFULL) return fail(c, GRMKM_E_INVALID, "at most 2^32 - 2 rules or nodes per job" + at);
-        if (j.kind == GRMKM_EVAL_SCM) {
-            if (j.model_type > GRMKM_SCM_DISJUNCTION) return fail(c, GRMKM_E_INVALID, "unknown model type" + at);
-            if (j.n_items && !j.rules) return fail(c, GRMKM_E_INVALID, "null rules" + at);
-            for (uint64_t r = 0; r < j.n_items; ++r)
-                if (j.rules[r] >= 2 * U) return fail(c, GRMKM_E_INVALID, "rule index >= 2 x n_kmers" + at);
-            n_rules += j.n_items;
-            pairs += j.n_items + 1;
-        } else {
-            if (j.model_type != 0) return fail(c, GRMKM_E_INVALID, "model_type of a tree must be 0" + at);
-            if (j.n_items == 0) return fail(c, GRMKM_E_INVALID, "a tree has at least its root node" + at);
-            if (!j.nodes) return fail(c, GRMKM_E_INVALID, "null nodes" + at);
-            const uint64_t n = j.n_items;
-            has_parent.assign(n, 0);
-            for (uint64_t k = 0; k < n; ++k) {
-                const grmkm_eval_node& e = j.nodes[k];
-                if (e.kmer == UINT64_MAX) continue;
-                const std::string nat = " (job " + std::to_string(i) + ", node " + std::to_string(k) + ")";
-                if (e.kmer >= U) return fail(c, GRMKM_E_INVALID, "split k-mer >= n_kmers" + nat);
-                for (uint32_t ch : {e.present_child, e.absent_child}) {
-                    if (ch <= k || ch >= n) return fail(c, GRMKM_E_INVALID, "a child index must be above its parent's and below n" + nat);
-                    if (has_parent[ch]) return fail(c, GRMKM_E_INVALID, "node " + std::to_string(ch) + " has two parents" + at);
-                    has_parent[ch] = 1;
+    auto validate = [&]() -> int {
+        if (!c->built) return fail(c, GRMKM_E_INVALID, "no result: call grmkm_build or grmkm_load_result first");
+        if (n_jobs && !jobs) return fail(c, GRMKM_E_INVALID, "null jobs");
+        std::vector<uint8_t> has_parent;
+        for (uint32_t i = 0; i < n_jobs; ++i) {
+            const grmkm_eval_job& j = jobs[i];
+            const std::string at = " (job " + std::to_string(i) + ")";
+            if (j.struct_size != sizeof(grmkm_eval_job)) return fail(c, GRMKM_E_INVALID, "job struct_size is not sizeof(grmkm_eval_job)" + at);
+            if (j.reserved != 0) return fail(c, GRMKM_E_INVALID, "reserved must be 0" + at);
+            if (j.kind > GRMKM_EVAL_CART) return fail(c, GRMKM_E_INVALID, "unknown job kind" + at);
+            if (j.n_items >= 0xFFFFFFFFULL) return fail(c, GRMKM_E_INVALID, "at most 2^32 - 2 rules or nodes per job" + at);
+            if (j.kind == GRMKM_EVAL_SCM) {
+                if (j.model_type > GRMKM_SCM_DISJUNCTION) return fail(c, GRMKM_E_INVALID, "unknown model type" + at);
+                if (j.n_items && !j.rules) return fail(c, GRMKM_E_INVALID, "null rules" + at);
+                for (uint64_t r = 0; r < j.n_items; ++r)
+                    if (j.rules[r] >= 2 * UG) return fail(c, GRMKM_E_INVALID, "rule index >= 2 x n_kmers" + at);
+                n_rules += j.n_items;
+                pairs += j.n_items + 1;
+            } else {
+                if (j.model_type != 0) return fail(c, GRMKM_E_INVALID, "model_type of a tree must be 0" + at);
+                if (j.n_items == 0) return fail(c, GRMKM_E_INVALID, "a tree has at least its root node" + at);
+                if (!j.nodes) return fail(c, GRMKM_E_INVALID, "null nodes" + at);
+                const uint64_t n = j.n_items;
+                has_parent.assign(n, 0);
+                for (uint64_t k = 0; k < n; ++k) {
+                    const grmkm_eval_node& e = j.nodes[k];
+                    if (e.kmer == UINT64_MAX) continue;
+                    const std::string nat = " (job " + std::to_string(i) + ", node " + std::to_string(k) + ")";
+                    if (e.kmer >= UG) return fail(c, GRMKM_E_INVALID, "split k-mer >= n_kmers" + nat);
+                    for (uint32_t ch : {e.present_child, e.absent_child}) {
+                        if (ch <= k || ch >= n) return fail(c, GRMKM_E_INVALID, "a child index must be above its parent's and below n" + nat);
+                        if (has_parent[ch]) return fail(c, GRMKM_E_INVALID, "node " + std::to_string(ch) + " has two parents" + at);
+                        has_parent[ch] = 1;
+                    }
                 }
+                n_nodes += n;
+                pairs += n;
             }
-            n_nodes += n;
-            pairs += n;
+            if (W) {
+                int r = scm_check_mask(c, j.pos, "positive");
+                if (!r) r = scm_check_mask(c, j.neg, "negative");
+                if (r) return r;
+                for (uint32_t w = 0; w < W; ++w)
+                    if (j.pos[w] & j.neg[w]) return fail(c, GRMKM_E_INVALID, "positive and negative examples overlap" + at);
+            }
         }
-        if (W) {
-            int r = scm_check_mask(c, j.pos, "positive");
-            if (!r) r = scm_check_mask(c, j.neg, "negative");
-            if (r) return r;
-            for (uint32_t w = 0; w < W; ++w)
-                if (j.pos[w] & j.neg[w]) return fail(c, GRMKM_E_INVALID, "positive and negative examples overlap" + at);
-        }
-    }
-    if (cap < 2 * pairs) return fail(c, GRMKM_E_CAPACITY, "counts holds fewer than 2 x the count pairs of the jobs");
-    if (pairs && !counts) return fail(c, GRMKM_E_INVALID, "null counts");
+        if (cap < 2 * pairs) return fail(c, GRMKM_E_CAPACITY, "counts holds fewer than 2 x the count pairs of the jobs");
+        if (pairs && !counts) return fail(c, GRMKM_E_INVALID, "null counts");
+        return GRMKM_OK;
+    };
+    if (int r = shard_agree(c, sh, validate())) return r;
     if (!pairs) return GRMKM_OK;
 
     NvtxRange nv("grmkm_eval_run");
@@ -2815,6 +3184,20 @@ int grmkm_eval_run(grmkm_ctx* c, uint32_t n_jobs, const grmkm_eval_job* jobs, ui
         }
     }
     CU_TRY(c, cudaSetDevice(c->device));
+    const unsigned long long* mat = (const unsigned long long*)c->matrix.p;
+    uint64_t mU = c->U, mpitch = c->pitch;
+    if (sh.on()) {
+        // the columns of every rule and split k-mer, from their owners; the jobs name them by their compact index
+        std::vector<uint64_t> cols;
+        for (uint64_t r : h_rules) cols.push_back(r % UG);
+        for (const grmkm_eval_node& e : h_nodes) if (e.kmer != UINT64_MAX) cols.push_back(e.kmer);
+        cols = distinct(cols);
+        if (!cols.empty())
+            if (int r = shard_columns(c, sh, cols, &mat)) return r;
+        mU = mpitch = cols.size();
+        for (uint64_t& r : h_rules) r = position(cols, r % UG) + (r >= UG ? mU : 0);
+        for (grmkm_eval_node& e : h_nodes) if (e.kmer != UINT64_MAX) e.kmer = position(cols, e.kmer);
+    }
     auto al = [](size_t b) { return (b + 255) & ~size_t(255); };
     const size_t o_args = 0, o_rules = al((size_t)n_jobs * sizeof(EvalJobArg)), o_nodes = o_rules + al(n_rules * 8),
                  o_masks = o_nodes + al(n_nodes * sizeof(EvalNode)), o_cnt = o_masks + al(h_masks.size() * 8),
@@ -2830,7 +3213,7 @@ int grmkm_eval_run(grmkm_ctx* c, uint32_t n_jobs, const grmkm_eval_job* jobs, ui
     const uint32_t warps_per_cta = kEvalThreads / 32;
     const uint32_t grid = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((n_jobs + warps_per_cta - 1) / warps_per_cta,
                                                                               (uint64_t)c->sm_count * 8));
-    k_eval<<<grid, kEvalThreads, 0, st>>>((const unsigned long long*)c->matrix.p, U, c->pitch, W, (const EvalJobArg*)(base + o_args),
+    k_eval<<<grid, kEvalThreads, 0, st>>>(mat, mU, mpitch, W, (const EvalJobArg*)(base + o_args),
                                           n_jobs, (const unsigned long long*)(base + o_rules), (const EvalNode*)(base + o_nodes),
                                           (const unsigned long long*)(base + o_masks), (uint32_t*)(base + o_cnt));
     CU_TRY(c, cudaGetLastError());
@@ -2838,6 +3221,39 @@ int grmkm_eval_run(grmkm_ctx* c, uint32_t n_jobs, const grmkm_eval_job* jobs, ui
     CU_TRY(c, cudaMemcpyAsync(counts, base + o_cnt, pairs * 8, cudaMemcpyDeviceToHost, st));
     CU_TRY(c, cudaStreamSynchronize(st));
     return GRMKM_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int grmkm_eval_run(grmkm_ctx* c, uint32_t n_jobs, const grmkm_eval_job* jobs, uint32_t* counts, uint64_t cap) {
+    if (check_ctx(c)) return GRMKM_E_INVALID;
+    if (c->built && c->slice)
+        return fail(c, GRMKM_E_UNSUPPORTED, "the result is one owner's slice of a multi-GPU build: it holds some k-mers only");
+    Shard sh = whole_matrix(c);
+    return eval_run(c, n_jobs, jobs, counts, cap, sh);
+}
+
+int grmkm_eval_run_sharded(grmkm_ctx* c, uint32_t n_jobs, const grmkm_eval_job* jobs, uint32_t* counts, uint64_t cap,
+                           const grmkm_shard* shard) {
+    if (check_ctx(c)) return GRMKM_E_INVALID;
+    Shard sh;
+    if (int r = shard_from(c, shard, sh)) return r;
+    return eval_run(c, n_jobs, jobs, counts, cap, sh);
+}
+
+int grmkm_copy_columns(grmkm_ctx* c, const uint64_t* idx, uint64_t n, uint64_t* dst, uint64_t cap) {
+    if (check_ctx(c)) return GRMKM_E_INVALID;
+    if (!c->built) return fail(c, GRMKM_E_INVALID, "no result: call grmkm_build or grmkm_load_result first");
+    if (n && !idx) return fail(c, GRMKM_E_INVALID, "null column indices");
+    if (n > 0xFFFFFFFFULL) return fail(c, GRMKM_E_INVALID, "at most 2^32 - 1 columns in one call");
+    for (uint64_t i = 0; i < n; ++i)
+        if (idx[i] >= c->U) return fail(c, GRMKM_E_INVALID, "column index >= n_kmers");
+    if (cap < n * c->W) return fail(c, GRMKM_E_CAPACITY, "dst holds fewer than n_words x n words");
+    if (n && c->W && !dst) return fail(c, GRMKM_E_INVALID, "null dst");
+    CU_TRY(c, cudaSetDevice(c->device));
+    return pack_columns(c, idx, n, dst);
 }
 
 }  // extern "C"

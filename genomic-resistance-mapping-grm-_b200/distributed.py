@@ -56,6 +56,69 @@ def init_process_group_from_env(backend: str | None = None):
     return dist
 
 
+class TorchExchange:
+    """The all-gather of the sharded runs (learning.ShardedRuleClassifications) over a torch.distributed process group,
+    the one the build used by default: the block sizes first, then one all_gather_into_tensor of the blocks padded to
+    the largest.  Tensors live on the GPU for NCCL and on the host for gloo, as in DistributedBuilder.slice_counts."""
+
+    def __init__(self, group=None):
+        import torch.distributed as dist
+        self.group = group
+        self.rank, self.world = dist.get_rank(group), dist.get_world_size(group)
+        self.device = "cuda" if dist.get_backend(group) == "nccl" else "cpu"
+
+    def allgather(self, data: bytes) -> list[bytes]:
+        import torch
+        import torch.distributed as dist
+        sizes = torch.empty(self.world, dtype=torch.int64, device=self.device)
+        dist.all_gather_into_tensor(sizes, torch.tensor([len(data)], dtype=torch.int64, device=self.device), group=self.group)
+        sizes = sizes.tolist()
+        width = max(sizes)
+        if width == 0:
+            return [b""] * self.world
+        mine = torch.zeros(width, dtype=torch.uint8)
+        if len(data):
+            mine[: len(data)] = torch.frombuffer(bytearray(data), dtype=torch.uint8)
+        out = torch.empty(self.world * width, dtype=torch.uint8, device=self.device)
+        dist.all_gather_into_tensor(out, mine.to(self.device), group=self.group)
+        out = out.cpu().numpy()
+        return [out[r * width: r * width + sizes[r]].tobytes() for r in range(self.world)]
+
+
+class ThreadExchange:
+    """The all-gather of the sharded runs among `world` threads of one process, each driving its own context (tests,
+    or several contexts on one GPU).  ThreadExchange.group(world) makes the ends of all ranks.  A rank that does not
+    arrive within `timeout` seconds breaks the barrier: every waiting rank raises TimeoutError instead of hanging."""
+
+    class _Shared:
+        def __init__(self, world: int, timeout: float):
+            import threading
+            self.slots = [b""] * world
+            self.barrier = threading.Barrier(world, timeout=timeout)
+
+    def __init__(self, shared: "_Shared", rank: int, world: int):
+        self._shared, self.rank, self.world = shared, rank, world
+
+    @classmethod
+    def group(cls, world: int, timeout: float = 60.0) -> list["ThreadExchange"]:
+        shared = cls._Shared(int(world), float(timeout))
+        return [cls(shared, r, int(world)) for r in range(int(world))]
+
+    def _wait(self):
+        import threading
+        try:
+            self._shared.barrier.wait()
+        except threading.BrokenBarrierError:
+            raise TimeoutError(f"rank {self.rank}: a rank of the thread exchange did not arrive") from None
+
+    def allgather(self, data: bytes) -> list[bytes]:
+        self._shared.slots[self.rank] = bytes(data)
+        self._wait()                    # every block is in
+        out = list(self._shared.slots)
+        self._wait()                    # every rank has read them: the slots may be written again
+        return out
+
+
 class HostCounts:
     """The P x P table of partial-column counts, exchanged on the HOST through a file in /dev/shm (the ranks of this
     path share one node, SURVEY.md section 8e): a rank writes its row and then a sequence number, and spins until every

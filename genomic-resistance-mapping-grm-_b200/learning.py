@@ -28,6 +28,8 @@ class KmerRuleClassifications:
     """Rule classifications of a built matrix.  ``builder`` is a KmerMatrixBuilder (or DistributedBuilder rank)
     whose result is resident; ``n_rows`` the number of genomes (examples)."""
 
+    shard = None                        # the whole matrix: the learners' runs exchange nothing
+
     def __init__(self, builder, n_rows: int):
         self.builder = builder
         self.dataset_initial_n_rows = int(n_rows)
@@ -86,6 +88,98 @@ class KmerRuleClassifications:
         result = _unpack_binary_bytes_from_ints(self._matrix[:, cols])[row_mask]
         result[:, invert] = 1 - result[:, invert]
         return result.reshape(-1) if columns_is_int else result
+
+    def kmers_at(self, idx) -> np.ndarray:
+        """The packed k-mers of columns ``idx`` (the k-mers are fetched once)."""
+        if self._kmers is None:
+            self._kmers = self.builder.kmers()
+        return self._kmers[np.asarray(idx, dtype=np.int64)]
+
+
+def column_owners(col_counts, columns) -> tuple[np.ndarray, np.ndarray]:
+    """Global columns -> (owner rank, index in the owner's slice), the slices of ``col_counts`` columns in rank order."""
+    starts = np.concatenate([[0], np.cumsum(np.asarray(col_counts, dtype=np.int64))])
+    columns = np.asarray(columns, dtype=np.int64).reshape(-1)
+    if len(columns) and (columns.min() < 0 or columns.max() >= starts[-1]):
+        raise IndexError(f"column index out of range for {int(starts[-1])} columns")
+    owner = np.searchsorted(starts, columns, side="right") - 1
+    return owner, columns - starts[owner]
+
+
+class ShardedRuleClassifications(KmerRuleClassifications):
+    """Rule classifications of a matrix held as column slices by ``world`` ranks, the matrix never gathered: rank r's
+    ``builder`` holds columns [sum(col_counts[:r]), sum(col_counts[:r + 1])) of the global order (the owner slices of
+    a multi-GPU build, in rank order).  ``exchange``: this rank's end of an all-gather (distributed.TorchExchange or
+    ThreadExchange).  Every rank makes the same calls in the same order; each gets the global result, which is the one
+    the whole matrix gives: rule, k-mer and column indices are global (presence j, absence U + j, U the global count)."""
+
+    def __init__(self, builder, n_rows: int, rank: int, world: int, col_counts, exchange):
+        super().__init__(builder, n_rows)
+        col_counts = [int(x) for x in col_counts]
+        if len(col_counts) != int(world) or not 0 <= int(rank) < int(world) or min(col_counts) < 0:
+            raise ValueError(f"col_counts must give the columns of each of the {world} ranks, rank in 0..{int(world) - 1}")
+        if col_counts[int(rank)] != self._U:
+            raise ValueError(f"col_counts say rank {rank} holds {col_counts[int(rank)]} columns, its builder holds "
+                             f"{self._U}: the counts do not sum to the matrix's U")
+        self.rank, self.world, self.col_counts, self.exchange = int(rank), int(world), col_counts, exchange
+        self.col_offset = sum(col_counts[: self.rank])
+        self.n_kmers_total = self._U = sum(col_counts)
+        self.shard = self
+
+    @classmethod
+    def from_distributed(cls, dbuilder, n_rows: int, exchange=None) -> "ShardedRuleClassifications":
+        """This rank's view of a DistributedBuilder's result (collective: one all-gather of the slice sizes);
+        exchange defaults to a TorchExchange over the default process group."""
+        if exchange is None:
+            from .distributed import ThreadExchange, TorchExchange
+            exchange = TorchExchange() if dbuilder.world > 1 else ThreadExchange.group(1)[0]
+        return cls(dbuilder.builder, n_rows, dbuilder.rank, dbuilder.world, dbuilder.slice_counts(), exchange)
+
+    def _gather_columns(self, words, columns, n_words: int) -> np.ndarray:
+        """Every rank sends the [n_words][n] uint64 of the columns of ``columns`` it owns (``words(local indices)``);
+        -> the [n_words][len(columns)] words of all of them.  Collective."""
+        owner, local = column_owners(self.col_counts, columns)
+        blocks = self.exchange.allgather(np.ascontiguousarray(words(local[owner == self.rank]), dtype=np.uint64).tobytes())
+        out = np.zeros((n_words, len(owner)), dtype=np.uint64)
+        for r in range(self.world):
+            sel = owner == r
+            out[:, sel] = np.frombuffer(blocks[r], dtype=np.uint64).reshape(n_words, int(sel.sum()))
+        return out
+
+    def sum_rows(self, rows):
+        """As KmerRuleClassifications.sum_rows, for the global rules (one exchange of the slices' sums).  Collective."""
+        rows = np.asarray(rows)
+        mask = np.zeros(self._W, dtype=np.uint64)
+        for idx in self._absolute_rows(np.sort(rows)):
+            mask[idx // 64] |= np.uint64(1) << np.uint64(64 - (idx - 64 * (idx // 64)) - 1)
+        mine = self.builder.sum_rows(mask) if self.col_counts[self.rank] else np.zeros(0, dtype=np.uint32)
+        sums = np.concatenate([np.frombuffer(b, dtype=np.uint32) for b in
+                               self.exchange.allgather(np.ascontiguousarray(mine, dtype=np.uint32).tobytes())])
+        result = np.zeros(self._U * 2, dtype=_minimum_uint_size(rows.shape[0]))
+        result[: self._U] = sums
+        result[self._U:] = len(rows) - sums.astype(np.int64)
+        return result
+
+    def get_columns(self, columns):
+        """As KmerRuleClassifications.get_columns, for global rule indices: each owner packs its requested columns on
+        its device (KmerMatrixBuilder.columns), one exchange.  Collective."""
+        columns_is_int = hasattr(columns, "__index__")
+        columns = [columns.__index__()] if columns_is_int else [int(c) for c in columns]
+        invert = np.array([c >= self._U for c in columns], dtype=bool)
+        cols = np.array([c % self._U if c >= self._U else c for c in columns], dtype=np.int64)
+        words = self._gather_columns(lambda local: self.builder.columns(local), cols, self._W)
+        row_mask = np.ones(self._W * 64, dtype=bool)
+        row_mask[self.dataset_initial_n_rows:] = False
+        row_mask[self.dataset_removed_rows] = False
+        result = _unpack_binary_bytes_from_ints(words)[row_mask]
+        result[:, invert] = 1 - result[:, invert]
+        return result.reshape(-1) if columns_is_int else result
+
+    def kmers_at(self, idx) -> np.ndarray:
+        """The packed k-mers of global columns ``idx``, from their owners (one exchange).  Collective."""
+        if self._kmers is None:
+            self._kmers = self.builder.kmers() if self.col_counts[self.rank] else np.zeros(0, dtype=np.uint64)
+        return self._gather_columns(lambda local: self._kmers[local][None, :], idx, 1)[0]
 
 
 _BASE_CODE = np.full(256, 255, dtype=np.uint64)

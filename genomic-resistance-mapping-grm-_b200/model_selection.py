@@ -185,7 +185,7 @@ def cross_validate_scm(rc, train_pos, train_neg, model_types, p_values, max_rule
         for m in machines[min(e, k)]:
             jobs.append((native.EVAL_SCM, scm._MODEL_TYPES[m.model_type], m.rule_indices, pm, nm))
     t0 = time.perf_counter()
-    counts = rc.builder.eval_run(jobs)
+    counts = rc.builder.eval_run(jobs, shard=rc.shard)
     t_eval = time.perf_counter() - t0
 
     n_cand = nT * nP
@@ -335,7 +335,7 @@ def cross_validate_cart(rc, train_pos, train_neg, class_importances, max_depths,
         for t in trees[min(e, k)]:
             jobs.append((native.EVAL_CART, 0, _eval_nodes(t.nodes), pm, nm))
     t0 = time.perf_counter()
-    counts = rc.builder.eval_run(jobs)
+    counts = rc.builder.eval_run(jobs, shard=rc.shard)
     t_eval = time.perf_counter() - t0
 
     nW = len(weights)

@@ -6,7 +6,7 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("GRMKM_LIB") or os.path.join(_HERE, "libgrmkm.so")   # GRMKM_LIB: another build of the same library (kernel experiments)
-ABI_VERSION = 14
+ABI_VERSION = 15
 
 OK = 0
 E_INVALID, E_UNSUPPORTED_K, E_NOMEM, E_CUDA, E_IO, E_CAPACITY, E_NO_DEVICE, E_UNSUPPORTED = -1, -2, -3, -4, -5, -6, -7, -8
@@ -24,6 +24,7 @@ SYMBOLS = [
     "grmkm_result_checksum", "grmkm_sum_rows", "grmkm_gram", "grmkm_tsv_pack",
     "grmkm_load_result", "grmkm_scm_run", "grmkm_scm_result",
     "grmkm_cart_run", "grmkm_cart_result", "grmkm_query", "grmkm_eval_run",
+    "grmkm_scm_run_sharded", "grmkm_cart_run_sharded", "grmkm_eval_run_sharded", "grmkm_copy_columns",
 ]
 SCM_CONJUNCTION, SCM_DISJUNCTION = 0, 1
 EVAL_SCM, EVAL_CART = 0, 1
@@ -104,6 +105,17 @@ class EvalJob(C.Structure):
                 ("neg", C.c_void_p)]
 
 
+# int exchange(void* user, const void* send, uint64_t n, const void** recv, uint64_t* sizes): the all-gather of the
+# sharded runs
+EXCHANGE_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64))
+
+
+class Shard(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("rank", C.c_uint32), ("n_ranks", C.c_uint32), ("reserved", C.c_uint32),
+                ("col_offset", C.c_uint64), ("n_kmers_total", C.c_uint64), ("exchange", EXCHANGE_FN),
+                ("user", C.c_void_p)]
+
+
 _lib = None
 
 
@@ -158,6 +170,10 @@ def load() -> C.CDLL:
         "grmkm_cart_result": (i32, [vp, u32, vp, u64, C.POINTER(u64), vp, u64, C.POINTER(u64)]),
         "grmkm_query": (i32, [vp, vp, u64, vp, u64, C.POINTER(QueryStats)]),
         "grmkm_eval_run": (i32, [vp, u32, vp, vp, u64]),
+        "grmkm_scm_run_sharded": (i32, [vp, u32, vp, vp, u64, C.POINTER(Shard)]),
+        "grmkm_cart_run_sharded": (i32, [vp, u32, vp, vp, u64, C.POINTER(Shard)]),
+        "grmkm_eval_run_sharded": (i32, [vp, u32, vp, vp, u64, C.POINTER(Shard)]),
+        "grmkm_copy_columns": (i32, [vp, vp, u64, vp, u64]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)

@@ -71,7 +71,8 @@ def _refuse_slices(rule_classifications):
     b = rule_classifications.builder
     if getattr(b, "world", 1) > 1:
         raise ValueError("the matrix is this rank's slice of a multi-GPU build: its best rule is not the answer; "
-                         "learn from the gathered matrix (DistributedBuilder.gather, then load_result)")
+                         "learn on all slices (learning.ShardedRuleClassifications.from_distributed), or from the "
+                         "gathered matrix (DistributedBuilder.gather, then load_result)")
 
 
 def _row_mask(rule_classifications, idx, W: int) -> np.ndarray:
@@ -95,10 +96,9 @@ def fit_many(rule_classifications, fits, rule_blacklist=None, tiebreaker="risk")
         jobs.append((_MODEL_TYPES[m.model_type], m.p, m.max_rules, tiebreaker == "risk",
                      _row_mask(rc, pos, W), _row_mask(rc, neg, W)))
     blacklist = np.asarray(rule_blacklist if rule_blacklist is not None else [], dtype=np.uint64).reshape(-1)
-    results = b.scm_run(jobs, blacklist)
-    seqs = {}
-    if any(len(s) for s, _ in results) and rc._kmers is None:
-        rc._kmers = b.kmers()
+    results = b.scm_run(jobs, blacklist, shard=rc.shard)
+    needed = sorted({int(s["rule"]) % U for _, (steps, _) in zip(fits, results) for s in steps})
+    seqs = dict(zip(needed, (_kmer_string(int(x), b.k) for x in rc.kmers_at(needed)))) if needed else {}
     for (m, _, _), (steps, eq) in zip(fits, results):
         m.model, m.iterations, m.rule_indices = [], [], []
         for s in steps:
@@ -108,8 +108,6 @@ def fit_many(rule_classifications, fits, rule_blacklist=None, tiebreaker="risk")
                                           eq[o:o + n].astype(np.int64)))
             mr = r if m.model_type == "conjunction" else (r + U if r < U else r - U)
             j = mr % U
-            if j not in seqs:
-                seqs[j] = _kmer_string(int(rc._kmers[j]), b.k)
             m.rule_indices.append(mr)
             m.model.append(KmerRule(j, seqs[j], "presence" if mr < U else "absence"))
     return [m for m, _, _ in fits]

@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define GRMKM_ABI_VERSION 14
+#define GRMKM_ABI_VERSION 15
 
 enum {
     GRMKM_OK = 0,
@@ -411,6 +411,58 @@ typedef struct grmkm_eval_job {
 } grmkm_eval_job;
 
 int grmkm_eval_run(grmkm_ctx* ctx, uint32_t n_jobs, const grmkm_eval_job* jobs, uint32_t* counts, uint64_t cap);
+
+/*
+ * Sharded runs: learning and evaluation on the column slices of a multi-GPU build, the matrix never gathered.
+ *
+ * Rank r of P holds the global columns [col_offset, col_offset + U_r) of a matrix of n_kmers_total columns; the
+ * slices, in rank order, tile [0, n_kmers_total) (the owner slices of grmkm_merge_partials do; so do column ranges
+ * loaded with grmkm_load_result).  Every rank calls the same sharded function with the same jobs, blacklist and
+ * n_kmers_total, and gets the same global result, bit for bit the result of the unsharded call on the whole matrix:
+ * rule, k-mer, blacklist and split indices are global (presence rule j, absence rule n_kmers_total + j), and results
+ * are read with grmkm_scm_result / grmkm_cart_result / the counts buffer as usual.
+ *
+ * The ranks talk through one collective, an all-gather of variable-size byte blocks: exchange(user, send, n, &recv,
+ * sizes) returns in recv the concatenation of every rank's block in rank order (sizes[r] bytes from rank r), valid
+ * until the next call on this rank.  A non-zero return aborts the run on this rank with GRMKM_E_INVALID.  The first
+ * exchange of a run carries every rank's validation status, column range and n_kmers_total: if any rank fails (bad
+ * jobs, no result, ranges that do not tile [0, n_kmers_total), ranks given different n_kmers_total), every rank
+ * returns the first failing rank's code before any device work, and no rank is left waiting.  A rank that owns no
+ * columns launches nothing but takes part in every exchange.
+ *
+ * Failures that are not collective: a bad shard (NULL, wrong struct_size, NULL exchange, rank >= n_ranks) returns on
+ * that rank before the first exchange, and an error after it (device memory, a CUDA error, a failed exchange) returns
+ * on the rank that meets it.  Either way the other ranks wait in their next exchange until it fails: the exchange
+ * must give up after a timeout (distributed.ThreadExchange has one; a torch.distributed process group has its own), and
+ * the caller treats such a failure on any rank as the failure of the whole run.
+ * Per SCM step: the best keys (8 bytes per pending fit), the tie lists with their statistics, the chosen columns
+ * (8 x n_words bytes each); per CART level: the best keys, the tie totals and lists, the split columns; per eval call:
+ * the columns of the jobs' rules and split k-mers.
+ */
+typedef int (*grmkm_exchange_fn)(void* user, const void* send, uint64_t n, const void** recv, uint64_t* sizes /*[n_ranks]*/);
+
+typedef struct grmkm_shard {
+    uint32_t struct_size;        /* = sizeof(grmkm_shard) */
+    uint32_t rank;               /* < n_ranks */
+    uint32_t n_ranks;            /* >= 1 */
+    uint32_t reserved;           /* 0 */
+    uint64_t col_offset;         /* the global index of this slice's first column */
+    uint64_t n_kmers_total;      /* U of the whole matrix */
+    grmkm_exchange_fn exchange;  /* not NULL */
+    void* user;                  /* passed to exchange */
+} grmkm_shard;
+
+int grmkm_scm_run_sharded(grmkm_ctx* ctx, uint32_t n_fits, const grmkm_scm_job* jobs, const uint64_t* blacklist,
+                          uint64_t n_blacklist, const grmkm_shard* shard);
+int grmkm_cart_run_sharded(grmkm_ctx* ctx, uint32_t n_trees, const grmkm_cart_job* jobs, const uint64_t* blacklist,
+                           uint64_t n_blacklist, const grmkm_shard* shard);
+int grmkm_eval_run_sharded(grmkm_ctx* ctx, uint32_t n_jobs, const grmkm_eval_job* jobs, uint32_t* counts, uint64_t cap,
+                           const grmkm_shard* shard);
+
+/* The words of columns idx[0 .. n) of the resident result, dst[w * n + i] = word row w of column idx[i] (n_words x n,
+ * row-major), packed on the device: the columns a model needs without copying the whole matrix.  idx[i] >= n_kmers or
+ * n >= 2^32: GRMKM_E_INVALID; cap < n_words x n: GRMKM_E_CAPACITY. */
+int grmkm_copy_columns(grmkm_ctx* ctx, const uint64_t* idx, uint64_t n, uint64_t* dst, uint64_t cap);
 
 #ifdef __cplusplus
 }
