@@ -25,6 +25,7 @@ class KmerMatrixBuilder:
         self._rows = 0           # max genome row + 1 of the inputs added since the last reset
         self._declared = 0       # set_genome_count
         self.k = int(k)
+        self.device = int(device)
         cfg = native.Config(C.sizeof(native.Config), int(k), int(min_abundance), int(bool(keep_singletons)),
                             int(input_kind), int(device), int(bucket_bits), int(flags),
                             C.c_void_p(stream) if stream else None)
@@ -236,6 +237,31 @@ class KmerMatrixBuilder:
         self._check(self._lib.grmkm_load_result(self._ctx, C.c_void_p(kmers.ctypes.data), C.c_void_p(matrix.ctypes.data),
                                                 kmers.size, int(n_genomes)))
         return self
+
+    def patterns(self, dst: "KmerMatrixBuilder", column_class=None, with_stats: bool = False):
+        """The distinct presence patterns of this result (grmkm_patterns): columns with equal words (and equal
+        ``column_class`` byte, 0..3, when given) form one pattern, patterns numbered by their first column.  ``dst``
+        (another builder on this device) receives the P x W pattern matrix, the k-mers of the patterns' first columns
+        and their multiplicities.  -> (pattern_of_column uint32[U], members uint32[U], member_offsets uint64[P + 1]):
+        the members of pattern p, ascending, are members[member_offsets[p]:member_offsets[p + 1]].  with_stats: also
+        the call's statistics (rounds, P, device ms) as a dict."""
+        U, _, _ = self.dims
+        cls = None
+        if column_class is not None:
+            cls = np.ascontiguousarray(column_class)
+            if cls.shape != (U,) or cls.dtype.kind not in "biu" or (U and (cls.min() < 0 or cls.max() > 255)):
+                raise ValueError(f"column_class must hold one integer class per column ({U}), not {cls.shape} {cls.dtype}")
+            cls = cls.astype(np.uint8)
+        pattern_of = np.empty(U, dtype=np.uint32)
+        members = np.empty(U, dtype=np.uint32)
+        offsets = np.empty(U + 1, dtype=np.uint64)
+        st = native.PatternStats()
+        st.struct_size = C.sizeof(native.PatternStats)
+        self._check(self._lib.grmkm_patterns(self._ctx, None if cls is None else C.c_void_p(cls.ctypes.data), dst._ctx,
+                                             C.c_void_p(pattern_of.ctypes.data), U, C.c_void_p(members.ctypes.data), U,
+                                             C.c_void_p(offsets.ctypes.data), U + 1, C.byref(st)))
+        out = (pattern_of, members, offsets[: int(st.n_patterns) + 1].copy())
+        return (*out, st.asdict()) if with_stats else out
 
     def _sharded(self, fn: str, shard, *args):
         """Call grmkm_<fn> (shard None), or grmkm_<fn>_sharded on this context's slice of the columns.  shard: rank,

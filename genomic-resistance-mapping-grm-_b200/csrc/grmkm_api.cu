@@ -10,6 +10,10 @@
 #include "grmkm_query.cuh"
 #include "grmkm_eval.cuh"
 #include "grmkm_shard.cuh"
+#include "grmkm_patterns.cuh"
+
+#include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 
 #include <nvtx3/nvToolsExt.h>      // header-only; the ranges cost nothing until a tool (nsys, ncu --nvtx) attaches
 #include <zlib.h>
@@ -113,7 +117,9 @@ struct grmkm_ctx {
         qout,            // grmkm_query: one row range's word rows in the caller's column order
         eval,            // grmkm_eval_run: job arguments, rules, nodes, example masks, counts
         shard_idx,       // sharded runs: the local indices of the columns this rank sends, and their packed words
-        shard_cols;      // sharded runs: the compact matrix of the exchanged columns
+        shard_cols,      // sharded runs: the compact matrix of the exchanged columns
+        pat,             // grmkm_patterns (source side): fingerprints, grouping table, ids, members, sort scratch
+        pat_mult;        // a pattern matrix (grmkm_patterns' destination): every column's multiplicity, uint32
     cudaEvent_t ev_query[2] = {nullptr, nullptr};   // grmkm_query: device time of the call
     uint64_t racc_hint = 0;        // records of the previous abundance build + headroom
     std::vector<uint64_t> merge_h_off;   // row-block merge of a partial build: chunk offsets of the merge buckets
@@ -140,6 +146,7 @@ struct grmkm_ctx {
                                    // the stride of its capacity guess, because U is only known when the last bucket is done)
     uint32_t W = 0, G = 0;
     bool slice = false;            // the result is one owner's slice of a multi-GPU merge (grmkm_merge_partials, n_ranks > 1)
+    bool pat_mult_on = false;      // the result is a pattern matrix whose pat_mult holds its columns' multiplicities
     grmkm_stats stats{};
     grmkm_times times{};
 
@@ -1316,6 +1323,7 @@ static int build_impl(grmkm_ctx* c, uint32_t mode /*0 final, 1 partial*/, uint32
 static int build_guarded(grmkm_ctx* c, uint32_t mode, uint32_t n_ranges) {
     NvtxRange nv(mode == 0 ? "grmkm_build" : "grmkm_build_partial");
     c->slice = false;
+    c->pat_mult_on = false;
     c->scm_steps.clear(); c->scm_equiv.clear();
     c->cart_nodes.clear(); c->cart_equiv.clear();
     const int r = build_impl(c, mode, n_ranges);
@@ -1438,6 +1446,7 @@ int grmkm_reset(grmkm_ctx* c) {
     c->U = 0; c->W = 0; c->G = 0;
     c->part_ranks = 0;
     c->slice = false;
+    c->pat_mult_on = false;
     c->scm_steps.clear(); c->scm_equiv.clear();
     c->cart_nodes.clear(); c->cart_equiv.clear();
     return GRMKM_OK;
@@ -1907,6 +1916,7 @@ int grmkm_merge_partials(grmkm_ctx* c, const void* dev_parts, uint32_t n_ranks, 
         return fail(c, GRMKM_E_INVALID, "grmkm_merge_partials needs the bucket count the partial builds agreed on (grmkm_set_bucket_bits)");
     const uint32_t ob = n_ranks > 1 ? std::min(kUnitMaxBucketBits, c->cfg.bucket_bits) : 0u;
     const uint64_t own_lo = ((1ULL << ob) * rank) / n_ranks, own_hi = ((1ULL << ob) * (rank + 1)) / n_ranks;
+    c->pat_mult_on = false;
     c->scm_steps.clear(); c->scm_equiv.clear();
     c->cart_nodes.clear(); c->cart_equiv.clear();
     const int r = merge_sources(c, dev_parts, n_ranks, src_counts, src_words, total_genomes, ob, own_lo, own_hi, n_ranks, false, false);
@@ -2041,7 +2051,7 @@ int grmkm_load_result(grmkm_ctx* c, const uint64_t* kmers, const uint64_t* matri
         CU_TRY(c, cudaStreamSynchronize(c->stream));
     }
     c->U = n_kmers; c->W = W; c->G = n_genomes; c->pitch = n_kmers;
-    c->built = true; c->slice = false; c->part_ranks = 0;
+    c->built = true; c->slice = false; c->part_ranks = 0; c->pat_mult_on = false;
     c->scm_steps.clear(); c->scm_equiv.clear();
     c->cart_nodes.clear(); c->cart_equiv.clear();
     c->stats = grmkm_stats{};
@@ -2543,11 +2553,12 @@ template <bool CACHED>
 int cart_allow_smem(grmkm_ctx* c, size_t smem) {
     CU_TRY(c, cudaFuncSetAttribute(k_cart_scan<CACHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CU_TRY(c, cudaFuncSetAttribute(k_cart_ties<CACHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CU_TRY(c, cudaFuncSetAttribute(k_cart_ties<CACHED, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     return GRMKM_OK;
 }
 
 // the scan (passes bit 0) and both tie passes (bit 1) of one chunk of open nodes; CTA b covers the tiles
-// [b tpc, (b + 1) tpc).  occ: resident CTAs per SM by chunk size, filled on first use (a run sees few sizes: full chunks
+// [b tpc, (b + 1) tpc).  A pattern matrix (c->pat_mult_on) counts its tie totals in k-mers (k_cart_ties<., true>).  occ: resident CTAs per SM by chunk size, filled on first use (a run sees few sizes: full chunks
 // and the tails of its levels)
 template <bool CACHED>
 int cart_launch_chunk(grmkm_ctx* c, int passes, const CartNodeArg* d_args, uint32_t n, const uint32_t* d_bl,
@@ -2573,9 +2584,15 @@ int cart_launch_chunk(grmkm_ctx* c, int passes, const CartNodeArg* d_args, uint3
         c->stats.n_launches++;
     }
     if (passes & SCM_TIES) {
-        for (int append = 0; append < 2; ++append)
-            k_cart_ties<CACHED><<<grid, kScmThreads, smem, c->stream>>>(m, c->U, c->pitch, c->W, d_bl, d_args, n, d_masks, tpc, d_best,
-                                                                        d_tile, d_tcnt, d_total, append, d_list, d_count, cap);
+        for (int append = 0; append < 2; ++append) {
+            if (c->pat_mult_on)
+                k_cart_ties<CACHED, true><<<grid, kScmThreads, smem, c->stream>>>(
+                    m, c->U, c->pitch, c->W, d_bl, d_args, n, d_masks, tpc, d_best, d_tile, d_tcnt, d_total, append, d_list,
+                    d_count, cap, (const uint32_t*)c->pat_mult.p);
+            else
+                k_cart_ties<CACHED><<<grid, kScmThreads, smem, c->stream>>>(m, c->U, c->pitch, c->W, d_bl, d_args, n, d_masks, tpc, d_best,
+                                                                            d_tile, d_tcnt, d_total, append, d_list, d_count, cap);
+        }
         c->stats.n_launches += 2;
     }
     CU_TRY(c, cudaGetLastError());
@@ -2808,7 +2825,9 @@ int cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const u
             while (e < count && (h_list[e] >> 32) == i) ++e;
             if (h_best[i]) {            // else no admissible split: the node stays a leaf
                 const grmkm_cart_job& j = jobs[open[i].tree];
-                const uint64_t keep = std::min<uint64_t>(h_total[i], j.equiv_cap);
+                // a pattern matrix's total counts k-mers, its list patterns: the list holds every tie pattern or at
+                // least max(1, equiv_cap) of the smallest
+                const uint64_t keep = std::min<uint64_t>(c->pat_mult_on ? e - p : h_total[i], j.equiv_cap);
                 if (e - p < std::max<uint64_t>(1, keep))
                     return fail(c, GRMKM_E_CUDA, "grmkm_cart_run: the tie list of a node misses members of T");
                 std::vector<uint64_t>& eq = c->cart_equiv[open[i].tree];
@@ -3254,6 +3273,174 @@ int grmkm_copy_columns(grmkm_ctx* c, const uint64_t* idx, uint64_t n, uint64_t* 
     if (n && c->W && !dst) return fail(c, GRMKM_E_INVALID, "null dst");
     CU_TRY(c, cudaSetDevice(c->device));
     return pack_columns(c, idx, n, dst);
+}
+
+// ------------------------------------------------------------------------------------------------
+// grmkm_patterns: the distinct presence patterns of the result (grmkm_patterns.cuh)
+// ------------------------------------------------------------------------------------------------
+int grmkm_patterns(grmkm_ctx* c, const uint8_t* column_class, grmkm_ctx* d, uint32_t* pattern_of_column, uint64_t pattern_cap,
+                   uint32_t* members, uint64_t members_cap, uint64_t* member_offsets, uint64_t offsets_cap,
+                   grmkm_pattern_stats* stats) {
+    if (check_ctx(c)) return GRMKM_E_INVALID;
+    if (!d || d == c) return fail(c, GRMKM_E_INVALID, "dst must be a second context, not src");
+    if (stats && stats->struct_size != sizeof(grmkm_pattern_stats))
+        return fail(c, GRMKM_E_INVALID, "stats struct_size is not sizeof(grmkm_pattern_stats)");
+    if (!c->built) return fail(c, GRMKM_E_INVALID, "no result: call grmkm_build or grmkm_load_result first");
+    if (c->slice)
+        return fail(c, GRMKM_E_UNSUPPORTED, "the result is one owner's slice of a multi-GPU build: patterns across slices are not grouped");
+    if (d->device != c->device) return fail(c, GRMKM_E_INVALID, "dst is a context of another device");
+    const uint64_t U = c->U;
+    const uint32_t W = c->W;
+    if (U >= 0xFFFFFFFFULL) return fail(c, GRMKM_E_UNSUPPORTED, "patterns index columns with 32 bits: at most 2^32 - 2 columns");
+    if (column_class)
+        for (uint64_t j = 0; j < U; ++j)
+            if (column_class[j] > 3) return fail(c, GRMKM_E_INVALID, "column class " + std::to_string(column_class[j]) + " > 3");
+    uint32_t bits = 64;
+    if (const char* e = getenv("GRMKM_PATTERN_HASH_BITS")) bits = (uint32_t)std::min(64, std::max(1, atoi(e)));   // tests: collisions
+    CU_TRY(c, cudaSetDevice(c->device));
+    cudaStream_t st = c->stream;
+    NvtxRange nv("grmkm_patterns");
+
+    // scratch, all of it before any launch: U' = max(U, 1) columns, T = the least power of two >= 2 U' table slots
+    // (< 4 U'); per column fp 8, slot / flag 4, two active lists 8, head 4, pid 4, pattern 4, member 4, head column 8,
+    // multiplicity 4, offset 4, class 1, plus the table's 12 per slot and CUB's scan and sort scratch
+    const uint64_t Uc = std::max<uint64_t>(U, 1), U1 = Uc + 1;
+    const uint64_t tcap = 1ULL << ceil_log2(2 * Uc);
+    size_t scan_tmp = 0, sort_tmp = 0;
+    CU_TRY(c, cub::DeviceScan::ExclusiveSum(nullptr, scan_tmp, (const uint32_t*)nullptr, (uint32_t*)nullptr, (uint32_t)U1, st));
+    CU_TRY(c, cub::DeviceRadixSort::SortPairs(nullptr, sort_tmp, (const uint32_t*)nullptr, (uint32_t*)nullptr,
+                                              (const uint32_t*)nullptr, (uint32_t*)nullptr, (uint32_t)Uc, 0, 32, st));
+    auto al = [](size_t b) { return (b + 255) & ~size_t(255); };
+    const size_t o_fp = 0, o_tkey = o_fp + al(Uc * 8), o_thead = o_tkey + al(tcap * 8), o_slot = o_thead + al(tcap * 4),
+                 o_act0 = o_slot + al(U1 * 4), o_act1 = o_act0 + al(Uc * 4), o_head = o_act1 + al(Uc * 4),
+                 o_pid = o_head + al(Uc * 4), o_pat = o_pid + al(U1 * 4), o_mem = o_pat + al(Uc * 4),
+                 o_heads = o_mem + al(Uc * 4), o_mult = o_heads + al(Uc * 8), o_offs = o_mult + al(U1 * 4),
+                 o_cls = o_offs + al(U1 * 4), o_next = o_cls + al(Uc), o_tmp = o_next + 256,
+                 total = o_tmp + al(std::max(scan_tmp, sort_tmp));
+    ENSURE(c, c->pat, total);
+    uint8_t* base = (uint8_t*)c->pat.p;
+    unsigned long long* fp = (unsigned long long*)(base + o_fp);
+    unsigned long long* tkey = (unsigned long long*)(base + o_tkey);
+    uint32_t* thead = (uint32_t*)(base + o_thead);
+    uint32_t* slot_of = (uint32_t*)(base + o_slot);     // the rounds: slot of each active column; then the head flags
+    uint32_t* act[2] = {(uint32_t*)(base + o_act0), (uint32_t*)(base + o_act1)};   // then the sort's values in / keys out
+    uint32_t* head_of = (uint32_t*)(base + o_head);
+    uint32_t* pid = (uint32_t*)(base + o_pid);
+    uint32_t* pat_of = (uint32_t*)(base + o_pat);
+    uint32_t* mem = (uint32_t*)(base + o_mem);
+    unsigned long long* heads = (unsigned long long*)(base + o_heads);
+    uint32_t* mult = (uint32_t*)(base + o_mult);
+    uint32_t* offs = (uint32_t*)(base + o_offs);
+    uint8_t* cls = column_class ? base + o_cls : nullptr;
+    unsigned int* n_next = (unsigned int*)(base + o_next);
+    void* tmp = base + o_tmp;
+
+    cudaEvent_t ev[2] = {nullptr, nullptr};
+    CU_TRY(c, cudaEventCreate(&ev[0]));
+    CU_TRY(c, cudaEventCreate(&ev[1]));
+    struct EvGuard { cudaEvent_t* e; ~EvGuard() { cudaEventDestroy(e[0]); cudaEventDestroy(e[1]); } } ev_guard{ev};
+    CU_TRY(c, cudaEventRecord(ev[0], st));
+    const unsigned long long* m = (const unsigned long long*)c->matrix.p;
+    auto grid_of = [&](uint64_t n) { return (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((n + 255) / 256, (uint64_t)c->sm_count * 16)); };
+    uint32_t rounds = 0;
+    uint32_t P = 0;
+    if (U) {
+        if (cls) CU_TRY(c, cudaMemcpyAsync(cls, column_class, U, cudaMemcpyHostToDevice, st));
+        k_pat_hash<<<grid_of(U), 256, 0, st>>>(m, c->pitch, W, (uint32_t)U, cls, bits, fp);
+        CU_TRY(c, cudaGetLastError());
+        c->stats.n_launches++;
+        // rounds: every column of the round settles or moves to the next one, whose table has no settled head
+        uint32_t n = (uint32_t)U;
+        const uint32_t* cur = nullptr;          // round 1: all columns
+        for (int nxt = 0; n; ++rounds) {
+            const uint64_t T = 1ULL << ceil_log2(2 * (uint64_t)n);
+            CU_TRY(c, cudaMemsetAsync(tkey, 0xff, T * 8, st));
+            CU_TRY(c, cudaMemsetAsync(thead, 0xff, T * 4, st));
+            CU_TRY(c, cudaMemsetAsync(n_next, 0, 4, st));
+            k_pat_insert<<<grid_of(n), 256, 0, st>>>(cur, n, fp, tkey, thead, T - 1, slot_of);
+            k_pat_verify<<<grid_of(n), 256, 0, st>>>(m, c->pitch, W, cls, cur, n, slot_of, thead, head_of, act[nxt], n_next);
+            CU_TRY(c, cudaGetLastError());
+            c->stats.n_launches += 2;
+            unsigned int h_next = 0;
+            CU_TRY(c, cudaMemcpyAsync(&h_next, n_next, 4, cudaMemcpyDeviceToHost, st));
+            CU_TRY(c, cudaStreamSynchronize(st));
+            if (h_next >= n) return fail(c, GRMKM_E_CUDA, "grmkm_patterns: a grouping round settled no column");
+            n = h_next;
+            cur = act[nxt];
+            nxt ^= 1;
+        }
+        // numbering: pid = exclusive scan of the head flags (pid[U] = P)
+        k_pat_flags<<<grid_of(U + 1), 256, 0, st>>>(head_of, (uint32_t)U, slot_of);
+        CU_TRY(c, cudaGetLastError());
+        CU_TRY(c, cub::DeviceScan::ExclusiveSum(tmp, scan_tmp, (const uint32_t*)slot_of, pid, (uint32_t)(U + 1), st));
+        CU_TRY(c, cudaMemcpyAsync(&P, pid + U, 4, cudaMemcpyDeviceToHost, st));
+        CU_TRY(c, cudaMemsetAsync(mult, 0, (U + 1) * 4, st));
+        k_pat_assign<<<grid_of(U), 256, 0, st>>>(head_of, pid, (uint32_t)U, pat_of, act[0], heads, mult);
+        CU_TRY(c, cudaGetLastError());
+        CU_TRY(c, cudaStreamSynchronize(st));
+        // member offsets = exclusive scan of the multiplicities (mult[P] = 0); members = the columns stably sorted by
+        // pattern (radix sort over the bits of P - 1: the columns come in ascending order, and stay so in each pattern)
+        CU_TRY(c, cub::DeviceScan::ExclusiveSum(tmp, scan_tmp, (const uint32_t*)mult, offs, P + 1, st));
+        const int end_bit = (int)std::max<uint32_t>(1, ceil_log2(P));
+        size_t need = 0;
+        CU_TRY(c, cub::DeviceRadixSort::SortPairs(nullptr, need, (const uint32_t*)pat_of, act[1], (const uint32_t*)act[0], mem,
+                                                  (uint32_t)U, 0, end_bit, st));
+        if (need > sort_tmp) return fail(c, GRMKM_E_CUDA, "grmkm_patterns: the sort asks for more scratch than was reserved");
+        CU_TRY(c, cub::DeviceRadixSort::SortPairs(tmp, sort_tmp, (const uint32_t*)pat_of, act[1], (const uint32_t*)act[0], mem,
+                                                  (uint32_t)U, 0, end_bit, st));
+        c->stats.n_launches += 3;
+    }
+
+    // dst: the P x W matrix of the heads, their k-mers and multiplicities, copied on the device
+    if (d->aux_stream) CU_TRY(d, cudaStreamSynchronize(d->aux_stream));
+    d->built = false;
+    auto dst_ensure = [&](DevBuf& b, size_t bytes) {
+        const int r = ensure(d, b, bytes);
+        if (r) c->err = d->err;
+        return r;
+    };
+    if (int r = dst_ensure(d->kmers, (size_t)P * 8)) return r;
+    if (int r = dst_ensure(d->matrix, (size_t)P * W * 8)) return r;
+    if (int r = dst_ensure(d->pat_mult, (size_t)P * 4)) return r;
+    if (P) {
+        k_gather_columns<<<grid_of((uint64_t)P * 32), 256, 0, st>>>((const unsigned long long*)c->kmers.p, 0, 1, heads, P,
+                                                                    (unsigned long long*)d->kmers.p);
+        if (W)
+            k_gather_columns<<<grid_of((uint64_t)P * 32), 256, 0, st>>>(m, c->pitch, W, heads, P, (unsigned long long*)d->matrix.p);
+        CU_TRY(c, cudaGetLastError());
+        c->stats.n_launches += W ? 2 : 1;
+        CU_TRY(c, cudaMemcpyAsync(d->pat_mult.p, mult, (size_t)P * 4, cudaMemcpyDeviceToDevice, st));
+    }
+    CU_TRY(c, cudaEventRecord(ev[1], st));
+    CU_TRY(c, cudaStreamSynchronize(st));
+    float ms = 0.f;
+    CU_TRY(c, cudaEventElapsedTime(&ms, ev[0], ev[1]));
+    d->U = P; d->W = W; d->G = c->G; d->pitch = P;
+    d->built = true; d->slice = false; d->part_ranks = 0; d->pat_mult_on = true;
+    d->scm_steps.clear(); d->scm_equiv.clear();
+    d->cart_nodes.clear(); d->cart_equiv.clear();
+    d->stats = grmkm_stats{};
+    d->stats.n_kmers = d->stats.n_distinct = P;
+    d->stats.n_words = W; d->stats.n_genomes = c->G;
+    d->times = grmkm_times{};
+    if (stats) { stats->n_rounds = rounds; stats->n_patterns = P; stats->ms = ms; }
+
+    // the mapping to the host: what fits, or GRMKM_E_CAPACITY (dst's result stands either way)
+    const bool fits = (pattern_of_column || !U) && pattern_cap >= U && (members || !U) && members_cap >= U &&
+                      member_offsets && offsets_cap >= (uint64_t)P + 1;
+    if (U && pattern_of_column && pattern_cap >= U)
+        CU_TRY(c, cudaMemcpyAsync(pattern_of_column, pat_of, U * 4, cudaMemcpyDeviceToHost, st));
+    if (U && members && members_cap >= U) CU_TRY(c, cudaMemcpyAsync(members, mem, U * 4, cudaMemcpyDeviceToHost, st));
+    std::vector<uint32_t> h_offs(U ? (size_t)P + 1 : 0);
+    if (U && member_offsets && offsets_cap >= (uint64_t)P + 1)
+        CU_TRY(c, cudaMemcpyAsync(h_offs.data(), offs, ((size_t)P + 1) * 4, cudaMemcpyDeviceToHost, st));
+    CU_TRY(c, cudaStreamSynchronize(st));
+    if (member_offsets && offsets_cap >= (uint64_t)P + 1) {
+        for (uint32_t p = 0; p < P && U; ++p) member_offsets[p] = h_offs[p];
+        member_offsets[P] = U;
+    }
+    if (!fits) return fail(c, GRMKM_E_CAPACITY, "pattern_of_column / members need U entries, member_offsets P + 1 (P = dst's n_kmers)");
+    return GRMKM_OK;
 }
 
 }  // extern "C"

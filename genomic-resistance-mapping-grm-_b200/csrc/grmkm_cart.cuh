@@ -16,6 +16,8 @@
 //                 smallest members of T are always in the list, and the list of a node holds fewer than
 //                 need + (columns of one CTA) entries however large T is.  The list is complete for what the host
 //                 keeps or its counter says by how much it overflowed (the host grows it and redoes the level).
+//                 WEIGHTED (a pattern matrix, grmkm_patterns): total[slot] adds every tie column's multiplicity mult[j],
+//                 so it counts k-mers; tile_cnt, and with it the append cap, still counts columns (patterns).
 //   k_cart_gather pL, nL of the chosen rule of every split node (all of T share the score, not the counts).
 //   k_cart_split  P & col, P & ~col, N & col, N & ~col of every split node into the masks of its open children.
 //
@@ -123,15 +125,16 @@ k_cart_scan(const unsigned long long* __restrict__ matrix, unsigned long long U,
     }
 }
 
-// append = 0: the count pass (tile_cnt, total); append = 1: the append pass (list, count)
-template <bool CACHED>
+// append = 0: the count pass (tile_cnt, total); append = 1: the append pass (list, count).  mult: WEIGHTED only, the
+// columns' multiplicities
+template <bool CACHED, bool WEIGHTED = false>
 __global__ void __launch_bounds__(kScmThreads)
 k_cart_ties(const unsigned long long* __restrict__ matrix, unsigned long long U, unsigned long long pitch, uint32_t W,
             const uint32_t* __restrict__ blacklist, const CartNodeArg* __restrict__ args, uint32_t n,
             const unsigned long long* __restrict__ masks, unsigned long long tpc, const unsigned long long* __restrict__ best,
             const unsigned long long* __restrict__ tile_best, uint32_t* __restrict__ tile_cnt /* [n][grid] */,
             unsigned long long* __restrict__ total /* [slots] */, int append, unsigned long long* __restrict__ list,
-            unsigned long long* __restrict__ count, unsigned long long cap) {
+            unsigned long long* __restrict__ count, unsigned long long cap, const uint32_t* __restrict__ mult = nullptr) {
     static_assert(kScmWarps >= 2, "the tie passes keep two words per node in the per-warp area");
     extern __shared__ unsigned long long scm_sm[];
     const ScmShared s = scm_shared(scm_sm, n, W);
@@ -194,8 +197,9 @@ k_cart_ties(const unsigned long long* __restrict__ matrix, unsigned long long U,
                 base = __shfl_sync(0xffffffffu, base, 0);
                 const unsigned long long i = base + (unsigned long long)__popc(m & ((1u << lane) - 1u));
                 if (tie && i < cap) list[i] = ((unsigned long long)args[f].slot << 32) | j;
-            } else if (lane == 0) {
-                atomicAdd(cnt + f, (unsigned long long)__popc(m));
+            } else {
+                if (lane == 0) atomicAdd(cnt + f, (unsigned long long)__popc(m));
+                if (WEIGHTED && tie) atomicAdd(total + args[f].slot, (unsigned long long)mult[j]);
             }
         }
     }
@@ -204,7 +208,7 @@ k_cart_ties(const unsigned long long* __restrict__ matrix, unsigned long long U,
     for (uint32_t f = threadIdx.x; f < n; f += blockDim.x) {
         if (!key[f]) continue;
         tile_cnt[(size_t)f * gridDim.x + blockIdx.x] = (uint32_t)cnt[f];
-        if (cnt[f]) atomicAdd(total + args[f].slot, cnt[f]);
+        if (!WEIGHTED && cnt[f]) atomicAdd(total + args[f].slot, cnt[f]);
     }
 }
 

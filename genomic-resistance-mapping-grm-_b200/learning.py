@@ -12,6 +12,7 @@ from __future__ import annotations
 
 import numpy as np
 
+from . import native
 from .create import _minimum_uint_size
 
 
@@ -180,6 +181,182 @@ class ShardedRuleClassifications(KmerRuleClassifications):
         if self._kmers is None:
             self._kmers = self.builder.kmers() if self.col_counts[self.rank] else np.zeros(0, dtype=np.uint64)
         return self._gather_columns(lambda local: self._kmers[local][None, :], idx, 1)[0]
+
+
+def _rule_set(rule_blacklist) -> np.ndarray:
+    return np.unique(np.asarray(rule_blacklist if rule_blacklist is not None else [], dtype=np.uint64).reshape(-1))
+
+
+class PatternRuleClassifications(KmerRuleClassifications):
+    """A view of ``rc`` (a KmerRuleClassifications) that learns on one column per distinct presence pattern.
+
+    Columns with equal words score the same in every learner and fall into the same tie sets, so the SCM, CART, both
+    cross-validated selections, ``predict``, ``get_columns`` and ``sum_rows`` give on this view exactly what they give on
+    ``rc``, while their scans read P instead of U columns (``KmerMatrixBuilder.patterns``, DESIGN.md section 7f).  Every
+    index the view takes and returns is an index of the whole matrix: presence rule j, absence rule U + j; the SCM's
+    equivalent rules are complete, CART's are the ``max_equivalent_rules`` smallest, with ``equivalent_total`` in k-mers.
+
+    ``rule_blacklist`` is applied here, when the view is built: presence- and absence-blacklisted columns never share a
+    pattern with other columns.  The learners must then be called on the view with that same blacklist (or its rules in
+    any order); another one raises ValueError.  The view owns a second builder on rc's device holding the pattern matrix
+    (``pattern_builder``), and row bookkeeping of its own, starting from rc's."""
+
+    def __init__(self, rc: KmerRuleClassifications, rule_blacklist=None):
+        if rc.shard is not None or isinstance(rc, PatternRuleClassifications):
+            raise ValueError("a PatternRuleClassifications is a view of a whole matrix held by one builder: the column "
+                             "slices of a multi-GPU build, or another view, are not supported")
+        U = rc._U
+        self.rule_blacklist = _rule_set(rule_blacklist)
+        if self.rule_blacklist.size and int(self.rule_blacklist[-1]) >= 2 * U:
+            raise ValueError(f"blacklisted rule index >= 2 x {U} k-mers")
+        bl = self.rule_blacklist.astype(np.int64)
+        column_class = np.zeros(U, dtype=np.uint8)
+        column_class[bl[bl < U]] |= 1
+        column_class[bl[bl >= U] - U] |= 2
+        src = rc.builder
+        self.pattern_builder = type(src)(k=src.k, device=getattr(src, "device", -1))       # a second context, same kind
+        pattern_of, members, offsets = src.patterns(self.pattern_builder, column_class if bl.size else None)
+        self.pattern_of = pattern_of.astype(np.int64)
+        self.members = members.astype(np.int64)
+        self.member_offsets = offsets.astype(np.int64)
+        self.n_patterns = P = len(offsets) - 1
+        self.heads = self.members[self.member_offsets[:-1]]           # a pattern's first column heads its members
+        head_class = column_class[self.heads]
+        self.pattern_blacklist = np.concatenate([np.nonzero(head_class & 1)[0], P + np.nonzero(head_class & 2)[0]]
+                                                ).astype(np.uint64)
+        self._rc = rc
+        super().__init__(_PatternBuilder(self), rc.dataset_initial_n_rows)
+        self.dataset_n_rows = rc.dataset_n_rows
+        self.dataset_removed_rows = list(rc.dataset_removed_rows)
+        self.dataset_removed_rows_mask = rc.dataset_removed_rows_mask.copy()
+
+    def close(self):
+        self.pattern_builder.close()
+
+    # -- patterns <-> columns ----------------------------------------------------------------------------------------
+    def members_of(self, patterns) -> np.ndarray:
+        """The members of ``patterns`` (pattern indices), pattern after pattern, each ascending."""
+        patterns = np.asarray(patterns, dtype=np.int64).reshape(-1)
+        start = self.member_offsets[patterns]
+        count = self.member_offsets[patterns + 1] - start
+        at = np.repeat(start - (np.cumsum(count) - count), count) + np.arange(int(count.sum()), dtype=np.int64)
+        return self.members[at]
+
+    def expand_rules(self, rules) -> np.ndarray:
+        """Pattern rules (p, P + p) -> the rules of all their members (j, U + j), ascending."""
+        rules = np.asarray(rules, dtype=np.int64).reshape(-1)
+        P = self.n_patterns
+        return np.sort(np.concatenate([self.members_of(rules[rules < P]), self._U + self.members_of(rules[rules >= P] - P)]))
+
+    def rule_of_pattern(self, rules) -> np.ndarray:
+        """Pattern rules -> the rules of their first columns."""
+        rules = np.asarray(rules, dtype=np.int64)
+        P = self.n_patterns
+        return np.where(rules < P, self.heads[rules % max(P, 1)], self._U + self.heads[(rules - P) % max(P, 1)])
+
+    def pattern_rules(self, rules) -> np.ndarray:
+        """Column rules (j, U + j) -> the rules of their patterns (p, P + p)."""
+        rules = np.asarray(rules, dtype=np.int64)
+        return np.where(rules < self._U, self.pattern_of[rules % max(self._U, 1)],
+                        self.n_patterns + self.pattern_of[(rules - self._U) % max(self._U, 1)])
+
+    # -- KmerRuleClassifications ---------------------------------------------------------------------------------------
+    def get_columns(self, columns):
+        columns_is_int = hasattr(columns, "__index__")
+        columns = [columns.__index__()] if columns_is_int else [int(c) for c in columns]
+        invert = np.array([c >= self._U for c in columns], dtype=bool)
+        cols = np.array([c % self._U if c >= self._U else c for c in columns], dtype=np.int64)
+        row_mask = np.ones(self._W * 64, dtype=bool)
+        row_mask[self.dataset_initial_n_rows:] = False
+        row_mask[self.dataset_removed_rows] = False
+        result = _unpack_binary_bytes_from_ints(self.builder.columns(cols))[row_mask]
+        result[:, invert] = 1 - result[:, invert]
+        return result.reshape(-1) if columns_is_int else result
+
+    def kmers_at(self, idx) -> np.ndarray:
+        return self._rc.kmers_at(idx)
+
+
+class _PatternBuilder:
+    """The builder calls of the learners (scm_run, cart_run, eval_run, columns, sum_rows) on a
+    PatternRuleClassifications, run on its pattern matrix: column indices go in as their patterns, and patterns come
+    back as their first columns with their tie sets expanded to the members."""
+
+    world = 1
+
+    def __init__(self, view: PatternRuleClassifications):
+        self.view = view
+        self.pb = view.pattern_builder
+        self.k = self.pb.k
+
+    @property
+    def dims(self):
+        _, W, G = self.pb.dims
+        return self.view._rc._U, W, G
+
+    def _pattern_blacklist(self, blacklist) -> np.ndarray:
+        if not np.array_equal(_rule_set(blacklist), self.view.rule_blacklist):
+            raise ValueError("this PatternRuleClassifications applies the rule_blacklist it was built with; for another "
+                             "blacklist, build a PatternRuleClassifications(rc, rule_blacklist) with that blacklist")
+        return self.view.pattern_blacklist
+
+    @staticmethod
+    def _no_shard(shard):
+        if shard is not None:
+            raise ValueError("a PatternRuleClassifications holds a whole matrix: it takes no shard")
+
+    def scm_run(self, jobs, blacklist=(), shard=None):
+        self._no_shard(shard)
+        v = self.view
+        out = []
+        for steps, eq in self.pb.scm_run(jobs, self._pattern_blacklist(blacklist)):
+            steps = steps.copy()
+            lists = [v.expand_rules(eq[int(s["equiv_offset"]):int(s["equiv_offset"]) + int(s["equiv_count"])]) for s in steps]
+            counts = np.array([len(x) for x in lists], dtype=np.uint64)
+            steps["equiv_count"] = counts
+            steps["equiv_offset"] = np.cumsum(counts) - counts
+            steps["rule"] = v.rule_of_pattern(steps["rule"].astype(np.int64)).astype(np.uint64)
+            out.append((steps, np.concatenate(lists).astype(np.uint64) if lists else np.zeros(0, dtype=np.uint64)))
+        return out
+
+    def cart_run(self, jobs, blacklist=(), shard=None):
+        self._no_shard(shard)
+        v = self.view
+        out = []
+        for job, (nodes, eq) in zip(jobs, self.pb.cart_run(jobs, self._pattern_blacklist(blacklist))):
+            cap = int(job[2])
+            nodes = nodes.copy()
+            # the recorded tie patterns are the smallest ones, and they hold the cap smallest tie k-mers
+            lists = [np.sort(v.members_of(eq[int(x["equiv_offset"]):int(x["equiv_offset"]) + int(x["equiv_count"])]))[:cap]
+                     for x in nodes]
+            counts = np.array([len(x) for x in lists], dtype=np.uint64)
+            nodes["equiv_count"] = counts
+            nodes["equiv_offset"] = np.cumsum(counts) - counts
+            split = nodes["present_child"] != 0xFFFFFFFF
+            nodes["rule"][split] = v.heads[nodes["rule"][split].astype(np.int64)].astype(np.uint64)
+            out.append((nodes, np.concatenate(lists).astype(np.uint64) if lists else np.zeros(0, dtype=np.uint64)))
+        return out
+
+    def eval_run(self, jobs, shard=None):
+        self._no_shard(shard)
+        v = self.view
+        mapped = []
+        for kind, model_type, items, pos, neg in jobs:
+            if kind == native.EVAL_SCM:
+                items = v.pattern_rules(np.asarray(items, dtype=np.int64).reshape(-1)).astype(np.uint64)
+            else:
+                from .builder import KmerMatrixBuilder
+                items = np.array(items, dtype=KmerMatrixBuilder.EVAL_NODE_DTYPE).reshape(-1)
+                split = items["kmer"] != np.iinfo(np.uint64).max
+                items["kmer"][split] = v.pattern_of[items["kmer"][split].astype(np.int64)].astype(np.uint64)
+            mapped.append((kind, model_type, items, pos, neg))
+        return self.pb.eval_run(mapped)
+
+    def columns(self, idx) -> np.ndarray:
+        return self.pb.columns(self.view.pattern_of[np.asarray(idx, dtype=np.int64).reshape(-1)])
+
+    def sum_rows(self, row_mask) -> np.ndarray:
+        return self.pb.sum_rows(row_mask)[self.view.pattern_of]
 
 
 _BASE_CODE = np.full(256, 255, dtype=np.uint64)

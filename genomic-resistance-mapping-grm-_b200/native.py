@@ -6,7 +6,7 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("GRMKM_LIB") or os.path.join(_HERE, "libgrmkm.so")   # GRMKM_LIB: another build of the same library (kernel experiments)
-ABI_VERSION = 15
+ABI_VERSION = 16
 
 OK = 0
 E_INVALID, E_UNSUPPORTED_K, E_NOMEM, E_CUDA, E_IO, E_CAPACITY, E_NO_DEVICE, E_UNSUPPORTED = -1, -2, -3, -4, -5, -6, -7, -8
@@ -25,6 +25,7 @@ SYMBOLS = [
     "grmkm_load_result", "grmkm_scm_run", "grmkm_scm_result",
     "grmkm_cart_run", "grmkm_cart_result", "grmkm_query", "grmkm_eval_run",
     "grmkm_scm_run_sharded", "grmkm_cart_run_sharded", "grmkm_eval_run_sharded", "grmkm_copy_columns",
+    "grmkm_patterns",
 ]
 SCM_CONJUNCTION, SCM_DISJUNCTION = 0, 1
 EVAL_SCM, EVAL_CART = 0, 1
@@ -105,6 +106,13 @@ class EvalJob(C.Structure):
                 ("neg", C.c_void_p)]
 
 
+class PatternStats(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("n_rounds", C.c_uint32), ("n_patterns", C.c_uint64), ("ms", C.c_float)]
+
+    def asdict(self):
+        return {n: (float if n == "ms" else int)(getattr(self, n)) for n, _ in self._fields_ if n != "struct_size"}
+
+
 # int exchange(void* user, const void* send, uint64_t n, const void** recv, uint64_t* sizes): the all-gather of the
 # sharded runs
 EXCHANGE_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64))
@@ -174,6 +182,7 @@ def load() -> C.CDLL:
         "grmkm_cart_run_sharded": (i32, [vp, u32, vp, vp, u64, C.POINTER(Shard)]),
         "grmkm_eval_run_sharded": (i32, [vp, u32, vp, vp, u64, C.POINTER(Shard)]),
         "grmkm_copy_columns": (i32, [vp, vp, u64, vp, u64]),
+        "grmkm_patterns": (i32, [vp, vp, vp, vp, u64, vp, u64, vp, u64, C.POINTER(PatternStats)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)

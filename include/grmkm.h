@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define GRMKM_ABI_VERSION 15
+#define GRMKM_ABI_VERSION 16
 
 enum {
     GRMKM_OK = 0,
@@ -463,6 +463,43 @@ int grmkm_eval_run_sharded(grmkm_ctx* ctx, uint32_t n_jobs, const grmkm_eval_job
  * row-major), packed on the device: the columns a model needs without copying the whole matrix.  idx[i] >= n_kmers or
  * n >= 2^32: GRMKM_E_INVALID; cap < n_words x n: GRMKM_E_CAPACITY. */
 int grmkm_copy_columns(grmkm_ctx* ctx, const uint64_t* idx, uint64_t n, uint64_t* dst, uint64_t cap);
+
+/*
+ * Distinct presence patterns: the columns of src's result grouped by exact equality of their n_words words and of
+ * column_class[j] (U bytes, each 0..3, or NULL: all 0), a pattern numbered by its first column (patterns 0..P-1 in the
+ * order of their least member).  k-mers that share one presence vector (the k-mers of one variant, of one accessory
+ * island, of the core genome) score the same in every learner, so learning on one column per pattern gives the
+ * result of the whole matrix once the tie sets are expanded back to their members (DESIGN.md section 7f).
+ *
+ *   dst                a second context of the same device: its result becomes the P x n_words pattern matrix (column p =
+ *                      the words of pattern p), its k-mers the k-mers of the patterns' first columns, its genome count
+ *                      src's; copied on the device.  dst's result carries every pattern's multiplicity (its number of
+ *                      members) until its next build / load / reset / grmkm_patterns: grmkm_cart_run on it then reports
+ *                      equiv_total as the sum of the tie patterns' multiplicities (|T| in k-mers), while equiv_cap still
+ *                      counts patterns (the smallest tie patterns are recorded; their members hold the smallest tie k-mers).
+ *   pattern_of_column  [U]: the pattern of every column.
+ *   members            [U]: the columns of pattern 0 ascending, then those of pattern 1, ...
+ *   member_offsets     [P + 1]: the members of pattern p are members[member_offsets[p] .. member_offsets[p + 1]).
+ *   stats              may be NULL: grouping rounds, P, device time of the call (CUDA events).
+ *
+ * A NULL or short buffer: GRMKM_E_CAPACITY, the others are still filled and dst's result stands (P = dst's n_kmers,
+ * U + 1 offsets always suffice).  Rejected before any device work: src == dst, dst NULL or on another device, src
+ * without a result, a class byte > 3, a bad stats->struct_size (GRMKM_E_INVALID); a result that is one owner's slice
+ * of a multi-GPU merge, U >= 2^32 - 1 (GRMKM_E_UNSUPPORTED); device scratch of about 109 U bytes (fingerprints, the
+ * grouping table, ids and CSR) plus CUB's sort scratch that cannot be allocated (GRMKM_E_NOMEM).  The P x n_words
+ * matrix is allocated in dst once P is known.  The result does not depend on the grid or the order of atomics.
+ * GRMKM_PATTERN_HASH_BITS=n (1..64) truncates the fingerprint, for tests of the collision rounds.
+ */
+typedef struct grmkm_pattern_stats {
+    uint32_t struct_size;        /* = sizeof(grmkm_pattern_stats) */
+    uint32_t n_rounds;           /* grouping rounds: 1 unless fingerprints of different patterns collided */
+    uint64_t n_patterns;         /* P */
+    float ms;                    /* device time of the call, CUDA events on src's stream */
+} grmkm_pattern_stats;
+
+int grmkm_patterns(grmkm_ctx* src, const uint8_t* column_class, grmkm_ctx* dst, uint32_t* pattern_of_column,
+                   uint64_t pattern_cap, uint32_t* members, uint64_t members_cap, uint64_t* member_offsets,
+                   uint64_t offsets_cap, grmkm_pattern_stats* stats);
 
 #ifdef __cplusplus
 }
