@@ -22,7 +22,7 @@ from collections import namedtuple
 
 import numpy as np
 
-from .scm import KmerRule, _kmer_string, _refuse_slices, _row_mask
+from .scm import KmerRule, _kmer_string, _refuse_slices
 
 # rule: the split's KmerRule (type "presence": its examples go to present_child), None for a leaf.  prediction: the
 # leaf's output (1 iff w_pos * n_pos > w_neg * n_neg).  equivalent_rules: the k-mer indices of the splits tied with it
@@ -109,12 +109,11 @@ def fit_many(rule_classifications, trees, rule_blacklist=None):
     _refuse_slices(rule_classifications)
     rc = rule_classifications
     b = rc.builder
-    W = rc._W
     jobs = []
     for t, pos, neg in trees:
         jobs.append((_UNLIMITED_DEPTH if t.max_depth is None else t.max_depth, t.min_samples_split,
                      _ALL_EQUIVALENT if t.max_equivalent_rules is None else t.max_equivalent_rules,
-                     t.class_importance[0], t.class_importance[1], _row_mask(rc, pos, W), _row_mask(rc, neg, W)))
+                     t.class_importance[0], t.class_importance[1], rc.row_mask(pos), rc.row_mask(neg)))
     blacklist = np.asarray(rule_blacklist if rule_blacklist is not None else [], dtype=np.uint64).reshape(-1)
     results = b.cart_run(jobs, blacklist, shard=rc.shard)
     needed = sorted({int(x["rule"]) for nodes, _ in results for x in nodes if int(x["present_child"]) != 0xFFFFFFFF})

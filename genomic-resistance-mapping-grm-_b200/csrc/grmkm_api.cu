@@ -1318,14 +1318,34 @@ static int build_impl(grmkm_ctx* c, uint32_t mode /*0 final, 1 partial*/, uint32
     return GRMKM_OK;
 }
 
-// every failure of a build leaves the context quiet: nothing in flight reads borrowed host buffers any more, and no
-// side-stream clear is counted on
-static int build_guarded(grmkm_ctx* c, uint32_t mode, uint32_t n_ranges) {
-    NvtxRange nv(mode == 0 ? "grmkm_build" : "grmkm_build_partial");
+// What described the last result goes with it: its slice flag, pattern multiplicities and learners' results (all that
+// goes in the owner-side merge of a multi-GPU build, which sets built itself and keeps the partial state it merged)
+static void forget_result(grmkm_ctx* c) {
     c->slice = false;
     c->pat_mult_on = false;
     c->scm_steps.clear(); c->scm_equiv.clear();
     c->cart_nodes.clear(); c->cart_equiv.clear();
+}
+
+// A result replaces the last one.  built: the U x W matrix over G genomes in place is whole (patterns: a pattern matrix),
+// and the stats and times restart from it; else there is none, whole or partial (a reset, a build until it succeeds).
+static void set_result(grmkm_ctx* c, bool built, bool patterns = false) {
+    forget_result(c);
+    c->built = built;
+    c->part_ranks = 0;
+    c->pat_mult_on = patterns;
+    if (!built) return;
+    c->stats = grmkm_stats{};
+    c->stats.n_kmers = c->stats.n_distinct = c->U;
+    c->stats.n_words = c->W; c->stats.n_genomes = c->G;
+    c->times = grmkm_times{};
+}
+
+// every failure of a build leaves the context quiet: nothing in flight reads borrowed host buffers any more, and no
+// side-stream clear is counted on
+static int build_guarded(grmkm_ctx* c, uint32_t mode, uint32_t n_ranges) {
+    NvtxRange nv(mode == 0 ? "grmkm_build" : "grmkm_build_partial");
+    set_result(c, false);
     const int r = build_impl(c, mode, n_ranges);
     if (r != GRMKM_OK) {
         const std::string msg = c->err;
@@ -1334,8 +1354,7 @@ static int build_guarded(grmkm_ctx* c, uint32_t mode, uint32_t n_ranges) {
         if (c->aux_stream) cudaStreamSynchronize(c->aux_stream);
         cudaGetLastError();
         c->pre_pending = false;
-        c->built = false;
-        c->part_ranks = 0;
+        set_result(c, false);
         c->err = msg;
     }
     return r;
@@ -1442,13 +1461,8 @@ int grmkm_reset(grmkm_ctx* c) {
     if (check_ctx(c)) return GRMKM_E_INVALID;
     c->inputs.clear();
     c->n_genomes_decl = 0;
-    c->built = false;
     c->U = 0; c->W = 0; c->G = 0;
-    c->part_ranks = 0;
-    c->slice = false;
-    c->pat_mult_on = false;
-    c->scm_steps.clear(); c->scm_equiv.clear();
-    c->cart_nodes.clear(); c->cart_equiv.clear();
+    set_result(c, false);
     return GRMKM_OK;
 }
 
@@ -1916,9 +1930,7 @@ int grmkm_merge_partials(grmkm_ctx* c, const void* dev_parts, uint32_t n_ranks, 
         return fail(c, GRMKM_E_INVALID, "grmkm_merge_partials needs the bucket count the partial builds agreed on (grmkm_set_bucket_bits)");
     const uint32_t ob = n_ranks > 1 ? std::min(kUnitMaxBucketBits, c->cfg.bucket_bits) : 0u;
     const uint64_t own_lo = ((1ULL << ob) * rank) / n_ranks, own_hi = ((1ULL << ob) * (rank + 1)) / n_ranks;
-    c->pat_mult_on = false;
-    c->scm_steps.clear(); c->scm_equiv.clear();
-    c->cart_nodes.clear(); c->cart_equiv.clear();
+    forget_result(c);
     const int r = merge_sources(c, dev_parts, n_ranks, src_counts, src_words, total_genomes, ob, own_lo, own_hi, n_ranks, false, false);
     c->slice = r == GRMKM_OK && n_ranks > 1;
     return r;
@@ -2051,14 +2063,8 @@ int grmkm_load_result(grmkm_ctx* c, const uint64_t* kmers, const uint64_t* matri
         CU_TRY(c, cudaStreamSynchronize(c->stream));
     }
     c->U = n_kmers; c->W = W; c->G = n_genomes; c->pitch = n_kmers;
-    c->built = true; c->slice = false; c->part_ranks = 0; c->pat_mult_on = false;
-    c->scm_steps.clear(); c->scm_equiv.clear();
-    c->cart_nodes.clear(); c->cart_equiv.clear();
-    c->stats = grmkm_stats{};
-    c->stats.n_kmers = c->stats.n_distinct = n_kmers;
-    c->stats.n_words = W; c->stats.n_genomes = n_genomes;
+    set_result(c, true);
     c->stats.h2d_bytes = n_kmers * (W + 1) * 8;
-    c->times = grmkm_times{};
     return GRMKM_OK;
 }
 
@@ -2090,14 +2096,16 @@ struct Shard {
     uint64_t global_rule(uint64_t r, uint64_t U) const { return r < U ? off + r : total + off + (r - U); }
 };
 
-Shard whole_matrix(const grmkm_ctx* c) {
-    Shard s;
-    s.total = c->U;
-    s.offs = {0, c->U};
-    return s;
-}
-
-int shard_from(grmkm_ctx* c, const grmkm_shard* in, Shard& s) {
+// The Shard of a learner entry point: the plain call (refusal: what it answers for a slice) runs on the whole matrix,
+// the sharded call (refusal null) on the slice `in` describes.
+int run_shard(grmkm_ctx* c, const grmkm_shard* in, const char* refusal, Shard& s) {
+    if (check_ctx(c)) return GRMKM_E_INVALID;
+    if (refusal) {
+        if (c->built && c->slice) return fail(c, GRMKM_E_UNSUPPORTED, refusal);
+        s.total = c->U;
+        s.offs = {0, c->U};
+        return GRMKM_OK;
+    }
     if (!in) return fail(c, GRMKM_E_INVALID, "null shard");
     if (in->struct_size != sizeof(grmkm_shard)) return fail(c, GRMKM_E_INVALID, "shard struct_size is not sizeof(grmkm_shard)");
     if (!in->exchange) return fail(c, GRMKM_E_INVALID, "null shard exchange");
@@ -2176,45 +2184,136 @@ int pack_columns(grmkm_ctx* c, const uint64_t* idx, uint64_t m, uint64_t* dst) {
     return GRMKM_OK;
 }
 
-// The compact matrix [W][cols.size()] of the global columns `cols` (the same list on every rank), in c->shard_cols:
-// every rank packs the columns it owns (k_gather_columns), one exchange, every rank assembles and uploads the whole.
-int shard_columns(grmkm_ctx* c, const Shard& s, const std::vector<uint64_t>& cols, const unsigned long long** out) {
+// The matrix a step reads the columns it chose from.  On the whole matrix it is the resident one and global column j is
+// its column j.  On a slice it is the compact [W][n] matrix of the n distinct chosen columns, and global column j is its
+// position among them.
+struct ColumnView {
+    const unsigned long long* matrix = nullptr;
+    uint64_t U = 0, pitch = 0;
+    bool whole = true;
+    std::vector<uint64_t> cols;             // a slice's view: the distinct global columns, ascending
+    uint64_t col(uint64_t j) const {
+        return whole ? j : (uint64_t)(std::lower_bound(cols.begin(), cols.end(), j) - cols.begin());
+    }
+    // a global rule (j or UG + j) -> the rule of the view (col(j) or U + col(j))
+    uint64_t rule(uint64_t r, uint64_t UG) const { return col(r % UG) + (r >= UG ? U : 0); }
+};
+
+// cols: the global columns the step needs, the same list on every rank (any order, repeats allowed).  On a slice every
+// rank packs the ones it owns (k_gather_columns), one exchange, and every rank assembles the whole in c->shard_cols.
+int column_view(grmkm_ctx* c, const Shard& sh, std::vector<uint64_t> cols, ColumnView& v) {
+    v.matrix = (const unsigned long long*)c->matrix.p;
+    v.whole = !sh.on();
+    if (v.whole) {
+        v.U = c->U; v.pitch = c->pitch;
+        return GRMKM_OK;
+    }
+    std::sort(cols.begin(), cols.end());
+    cols.erase(std::unique(cols.begin(), cols.end()), cols.end());
+    v.cols = std::move(cols);
     const uint32_t W = c->W;
-    const uint64_t n = cols.size();
-    std::vector<uint64_t> own, cnt(s.n_ranks, 0);
-    for (uint64_t j : cols) {
-        const uint32_t o = s.owner(j);
+    const uint64_t n = v.U = v.pitch = v.cols.size();
+    if (!n) return GRMKM_OK;
+    std::vector<uint64_t> own, cnt(sh.n_ranks, 0);
+    for (uint64_t j : v.cols) {
+        const uint32_t o = sh.owner(j);
         ++cnt[o];
-        if (o == s.rank) own.push_back(j - s.off);
+        if (o == sh.rank) own.push_back(j - sh.off);
     }
     const uint64_t m = own.size();
     std::vector<uint64_t> packed(m * W);
     if (int r = pack_columns(c, own.data(), m, packed.data())) return r;
     Gathered g;
-    if (int r = shard_exchange(c, s, packed.data(), m * W * 8, g)) return r;
-    for (uint32_t r = 0; r < s.n_ranks; ++r)
+    if (int r = shard_exchange(c, sh, packed.data(), m * W * 8, g)) return r;
+    for (uint32_t r = 0; r < sh.n_ranks; ++r)
         if (g.len[r] != cnt[r] * W * 8) return fail(c, GRMKM_E_INVALID, "rank " + std::to_string(r) + " sent other columns");
-    std::vector<uint64_t> h(n * W), at(s.n_ranks, 0);
+    std::vector<uint64_t> h(n * W), at(sh.n_ranks, 0);
     for (uint64_t i = 0; i < n; ++i) {
-        const uint32_t o = s.owner(cols[i]);
+        const uint32_t o = sh.owner(v.cols[i]);
         const uint64_t k = at[o]++;
         for (uint32_t w = 0; w < W; ++w) memcpy(&h[(uint64_t)w * n + i], g.blk[o] + ((uint64_t)w * cnt[o] + k) * 8, 8);
     }
     ENSURE(c, c->shard_cols, n * W * 8);
     CU_TRY(c, cudaMemcpyAsync(c->shard_cols.p, h.data(), n * W * 8, cudaMemcpyHostToDevice, c->stream));
     CU_TRY(c, cudaStreamSynchronize(c->stream));
-    *out = (const unsigned long long*)c->shard_cols.p;
+    v.matrix = (const unsigned long long*)c->shard_cols.p;
     return GRMKM_OK;
 }
 
-// the position of every global column in the ascending list of the distinct ones
-std::vector<uint64_t> distinct(std::vector<uint64_t> v) {
-    std::sort(v.begin(), v.end());
-    v.erase(std::unique(v.begin(), v.end()), v.end());
-    return v;
+// The exchange between the scan and the tie pass: keys[i] = the max of keys[i] over the ranks, the global best.
+// Nothing is exchanged on the whole matrix.  other: the error for a rank that sent another number of keys.
+int shard_max(grmkm_ctx* c, const Shard& sh, std::vector<uint64_t>& keys, const char* other) {
+    if (!sh.on()) return GRMKM_OK;
+    Gathered g;
+    if (int r = shard_exchange(c, sh, keys.data(), keys.size() * 8, g)) return r;
+    for (uint32_t q = 0; q < sh.n_ranks; ++q) {
+        if (g.len[q] != keys.size() * 8) return fail(c, GRMKM_E_INVALID, other);
+        for (size_t i = 0; i < keys.size(); ++i) {
+            uint64_t x;
+            memcpy(&x, g.blk[q] + i * 8, 8);
+            keys[i] = std::max(keys[i], x);
+        }
+    }
+    return GRMKM_OK;
 }
-uint64_t position(const std::vector<uint64_t>& cols, uint64_t j) {
-    return (uint64_t)(std::lower_bound(cols.begin(), cols.end(), j) - cols.begin());
+
+struct TieList { uint64_t n; const uint8_t* p; };       // one rank's tie list: n entries, its payload at p
+
+// The exchange of the tie lists after the tie pass.  A rank sends [count][payload] with a payload of fixed + per x count
+// bytes (the caller's, from block[1] on), or the count alone when its list overflowed (over: count > the list's
+// capacity).  If any rank's list overflowed, any_over is set and every rank grows its list and redoes the step, so the
+// union is never short; else lists holds every rank's list in rank order.  On the whole matrix the one list is this rank's.
+int shard_ties(grmkm_ctx* c, const Shard& sh, uint64_t count, bool over, std::vector<uint64_t>& block, uint64_t fixed,
+               uint64_t per, std::vector<TieList>& lists, bool& any_over) {
+    any_over = over;
+    lists.assign(1, TieList{count, (const uint8_t*)(block.data() + 1)});
+    if (!sh.on()) return GRMKM_OK;
+    block[0] = count;
+    Gathered g;
+    if (int r = shard_exchange(c, sh, block.data(), 8 + (over ? 0 : fixed + per * count), g)) return r;
+    lists.clear();
+    for (uint32_t q = 0; q < sh.n_ranks; ++q) {
+        uint64_t n = 0;
+        if (g.len[q] < 8) return fail(c, GRMKM_E_INVALID, "a rank sent no tie list");
+        memcpy(&n, g.blk[q], 8);
+        if (g.len[q] == 8 && n) { any_over = true; continue; }         // an overflow: the count only
+        if (g.len[q] != 8 + fixed + per * n) return fail(c, GRMKM_E_INVALID, "a rank sent a malformed tie list");
+        lists.push_back(TieList{n, g.blk[q] + 8});
+    }
+    return GRMKM_OK;
+}
+
+// fits or nodes per chunk: as many as share one CTA's shared memory at per_item bytes each, small enough for two CTAs
+// per SM
+uint32_t chunk_size(const grmkm_ctx* c, size_t per_item) {
+    const size_t smem_cap = (c->smem_optin ? c->smem_optin : 227 * 1024) - 1024;
+    return (uint32_t)std::max<size_t>(1, std::min<size_t>(smem_cap / 2, 64 * 1024) / per_item);
+}
+
+// What every learner run checks first: a result, at most 2^31 - 1 k-mers where the learner indexes them with 32 bits
+// (limit: how it says so; null where it does not), and the blacklist.
+int check_run(grmkm_ctx* c, const Shard& sh, const char* limit, const uint64_t* blacklist, uint64_t n_blacklist) {
+    if (!c->built) return fail(c, GRMKM_E_INVALID, "no result: call grmkm_build or grmkm_load_result first");
+    if (limit && sh.total >= (1ULL << 31))
+        return fail(c, GRMKM_E_UNSUPPORTED, std::string(limit) + " with 32 bits: at most 2^31 - 1 k-mers");
+    if (n_blacklist && !blacklist) return fail(c, GRMKM_E_INVALID, "null blacklist");
+    for (uint64_t i = 0; i < n_blacklist; ++i)
+        if (blacklist[i] >= 2 * sh.total) return fail(c, GRMKM_E_INVALID, "blacklisted rule index >= 2 x n_kmers");
+    return GRMKM_OK;
+}
+
+// a job's example masks: not null, no bits at rows >= n_genomes, no example both positive and negative (at: the job)
+int check_examples(grmkm_ctx* c, const uint64_t* pos, const uint64_t* neg, const std::string& at) {
+    const uint32_t W = c->W;
+    if (!W) return GRMKM_OK;
+    for (const auto& [m, what] : {std::pair{pos, "positive"}, std::pair{neg, "negative"}}) {
+        if (!m) return fail(c, GRMKM_E_INVALID, std::string("null ") + what + " mask");
+        if (c->G % 64 && (m[W - 1] & (~0ULL >> (c->G % 64))))
+            return fail(c, GRMKM_E_INVALID, std::string("the ") + what + " mask has bits at rows >= n_genomes");
+    }
+    for (uint32_t w = 0; w < W; ++w)
+        if (pos[w] & neg[w]) return fail(c, GRMKM_E_INVALID, "positive and negative examples overlap" + at);
+    return GRMKM_OK;
 }
 
 // SCM passes over this rank's columns: bit 0 the scan, bit 1 the tie pass (the same grid in both)
@@ -2246,21 +2345,10 @@ int scm_launch_chunk(grmkm_ctx* c, int passes, const ScmFitArg* d_args, uint32_t
     return GRMKM_OK;
 }
 
-int scm_check_mask(grmkm_ctx* c, const uint64_t* m, const char* what) {
-    if (!m) return fail(c, GRMKM_E_INVALID, std::string("null ") + what + " mask");
-    if (c->G % 64 && (m[c->W - 1] & (~0ULL >> (c->G % 64))))
-        return fail(c, GRMKM_E_INVALID, std::string("the ") + what + " mask has bits at rows >= n_genomes");
-    return GRMKM_OK;
-}
-
 int scm_validate(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, const uint64_t* blacklist, uint64_t n_blacklist,
                  const Shard& sh) {
-    if (!c->built) return fail(c, GRMKM_E_INVALID, "no result: call grmkm_build or grmkm_load_result first");
-    const uint64_t UG = sh.total;
-    const uint32_t W = c->W;
-    if (UG >= (1ULL << 31)) return fail(c, GRMKM_E_UNSUPPORTED, "the SCM indexes rules with 32 bits: at most 2^31 - 1 k-mers");
+    if (int r = check_run(c, sh, "the SCM indexes rules", blacklist, n_blacklist)) return r;
     if (n_fits && !jobs) return fail(c, GRMKM_E_INVALID, "null jobs");
-    if (n_blacklist && !blacklist) return fail(c, GRMKM_E_INVALID, "null blacklist");
     for (uint32_t f = 0; f < n_fits; ++f) {
         const grmkm_scm_job& j = jobs[f];
         const std::string at = " (fit " + std::to_string(f) + ")";
@@ -2269,23 +2357,18 @@ int scm_validate(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, const
         if (j.max_rules == 0) return fail(c, GRMKM_E_INVALID, "max_rules must be at least 1" + at);
         if (j.tiebreak > 1) return fail(c, GRMKM_E_INVALID, "tiebreak must be 0 or 1" + at);
         if (!(j.p >= 0.0) || j.p > 1.7976931348623157e308) return fail(c, GRMKM_E_INVALID, "p must be finite and >= 0" + at);
-        if (W) {
-            int r = scm_check_mask(c, j.pos, "positive");
-            if (!r) r = scm_check_mask(c, j.neg, "negative");
-            if (r) return r;
-            for (uint32_t w = 0; w < W; ++w)
-                if (j.pos[w] & j.neg[w]) return fail(c, GRMKM_E_INVALID, "positive and negative examples overlap" + at);
-        }
+        if (int r = check_examples(c, j.pos, j.neg, at)) return r;
     }
-    for (uint64_t i = 0; i < n_blacklist; ++i)
-        if (blacklist[i] >= 2 * UG) return fail(c, GRMKM_E_INVALID, "blacklisted rule index >= 2 x n_kmers");
     return GRMKM_OK;
 }
 
 // The greedy loop of a batch of fits on this rank's columns; sh: the whole matrix (no exchange) or one slice of it.
 // Sharded, each step is: scan -> exchange the best keys -> tie pass and statistics against the global keys -> exchange
 // the tie lists -> the same host selection on every rank -> exchange the chosen columns -> update the masks.
-int scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, const uint64_t* blacklist, uint64_t n_blacklist, Shard& sh) {
+int scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, const uint64_t* blacklist, uint64_t n_blacklist,
+            const grmkm_shard* shard, const char* refusal) {
+    Shard sh;
+    if (int r = run_shard(c, shard, refusal, sh)) return r;
     if (int r = shard_agree(c, sh, scm_validate(c, n_fits, jobs, blacklist, n_blacklist, sh))) return r;
     const uint64_t U = c->U, UG = sh.total;
     const uint32_t W = c->W;
@@ -2315,10 +2398,7 @@ int scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, const uint
     if (std::find(done.begin(), done.end(), 0) == done.end()) return GRMKM_OK;
 
     CU_TRY(c, cudaSetDevice(c->device));
-    // chunk = fits whose masks share one CTA's shared memory; small enough for two CTAs per SM
-    const size_t smem_cap = (c->smem_optin ? c->smem_optin : 227 * 1024) - 1024;
-    const size_t per_fit = scm_smem_bytes(1, W);
-    const uint32_t chunk = (uint32_t)std::max<size_t>(1, std::min<size_t>(smem_cap / 2, 64 * 1024) / per_fit);
+    const uint32_t chunk = chunk_size(c, scm_smem_bytes(1, W));
     const uint64_t bl_words = (2 * U + 31) / 32;
     const uint64_t max_grid = (uint64_t)c->sm_count * 8;
     // sharded, the tie pass runs after the exchange of the keys: every chunk keeps its per-CTA bests until then
@@ -2352,7 +2432,7 @@ int scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, const uint
     std::vector<uint64_t> h_list, h_best(n_fits), sel, keys, block, cols;
     std::vector<uint32_t> h_stats;
     std::vector<size_t> order;
-    Gathered g;
+    std::vector<TieList> lists;
     auto launch = [&](int passes) -> int {
         for (size_t a0 = 0; a0 < args.size(); a0 += chunk) {
             const uint32_t n = (uint32_t)std::min<size_t>(chunk, args.size() - a0);
@@ -2385,17 +2465,8 @@ int scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, const uint
             CU_TRY(c, cudaStreamSynchronize(c->stream));
             keys.resize(args.size());
             for (size_t a = 0; a < args.size(); ++a) keys[a] = h_best[args[a].fit];
-            if (int r = shard_exchange(c, sh, keys.data(), keys.size() * 8, g)) return r;
-            for (size_t a = 0; a < args.size(); ++a) {
-                uint64_t k = 0;
-                for (uint32_t q = 0; q < sh.n_ranks; ++q) {
-                    if (g.len[q] != keys.size() * 8) return fail(c, GRMKM_E_INVALID, "a rank sent keys of other fits");
-                    uint64_t x;
-                    memcpy(&x, g.blk[q] + a * 8, 8);
-                    k = std::max(k, x);
-                }
-                h_best[args[a].fit] = k;
-            }
+            if (int r = shard_max(c, sh, keys, "a rank sent keys of other fits")) return r;
+            for (size_t a = 0; a < args.size(); ++a) h_best[args[a].fit] = keys[a];
             CU_TRY(c, cudaMemcpyAsync(d_best, h_best.data(), (size_t)n_fits * 8, cudaMemcpyHostToDevice, c->stream));
             if (int r = launch(SCM_TIES)) return r;
         }
@@ -2420,29 +2491,22 @@ int scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, const uint
         if (!sharded) CU_TRY(c, cudaMemcpyAsync(h_best.data(), d_best, (size_t)n_fits * 8, cudaMemcpyDeviceToHost, c->stream));
         CU_TRY(c, cudaStreamSynchronize(c->stream));
         if (sharded) {
-            // exchange 2: [count][list, global rules][statistics]; an overflow anywhere redoes the step on every rank
+            // exchange 2: the tie lists with global rules, then their statistics (20 bytes per entry)
             block.assign(1 + n_local + (n_local * 3 + 1) / 2, 0);
-            block[0] = count;
             for (uint64_t i = 0; i < n_local; ++i)
                 block[1 + i] = (h_list[i] & ~0xffffffffULL) | sh.global_rule(h_list[i] & 0xffffffffULL, U);
             if (n_local) memcpy(block.data() + 1 + n_local, h_stats.data(), n_local * 12);
-            if (int r = shard_exchange(c, sh, block.data(), block.size() * 8, g)) return r;
             bool any_over = false;
-            h_list.clear(); h_stats.clear();
-            for (uint32_t q = 0; q < sh.n_ranks; ++q) {
-                uint64_t nq = 0;
-                if (g.len[q] < 8) return fail(c, GRMKM_E_INVALID, "a rank sent no tie list");
-                memcpy(&nq, g.blk[q], 8);
-                if (g.len[q] == 8) { any_over |= nq > 0; continue; }       // no ties, or an overflow: the count only
-                const uint64_t n = nq;
-                if (g.len[q] != 8 * (1 + n + (n * 3 + 1) / 2)) return fail(c, GRMKM_E_INVALID, "a rank sent a malformed tie list");
-                const size_t l0 = h_list.size();
-                h_list.resize(l0 + n); h_stats.resize((l0 + n) * 3);
-                memcpy(h_list.data() + l0, g.blk[q] + 8, n * 8);
-                memcpy(h_stats.data() + l0 * 3, g.blk[q] + 8 + n * 8, n * 12);
-            }
+            if (int r = shard_ties(c, sh, count, over, block, 0, 20, lists, any_over)) return r;
             if (over) cap = count + count / 4;
             if (any_over) continue;
+            h_list.clear(); h_stats.clear();
+            for (const TieList& l : lists) {
+                const size_t l0 = h_list.size();
+                h_list.resize(l0 + l.n); h_stats.resize((l0 + l.n) * 3);
+                memcpy(h_list.data() + l0, l.p, l.n * 8);
+                memcpy(h_stats.data() + l0 * 3, l.p + l.n * 8, l.n * 12);
+            }
             count = h_list.size();
         }
         // the list comes in the order of the atomics: sort it by (fit, rule)
@@ -2483,24 +2547,16 @@ int scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, const uint
             i = end;
         }
         if (!sel.empty()) {
-            const unsigned long long* mat = (const unsigned long long*)c->matrix.p;
-            uint64_t mU = U, mpitch = c->pitch;
-            if (sharded) {
-                // exchange 3: the chosen columns from their owners; the update runs on their compact matrix
-                cols.clear();
-                for (uint64_t e : sel) cols.push_back((e & 0xffffffffULL) % UG);
-                cols = distinct(cols);
-                if (int r = shard_columns(c, sh, cols, &mat)) return r;
-                mU = mpitch = cols.size();
-                for (uint64_t& e : sel) {
-                    const uint64_t r = e & 0xffffffffULL;
-                    e = (e & ~0xffffffffULL) | (position(cols, r % UG) + (r >= UG ? mU : 0));
-                }
-            }
+            // exchange 3 on a slice: the chosen columns from their owners; the update runs on their compact matrix
+            cols.clear();
+            for (uint64_t e : sel) cols.push_back((e & 0xffffffffULL) % UG);
+            ColumnView v;
+            if (int r = column_view(c, sh, cols, v)) return r;
+            for (uint64_t& e : sel) e = (e & ~0xffffffffULL) | v.rule(e & 0xffffffffULL, UG);
             CU_TRY(c, cudaMemcpyAsync(d_sel, sel.data(), sel.size() * 8, cudaMemcpyHostToDevice, c->stream));
             const uint64_t nw = (uint64_t)sel.size() * W;
             k_scm_update<<<(uint32_t)std::min<uint64_t>((nw + 255) / 256, (uint64_t)c->sm_count * 8), 256, 0, c->stream>>>(
-                mat, mU, mpitch, W, d_sel, (uint32_t)sel.size(), d_masks);
+                v.matrix, v.U, v.pitch, W, d_sel, (uint32_t)sel.size(), d_masks);
             CU_TRY(c, cudaGetLastError());
             c->stats.n_launches++;
         }
@@ -2509,39 +2565,40 @@ int scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, const uint
     return GRMKM_OK;
 }
 
+// one fit's steps or one tree's nodes and their equivalent rules, copied to the caller's buffers (n, n_equivalent: how
+// many there are, whether they fit or not)
+template <class T>
+int copy_result(grmkm_ctx* c, const std::vector<T>& s, const std::vector<uint64_t>& e, T* dst, uint64_t cap, uint64_t* n,
+                uint64_t* equivalent, uint64_t equiv_cap, uint64_t* n_equivalent, const char* too_small) {
+    if (n) *n = s.size();
+    if (n_equivalent) *n_equivalent = e.size();
+    if ((!dst && !s.empty()) || cap < s.size() || (!equivalent && !e.empty()) || equiv_cap < e.size())
+        return fail(c, GRMKM_E_CAPACITY, too_small);
+    if (!s.empty()) memcpy(dst, s.data(), s.size() * sizeof(T));
+    if (!e.empty()) memcpy(equivalent, e.data(), e.size() * 8);
+    return GRMKM_OK;
+}
+
 }  // namespace
 
 extern "C" {
 
 int grmkm_scm_run(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, const uint64_t* blacklist, uint64_t n_blacklist) {
-    if (check_ctx(c)) return GRMKM_E_INVALID;
-    if (c->built && c->slice)
-        return fail(c, GRMKM_E_UNSUPPORTED, "the result is one owner's slice of a multi-GPU build: its best rule is not the answer");
-    Shard sh = whole_matrix(c);
-    return scm_run(c, n_fits, jobs, blacklist, n_blacklist, sh);
+    return scm_run(c, n_fits, jobs, blacklist, n_blacklist, nullptr,
+                   "the result is one owner's slice of a multi-GPU build: its best rule is not the answer");
 }
 
 int grmkm_scm_run_sharded(grmkm_ctx* c, uint32_t n_fits, const grmkm_scm_job* jobs, const uint64_t* blacklist,
                           uint64_t n_blacklist, const grmkm_shard* shard) {
-    if (check_ctx(c)) return GRMKM_E_INVALID;
-    Shard sh;
-    if (int r = shard_from(c, shard, sh)) return r;
-    return scm_run(c, n_fits, jobs, blacklist, n_blacklist, sh);
+    return scm_run(c, n_fits, jobs, blacklist, n_blacklist, shard, nullptr);
 }
 
 int grmkm_scm_result(grmkm_ctx* c, uint32_t fit, grmkm_scm_step* steps, uint64_t steps_cap, uint64_t* n_steps,
                      uint64_t* equivalent, uint64_t equiv_cap, uint64_t* n_equivalent) {
     if (check_ctx(c)) return GRMKM_E_INVALID;
     if (fit >= c->scm_steps.size()) return fail(c, GRMKM_E_INVALID, "no such fit in the last grmkm_scm_run");
-    const std::vector<grmkm_scm_step>& s = c->scm_steps[fit];
-    const std::vector<uint64_t>& e = c->scm_equiv[fit];
-    if (n_steps) *n_steps = s.size();
-    if (n_equivalent) *n_equivalent = e.size();
-    if ((!steps && !s.empty()) || steps_cap < s.size() || (!equivalent && !e.empty()) || equiv_cap < e.size())
-        return fail(c, GRMKM_E_CAPACITY, "scm result buffers too small");
-    if (!s.empty()) memcpy(steps, s.data(), s.size() * sizeof(grmkm_scm_step));
-    if (!e.empty()) memcpy(equivalent, e.data(), e.size() * 8);
-    return GRMKM_OK;
+    return copy_result(c, c->scm_steps[fit], c->scm_equiv[fit], steps, steps_cap, n_steps, equivalent, equiv_cap, n_equivalent,
+                       "scm result buffers too small");
 }
 
 }  // extern "C"
@@ -2601,12 +2658,8 @@ int cart_launch_chunk(grmkm_ctx* c, int passes, const CartNodeArg* d_args, uint3
 
 int cart_validate(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const uint64_t* blacklist, uint64_t n_blacklist,
                   const Shard& sh) {
-    if (!c->built) return fail(c, GRMKM_E_INVALID, "no result: call grmkm_build or grmkm_load_result first");
-    const uint64_t UG = sh.total;
-    const uint32_t W = c->W;
-    if (UG >= (1ULL << 31)) return fail(c, GRMKM_E_UNSUPPORTED, "CART indexes k-mers with 32 bits: at most 2^31 - 1 k-mers");
+    if (int r = check_run(c, sh, "CART indexes k-mers", blacklist, n_blacklist)) return r;
     if (n_trees && !jobs) return fail(c, GRMKM_E_INVALID, "null jobs");
-    if (n_blacklist && !blacklist) return fail(c, GRMKM_E_INVALID, "null blacklist");
     for (uint32_t t = 0; t < n_trees; ++t) {
         const grmkm_cart_job& j = jobs[t];
         const std::string at = " (tree " + std::to_string(t) + ")";
@@ -2616,23 +2669,18 @@ int cart_validate(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, co
         if (j.min_samples_split < 2) return fail(c, GRMKM_E_INVALID, "min_samples_split must be at least 2" + at);
         if (!(j.w_neg > 0.0 && j.w_neg <= 1e100) || !(j.w_pos > 0.0 && j.w_pos <= 1e100))
             return fail(c, GRMKM_E_INVALID, "class importances must be finite, > 0 and <= 1e100" + at);
-        if (W) {
-            int r = scm_check_mask(c, j.pos, "positive");
-            if (!r) r = scm_check_mask(c, j.neg, "negative");
-            if (r) return r;
-            for (uint32_t w = 0; w < W; ++w)
-                if (j.pos[w] & j.neg[w]) return fail(c, GRMKM_E_INVALID, "positive and negative examples overlap" + at);
-        }
+        if (int r = check_examples(c, j.pos, j.neg, at)) return r;
     }
-    for (uint64_t i = 0; i < n_blacklist; ++i)
-        if (blacklist[i] >= 2 * UG) return fail(c, GRMKM_E_INVALID, "blacklisted rule index >= 2 x n_kmers");
     return GRMKM_OK;
 }
 
 // The level loop of a batch of trees on this rank's columns; sh: the whole matrix (no exchange) or one slice of it.
 // Sharded, each level is: scan -> exchange the best keys -> both tie passes against the global keys -> exchange the
 // tie totals and lists -> the same host selection on every rank -> exchange the split columns -> gather and split.
-int cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const uint64_t* blacklist, uint64_t n_blacklist, Shard& sh) {
+int cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const uint64_t* blacklist, uint64_t n_blacklist,
+             const grmkm_shard* shard, const char* refusal) {
+    Shard sh;
+    if (int r = run_shard(c, shard, refusal, sh)) return r;
     if (int r = shard_agree(c, sh, cart_validate(c, n_trees, jobs, blacklist, n_blacklist, sh))) return r;
     const uint64_t U = c->U, UG = sh.total;
     const uint32_t W = c->W;
@@ -2673,9 +2721,7 @@ int cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const u
     if (open.empty()) return GRMKM_OK;
 
     CU_TRY(c, cudaSetDevice(c->device));
-    // chunk = open nodes whose masks share one CTA's shared memory; small enough for two CTAs per SM (as the SCM's)
-    const size_t smem_cap = (c->smem_optin ? c->smem_optin : 227 * 1024) - 1024;
-    const uint32_t chunk = (uint32_t)std::max<size_t>(1, std::min<size_t>(smem_cap / 2, 64 * 1024) / cart_smem_bytes(1, W));
+    const uint32_t chunk = chunk_size(c, cart_smem_bytes(1, W));
     const uint64_t max_grid = (uint64_t)c->sm_count * 8;
     const uint64_t bl_words = (U + 31) / 32;
     std::vector<uint32_t> h_bl(bl_words, 0);
@@ -2701,7 +2747,7 @@ int cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const u
     std::vector<CartSplit> splits;
     std::vector<uint64_t> h_best, h_total, h_list, block, cols;
     std::vector<uint32_t> h_stats;
-    Gathered g;
+    std::vector<TieList> lists;
     auto al = [](size_t b) { return (b + 255) & ~size_t(255); };
     while (!open.empty()) {
         const uint32_t n_open = (uint32_t)open.size();
@@ -2758,15 +2804,7 @@ int cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const u
                 h_best.resize(n_open);
                 CU_TRY(c, cudaMemcpyAsync(h_best.data(), d_best, (size_t)n_open * 8, cudaMemcpyDeviceToHost, c->stream));
                 CU_TRY(c, cudaStreamSynchronize(c->stream));
-                if (int r = shard_exchange(c, sh, h_best.data(), (uint64_t)n_open * 8, g)) return r;
-                for (uint32_t q = 0; q < sh.n_ranks; ++q) {
-                    if (g.len[q] != (uint64_t)n_open * 8) return fail(c, GRMKM_E_INVALID, "a rank sent keys of other nodes");
-                    for (uint32_t i = 0; i < n_open; ++i) {
-                        uint64_t x;
-                        memcpy(&x, g.blk[q] + (size_t)i * 8, 8);
-                        h_best[i] = std::max(h_best[i], x);
-                    }
-                }
+                if (int r = shard_max(c, sh, h_best, "a rank sent keys of other nodes")) return r;
                 CU_TRY(c, cudaMemcpyAsync(d_best, h_best.data(), (size_t)n_open * 8, cudaMemcpyHostToDevice, c->stream));
                 if (int r = launch(SCM_TIES)) return r;
             }
@@ -2774,35 +2812,29 @@ int cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const u
             CU_TRY(c, cudaStreamSynchronize(c->stream));
             const bool over = count > cap;
             if (sharded) {
-                // exchange 2: [count][tie totals][list, global columns]; an overflow anywhere redoes the level on every rank
+                // exchange 2: the tie totals of the open nodes, then the tie list with global columns
                 const uint64_t n_local = over ? 0 : count;
                 block.assign(1 + n_open + n_local, 0);
-                block[0] = count;
                 CU_TRY(c, cudaMemcpyAsync(block.data() + 1, d_total, (size_t)n_open * 8, cudaMemcpyDeviceToHost, c->stream));
                 CU_TRY(c, cudaMemcpyAsync(block.data() + 1 + n_open, c->cart_list.p, n_local * 8, cudaMemcpyDeviceToHost, c->stream));
                 CU_TRY(c, cudaStreamSynchronize(c->stream));
                 for (uint64_t i = 0; i < n_local; ++i) block[1 + n_open + i] += sh.off;
-                if (int r = shard_exchange(c, sh, block.data(), block.size() * 8, g)) return r;
                 bool any_over = false;
+                if (int r = shard_ties(c, sh, count, over, block, (uint64_t)n_open * 8, 8, lists, any_over)) return r;
+                if (over) cap = count + count / 4;
+                if (any_over) continue;
                 h_total.assign(n_open, 0);
                 h_list.clear();
-                for (uint32_t q = 0; q < sh.n_ranks; ++q) {
-                    uint64_t nq = 0;
-                    if (g.len[q] < 8 * (1 + (uint64_t)n_open)) return fail(c, GRMKM_E_INVALID, "a rank sent no tie list");
-                    memcpy(&nq, g.blk[q], 8);
-                    const uint64_t n = g.len[q] / 8 - 1 - n_open;
-                    if (n != nq) { if (n == 0) { any_over = true; continue; } return fail(c, GRMKM_E_INVALID, "a rank sent a malformed tie list"); }
+                for (const TieList& l : lists) {
                     for (uint32_t i = 0; i < n_open; ++i) {
                         uint64_t x;
-                        memcpy(&x, g.blk[q] + 8 + (size_t)i * 8, 8);
+                        memcpy(&x, l.p + (size_t)i * 8, 8);
                         h_total[i] += x;
                     }
                     const size_t l0 = h_list.size();
-                    h_list.resize(l0 + n);
-                    memcpy(h_list.data() + l0, g.blk[q] + 8 * (1 + (uint64_t)n_open), n * 8);
+                    h_list.resize(l0 + l.n);
+                    memcpy(h_list.data() + l0, l.p + (size_t)n_open * 8, l.n * 8);
                 }
-                if (over) cap = count + count / 4;
-                if (any_over) continue;
                 count = h_list.size();
                 break;
             }
@@ -2845,20 +2877,15 @@ int cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const u
         next.clear();
         if (!splits.empty()) {
             const uint32_t n_split = (uint32_t)splits.size();
-            const unsigned long long* mat = (const unsigned long long*)c->matrix.p;
-            uint64_t mpitch = c->pitch;
-            if (sharded) {
-                // exchange 3: the split columns from their owners; gather and split run on their compact matrix
-                cols.clear();
-                for (const CartSplit& s : splits) cols.push_back(s.j);
-                cols = distinct(cols);
-                if (int r = shard_columns(c, sh, cols, &mat)) return r;
-                mpitch = cols.size();
-                for (CartSplit& s : splits) s.j = (uint32_t)position(cols, s.j);
-            }
+            // exchange 3 on a slice: the split columns from their owners; gather and split run on their compact matrix
+            cols.clear();
+            for (const CartSplit& s : splits) cols.push_back(s.j);
+            ColumnView v;
+            if (int r = column_view(c, sh, cols, v)) return r;
+            for (CartSplit& s : splits) s.j = (uint32_t)v.col(s.j);
             CU_TRY(c, cudaMemcpyAsync(d_split, splits.data(), n_split * sizeof(CartSplit), cudaMemcpyHostToDevice, c->stream));
             k_cart_gather<<<(uint32_t)std::min<uint64_t>((n_split + 7) / 8, (uint64_t)c->sm_count * 16), 256, 0, c->stream>>>(
-                mat, mpitch, W, d_masks, d_split, n_split, d_stats);
+                v.matrix, v.pitch, W, d_masks, d_split, n_split, d_stats);
             CU_TRY(c, cudaGetLastError());
             c->stats.n_launches++;
             h_stats.resize(2 * (size_t)n_split);
@@ -2881,7 +2908,7 @@ int cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const u
                 CU_TRY(c, cudaMemcpyAsync(d_split, splits.data(), n_split * sizeof(CartSplit), cudaMemcpyHostToDevice, c->stream));
                 const uint64_t nw = (uint64_t)n_split * W;
                 k_cart_split<<<(uint32_t)std::min<uint64_t>((nw + 255) / 256, (uint64_t)c->sm_count * 8), 256, 0, c->stream>>>(
-                    mat, mpitch, W, d_masks, d_split, n_split, (unsigned long long*)c->cart_masks[cur ^ 1].p);
+                    v.matrix, v.pitch, W, d_masks, d_split, n_split, (unsigned long long*)c->cart_masks[cur ^ 1].p);
                 CU_TRY(c, cudaGetLastError());
                 c->stats.n_launches++;
                 cur ^= 1;
@@ -2898,34 +2925,21 @@ int cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const u
 extern "C" {
 
 int grmkm_cart_run(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const uint64_t* blacklist, uint64_t n_blacklist) {
-    if (check_ctx(c)) return GRMKM_E_INVALID;
-    if (c->built && c->slice)
-        return fail(c, GRMKM_E_UNSUPPORTED, "the result is one owner's slice of a multi-GPU build: its best split is not the answer");
-    Shard sh = whole_matrix(c);
-    return cart_run(c, n_trees, jobs, blacklist, n_blacklist, sh);
+    return cart_run(c, n_trees, jobs, blacklist, n_blacklist, nullptr,
+                    "the result is one owner's slice of a multi-GPU build: its best split is not the answer");
 }
 
 int grmkm_cart_run_sharded(grmkm_ctx* c, uint32_t n_trees, const grmkm_cart_job* jobs, const uint64_t* blacklist,
                            uint64_t n_blacklist, const grmkm_shard* shard) {
-    if (check_ctx(c)) return GRMKM_E_INVALID;
-    Shard sh;
-    if (int r = shard_from(c, shard, sh)) return r;
-    return cart_run(c, n_trees, jobs, blacklist, n_blacklist, sh);
+    return cart_run(c, n_trees, jobs, blacklist, n_blacklist, shard, nullptr);
 }
 
 int grmkm_cart_result(grmkm_ctx* c, uint32_t tree, grmkm_cart_node* nodes, uint64_t nodes_cap, uint64_t* n_nodes,
                       uint64_t* equivalent, uint64_t equiv_cap, uint64_t* n_equivalent) {
     if (check_ctx(c)) return GRMKM_E_INVALID;
     if (tree >= c->cart_nodes.size()) return fail(c, GRMKM_E_INVALID, "no such tree in the last grmkm_cart_run");
-    const std::vector<grmkm_cart_node>& s = c->cart_nodes[tree];
-    const std::vector<uint64_t>& e = c->cart_equiv[tree];
-    if (n_nodes) *n_nodes = s.size();
-    if (n_equivalent) *n_equivalent = e.size();
-    if ((!nodes && !s.empty()) || nodes_cap < s.size() || (!equivalent && !e.empty()) || equiv_cap < e.size())
-        return fail(c, GRMKM_E_CAPACITY, "cart result buffers too small");
-    if (!s.empty()) memcpy(nodes, s.data(), s.size() * sizeof(grmkm_cart_node));
-    if (!e.empty()) memcpy(equivalent, e.data(), e.size() * 8);
-    return GRMKM_OK;
+    return copy_result(c, c->cart_nodes[tree], c->cart_equiv[tree], nodes, nodes_cap, n_nodes, equivalent, equiv_cap,
+                       n_equivalent, "cart result buffers too small");
 }
 
 }  // extern "C"
@@ -3125,12 +3139,15 @@ namespace {
 
 // The jobs scored on this rank's matrix; sh: the whole matrix (no exchange) or one slice of it.  Sharded, the columns
 // of the jobs' rules and split k-mers are exchanged once and every rank scores all jobs on their compact matrix.
-int eval_run(grmkm_ctx* c, uint32_t n_jobs, const grmkm_eval_job* jobs, uint32_t* counts, uint64_t cap, Shard& sh) {
+int eval_run(grmkm_ctx* c, uint32_t n_jobs, const grmkm_eval_job* jobs, uint32_t* counts, uint64_t cap,
+             const grmkm_shard* shard, const char* refusal) {
+    Shard sh;
+    if (int r = run_shard(c, shard, refusal, sh)) return r;
     const uint64_t UG = sh.total;
     const uint32_t W = c->W;
     uint64_t pairs = 0, n_rules = 0, n_nodes = 0;
     auto validate = [&]() -> int {
-        if (!c->built) return fail(c, GRMKM_E_INVALID, "no result: call grmkm_build or grmkm_load_result first");
+        if (int r = check_run(c, sh, nullptr, nullptr, 0)) return r;
         if (n_jobs && !jobs) return fail(c, GRMKM_E_INVALID, "null jobs");
         std::vector<uint8_t> has_parent;
         for (uint32_t i = 0; i < n_jobs; ++i) {
@@ -3167,13 +3184,7 @@ int eval_run(grmkm_ctx* c, uint32_t n_jobs, const grmkm_eval_job* jobs, uint32_t
                 n_nodes += n;
                 pairs += n;
             }
-            if (W) {
-                int r = scm_check_mask(c, j.pos, "positive");
-                if (!r) r = scm_check_mask(c, j.neg, "negative");
-                if (r) return r;
-                for (uint32_t w = 0; w < W; ++w)
-                    if (j.pos[w] & j.neg[w]) return fail(c, GRMKM_E_INVALID, "positive and negative examples overlap" + at);
-            }
+            if (int r = check_examples(c, j.pos, j.neg, at)) return r;
         }
         if (cap < 2 * pairs) return fail(c, GRMKM_E_CAPACITY, "counts holds fewer than 2 x the count pairs of the jobs");
         if (pairs && !counts) return fail(c, GRMKM_E_INVALID, "null counts");
@@ -3203,20 +3214,14 @@ int eval_run(grmkm_ctx* c, uint32_t n_jobs, const grmkm_eval_job* jobs, uint32_t
         }
     }
     CU_TRY(c, cudaSetDevice(c->device));
-    const unsigned long long* mat = (const unsigned long long*)c->matrix.p;
-    uint64_t mU = c->U, mpitch = c->pitch;
-    if (sh.on()) {
-        // the columns of every rule and split k-mer, from their owners; the jobs name them by their compact index
-        std::vector<uint64_t> cols;
-        for (uint64_t r : h_rules) cols.push_back(r % UG);
-        for (const grmkm_eval_node& e : h_nodes) if (e.kmer != UINT64_MAX) cols.push_back(e.kmer);
-        cols = distinct(cols);
-        if (!cols.empty())
-            if (int r = shard_columns(c, sh, cols, &mat)) return r;
-        mU = mpitch = cols.size();
-        for (uint64_t& r : h_rules) r = position(cols, r % UG) + (r >= UG ? mU : 0);
-        for (grmkm_eval_node& e : h_nodes) if (e.kmer != UINT64_MAX) e.kmer = position(cols, e.kmer);
-    }
+    // on a slice, the columns of every rule and split k-mer from their owners; the jobs name them by their compact index
+    std::vector<uint64_t> cols;
+    for (uint64_t r : h_rules) cols.push_back(r % UG);
+    for (const grmkm_eval_node& e : h_nodes) if (e.kmer != UINT64_MAX) cols.push_back(e.kmer);
+    ColumnView v;
+    if (int r = column_view(c, sh, std::move(cols), v)) return r;
+    for (uint64_t& r : h_rules) r = v.rule(r, UG);
+    for (grmkm_eval_node& e : h_nodes) if (e.kmer != UINT64_MAX) e.kmer = v.col(e.kmer);
     auto al = [](size_t b) { return (b + 255) & ~size_t(255); };
     const size_t o_args = 0, o_rules = al((size_t)n_jobs * sizeof(EvalJobArg)), o_nodes = o_rules + al(n_rules * 8),
                  o_masks = o_nodes + al(n_nodes * sizeof(EvalNode)), o_cnt = o_masks + al(h_masks.size() * 8),
@@ -3232,7 +3237,7 @@ int eval_run(grmkm_ctx* c, uint32_t n_jobs, const grmkm_eval_job* jobs, uint32_t
     const uint32_t warps_per_cta = kEvalThreads / 32;
     const uint32_t grid = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((n_jobs + warps_per_cta - 1) / warps_per_cta,
                                                                               (uint64_t)c->sm_count * 8));
-    k_eval<<<grid, kEvalThreads, 0, st>>>(mat, mU, mpitch, W, (const EvalJobArg*)(base + o_args),
+    k_eval<<<grid, kEvalThreads, 0, st>>>(v.matrix, v.U, v.pitch, W, (const EvalJobArg*)(base + o_args),
                                           n_jobs, (const unsigned long long*)(base + o_rules), (const EvalNode*)(base + o_nodes),
                                           (const unsigned long long*)(base + o_masks), (uint32_t*)(base + o_cnt));
     CU_TRY(c, cudaGetLastError());
@@ -3247,19 +3252,13 @@ int eval_run(grmkm_ctx* c, uint32_t n_jobs, const grmkm_eval_job* jobs, uint32_t
 extern "C" {
 
 int grmkm_eval_run(grmkm_ctx* c, uint32_t n_jobs, const grmkm_eval_job* jobs, uint32_t* counts, uint64_t cap) {
-    if (check_ctx(c)) return GRMKM_E_INVALID;
-    if (c->built && c->slice)
-        return fail(c, GRMKM_E_UNSUPPORTED, "the result is one owner's slice of a multi-GPU build: it holds some k-mers only");
-    Shard sh = whole_matrix(c);
-    return eval_run(c, n_jobs, jobs, counts, cap, sh);
+    return eval_run(c, n_jobs, jobs, counts, cap, nullptr,
+                    "the result is one owner's slice of a multi-GPU build: it holds some k-mers only");
 }
 
 int grmkm_eval_run_sharded(grmkm_ctx* c, uint32_t n_jobs, const grmkm_eval_job* jobs, uint32_t* counts, uint64_t cap,
                            const grmkm_shard* shard) {
-    if (check_ctx(c)) return GRMKM_E_INVALID;
-    Shard sh;
-    if (int r = shard_from(c, shard, sh)) return r;
-    return eval_run(c, n_jobs, jobs, counts, cap, sh);
+    return eval_run(c, n_jobs, jobs, counts, cap, shard, nullptr);
 }
 
 int grmkm_copy_columns(grmkm_ctx* c, const uint64_t* idx, uint64_t n, uint64_t* dst, uint64_t cap) {
@@ -3416,13 +3415,7 @@ int grmkm_patterns(grmkm_ctx* c, const uint8_t* column_class, grmkm_ctx* d, uint
     float ms = 0.f;
     CU_TRY(c, cudaEventElapsedTime(&ms, ev[0], ev[1]));
     d->U = P; d->W = W; d->G = c->G; d->pitch = P;
-    d->built = true; d->slice = false; d->part_ranks = 0; d->pat_mult_on = true;
-    d->scm_steps.clear(); d->scm_equiv.clear();
-    d->cart_nodes.clear(); d->cart_equiv.clear();
-    d->stats = grmkm_stats{};
-    d->stats.n_kmers = d->stats.n_distinct = P;
-    d->stats.n_words = W; d->stats.n_genomes = c->G;
-    d->times = grmkm_times{};
+    set_result(d, true, true);
     if (stats) { stats->n_rounds = rounds; stats->n_patterns = P; stats->ms = ms; }
 
     // the mapping to the host: what fits, or GRMKM_E_CAPACITY (dst's result stands either way)

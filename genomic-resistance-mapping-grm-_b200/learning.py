@@ -43,12 +43,11 @@ class KmerRuleClassifications:
         self._kmers = None                 # packed k-mers, fetched once the SCM names a rule (scm.fit_many)
 
     # -- row bookkeeping (rules.py:171-199): rows are numbered among the rows not removed yet ------------
-    def _absolute_rows(self, rows) -> list[int]:
-        alive = np.nonzero(~self.dataset_removed_rows_mask)[0]
-        return [int(alive[int(r)]) for r in rows]
+    def _absolute_rows(self, rows) -> np.ndarray:
+        return np.nonzero(~self.dataset_removed_rows_mask)[0][np.asarray(rows, dtype=np.int64).reshape(-1)]
 
     def remove_rows(self, rows):
-        removed = self._absolute_rows(rows)
+        removed = self._absolute_rows(rows).tolist()
         if removed:
             self.dataset_removed_rows = sorted(set(self.dataset_removed_rows + removed))
             self.dataset_removed_rows_mask = np.zeros(self.dataset_initial_n_rows, dtype=bool)
@@ -59,36 +58,45 @@ class KmerRuleClassifications:
     def shape(self):
         return self.dataset_n_rows, self._U * 2
 
+    def row_mask(self, idx) -> np.ndarray:
+        """The W words with the bits of rows ``idx`` (among the rows not removed) set: build_row_mask, rules.py:209-222."""
+        rows = self._absolute_rows(idx)
+        mask = np.zeros(self._W, dtype=np.uint64)
+        np.bitwise_or.at(mask, rows // 64, np.left_shift(np.uint64(1), (63 - rows % 64).astype(np.uint64)))
+        return mask
+
     # -- sum_rows (rules.py:201-267) -----------------------------------------------------------------------
     def sum_rows(self, rows):
         """Number of the given rows (no duplicates) each rule classifies as positive: [presence rules | absence rules]."""
         rows = np.asarray(rows)
         result = np.zeros(self._U * 2, dtype=_minimum_uint_size(rows.shape[0]))
-        mask = np.zeros(self._W, dtype=np.uint64)
-        for idx in self._absolute_rows(np.sort(rows)):
-            mask[idx // 64] |= np.uint64(1) << np.uint64(64 - (idx - 64 * (idx // 64)) - 1)      # build_row_mask, rules.py:209-222
-        sums = self.builder.sum_rows(mask)
+        sums = self._column_sums(self.row_mask(rows))
         result[: self._U] = sums
         result[self._U:] = len(rows) - sums.astype(np.int64)
         return result
 
+    def _column_sums(self, row_mask) -> np.ndarray:
+        """The set bits of ``row_mask`` in each of the U columns."""
+        return self.builder.sum_rows(row_mask)
+
     # -- get_columns (rules.py:135-171) --------------------------------------------------------------------
     def get_columns(self, columns):
-        columns_is_int = False
-        if hasattr(columns, "__index__"):
-            columns = [columns.__index__()]
-            columns_is_int = True
-        columns = [int(c) for c in columns]
-        invert = np.array([c >= self._U for c in columns])
+        columns_is_int = hasattr(columns, "__index__")
+        columns = [columns.__index__()] if columns_is_int else [int(c) for c in columns]
+        invert = np.array([c >= self._U for c in columns], dtype=bool)
         cols = np.array([c % self._U if c >= self._U else c for c in columns], dtype=np.int64)
-        if self._matrix is None:
-            self._matrix = self.builder.matrix()
         row_mask = np.ones(self._W * 64, dtype=bool)
         row_mask[self.dataset_initial_n_rows:] = False
         row_mask[self.dataset_removed_rows] = False
-        result = _unpack_binary_bytes_from_ints(self._matrix[:, cols])[row_mask]
+        result = _unpack_binary_bytes_from_ints(self._column_words(cols))[row_mask]
         result[:, invert] = 1 - result[:, invert]
         return result.reshape(-1) if columns_is_int else result
+
+    def _column_words(self, cols) -> np.ndarray:
+        """The [W][len(cols)] words of columns ``cols``, from the host copy of the matrix (fetched once)."""
+        if self._matrix is None:
+            self._matrix = self.builder.matrix()
+        return self._matrix[:, cols]
 
     def kmers_at(self, idx) -> np.ndarray:
         """The packed k-mers of columns ``idx`` (the k-mers are fetched once)."""
@@ -147,34 +155,16 @@ class ShardedRuleClassifications(KmerRuleClassifications):
             out[:, sel] = np.frombuffer(blocks[r], dtype=np.uint64).reshape(n_words, int(sel.sum()))
         return out
 
-    def sum_rows(self, rows):
-        """As KmerRuleClassifications.sum_rows, for the global rules (one exchange of the slices' sums).  Collective."""
-        rows = np.asarray(rows)
-        mask = np.zeros(self._W, dtype=np.uint64)
-        for idx in self._absolute_rows(np.sort(rows)):
-            mask[idx // 64] |= np.uint64(1) << np.uint64(64 - (idx - 64 * (idx // 64)) - 1)
-        mine = self.builder.sum_rows(mask) if self.col_counts[self.rank] else np.zeros(0, dtype=np.uint32)
-        sums = np.concatenate([np.frombuffer(b, dtype=np.uint32) for b in
+    def _column_sums(self, row_mask) -> np.ndarray:
+        """The sums of the global columns: one exchange of the slices' sums.  sum_rows is collective."""
+        mine = self.builder.sum_rows(row_mask) if self.col_counts[self.rank] else np.zeros(0, dtype=np.uint32)
+        return np.concatenate([np.frombuffer(b, dtype=np.uint32) for b in
                                self.exchange.allgather(np.ascontiguousarray(mine, dtype=np.uint32).tobytes())])
-        result = np.zeros(self._U * 2, dtype=_minimum_uint_size(rows.shape[0]))
-        result[: self._U] = sums
-        result[self._U:] = len(rows) - sums.astype(np.int64)
-        return result
 
-    def get_columns(self, columns):
-        """As KmerRuleClassifications.get_columns, for global rule indices: each owner packs its requested columns on
-        its device (KmerMatrixBuilder.columns), one exchange.  Collective."""
-        columns_is_int = hasattr(columns, "__index__")
-        columns = [columns.__index__()] if columns_is_int else [int(c) for c in columns]
-        invert = np.array([c >= self._U for c in columns], dtype=bool)
-        cols = np.array([c % self._U if c >= self._U else c for c in columns], dtype=np.int64)
-        words = self._gather_columns(lambda local: self.builder.columns(local), cols, self._W)
-        row_mask = np.ones(self._W * 64, dtype=bool)
-        row_mask[self.dataset_initial_n_rows:] = False
-        row_mask[self.dataset_removed_rows] = False
-        result = _unpack_binary_bytes_from_ints(words)[row_mask]
-        result[:, invert] = 1 - result[:, invert]
-        return result.reshape(-1) if columns_is_int else result
+    def _column_words(self, cols) -> np.ndarray:
+        """The words of global columns: each owner packs its requested columns on its device
+        (KmerMatrixBuilder.columns), one exchange.  get_columns is collective."""
+        return self._gather_columns(self.builder.columns, cols, self._W)
 
     def kmers_at(self, idx) -> np.ndarray:
         """The packed k-mers of global columns ``idx``, from their owners (one exchange).  Collective."""
@@ -261,17 +251,8 @@ class PatternRuleClassifications(KmerRuleClassifications):
                         self.n_patterns + self.pattern_of[(rules - self._U) % max(self._U, 1)])
 
     # -- KmerRuleClassifications ---------------------------------------------------------------------------------------
-    def get_columns(self, columns):
-        columns_is_int = hasattr(columns, "__index__")
-        columns = [columns.__index__()] if columns_is_int else [int(c) for c in columns]
-        invert = np.array([c >= self._U for c in columns], dtype=bool)
-        cols = np.array([c % self._U if c >= self._U else c for c in columns], dtype=np.int64)
-        row_mask = np.ones(self._W * 64, dtype=bool)
-        row_mask[self.dataset_initial_n_rows:] = False
-        row_mask[self.dataset_removed_rows] = False
-        result = _unpack_binary_bytes_from_ints(self.builder.columns(cols))[row_mask]
-        result[:, invert] = 1 - result[:, invert]
-        return result.reshape(-1) if columns_is_int else result
+    def _column_words(self, cols) -> np.ndarray:
+        return self.builder.columns(cols)
 
     def kmers_at(self, idx) -> np.ndarray:
         return self._rc.kmers_at(idx)

@@ -19,7 +19,7 @@ import time
 import numpy as np
 
 from . import cart, native, scm
-from .scm import SetCoveringMachine, _refuse_slices, _row_mask
+from .scm import SetCoveringMachine, _refuse_slices
 
 
 def make_folds(labels, n_folds: int, random_seed: int = 0) -> np.ndarray:
@@ -175,11 +175,10 @@ def cross_validate_scm(rc, train_pos, train_neg, model_types, p_values, max_rule
     scm.fit_many(rc, [(m, s[0], s[1]) for ms, s in zip(machines, sets) for m in ms], rule_blacklist)
     t_fit = time.perf_counter() - t0
 
-    W = rc._W
     eval_sets = [(s[2], s[3]) for s in sets]
     if has_test:
         eval_sets.append((test_pos, test_neg))
-    masks = [(_row_mask(rc, a, W), _row_mask(rc, b, W)) for a, b in eval_sets]
+    masks = [(rc.row_mask(a), rc.row_mask(b)) for a, b in eval_sets]
     jobs = []
     for e, (pm, nm) in enumerate(masks):
         for m in machines[min(e, k)]:
@@ -325,13 +324,12 @@ def cross_validate_cart(rc, train_pos, train_neg, class_importances, max_depths,
     cart.fit_many(rc, [(t, s[0], s[1]) for ts, s in zip(trees, sets) for t in ts], rule_blacklist)
     t_fit = time.perf_counter() - t0
 
-    W = rc._W
     eval_sets = [(s[2], s[3]) for s in sets]
     if has_test:
         eval_sets.append((test_pos, test_neg))
     jobs = []
     for e, (a, b) in enumerate(eval_sets):
-        pm, nm = _row_mask(rc, a, W), _row_mask(rc, b, W)
+        pm, nm = rc.row_mask(a), rc.row_mask(b)
         for t in trees[min(e, k)]:
             jobs.append((native.EVAL_CART, 0, _eval_nodes(t.nodes), pm, nm))
     t0 = time.perf_counter()

@@ -75,13 +75,6 @@ def _refuse_slices(rule_classifications):
                          "gathered matrix (DistributedBuilder.gather, then load_result)")
 
 
-def _row_mask(rule_classifications, idx, W: int) -> np.ndarray:
-    rows = np.asarray(rule_classifications._absolute_rows(np.asarray(idx, dtype=np.int64).reshape(-1)), dtype=np.int64)
-    mask = np.zeros(W, dtype=np.uint64)
-    np.bitwise_or.at(mask, rows // 64, np.left_shift(np.uint64(1), (63 - rows % 64).astype(np.uint64)))
-    return mask
-
-
 def fit_many(rule_classifications, fits, rule_blacklist=None, tiebreaker="risk"):
     """Run every (machine, positive_example_idx, negative_example_idx) of ``fits`` to completion in one batch on the
     GPU (one pass over the matrix per greedy step of all pending fits).  The machines get their model and iterations."""
@@ -90,11 +83,11 @@ def fit_many(rule_classifications, fits, rule_blacklist=None, tiebreaker="risk")
         raise ValueError("tiebreaker must be 'risk' or None")
     rc = rule_classifications
     b = rc.builder
-    U, W = rc._U, rc._W
+    U = rc._U
     jobs = []
     for m, pos, neg in fits:
         jobs.append((_MODEL_TYPES[m.model_type], m.p, m.max_rules, tiebreaker == "risk",
-                     _row_mask(rc, pos, W), _row_mask(rc, neg, W)))
+                     rc.row_mask(pos), rc.row_mask(neg)))
     blacklist = np.asarray(rule_blacklist if rule_blacklist is not None else [], dtype=np.uint64).reshape(-1)
     results = b.scm_run(jobs, blacklist, shard=rc.shard)
     needed = sorted({int(s["rule"]) % U for _, (steps, _) in zip(fits, results) for s in steps})
